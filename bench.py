@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- pattern-optimisation scene samples/sec on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload = BASELINE.json configs[2] ("batched pattern optimisation": 4096 laser points into a 2048x2048
@@ -48,7 +48,13 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-side", action="store_true", help="skip the side measurements of the other single-GPU configs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy; with N GPUs "
+                         "rank 0 writes the allreduced gradient of the whole step and its own shard of the scene samples")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def config(batch, world):
@@ -210,6 +216,28 @@ def build_scene(ff, device):
     return sc
 
 
+DUMP_SUBSET = 1 << 20       # elements kept of an array larger than this: 4 MB each, about 13 MB for the whole dump
+
+
+def dump_outputs(dirname, dp, res, textures):
+    """Write what one PatternStep.forward_backward call returned as float32 ``<dirname>/<name>.npy``: the pattern gradient
+    ``dpoints`` [N,2] and the randomised ``world`` [B,E,4,4] and ``sampled`` [B,S,3] whole; of the transformed ``vertices``
+    [B,V,3] and of the step's textures (``PatternStep.last``: ``sum_texture`` [B,ts0,ts1], ``softor_texture`` [B,ts1,ts0]) the
+    elements at DUMP_SUBSET flat indices drawn, sorted, from torch.Generator().manual_seed(0) (``*_subset``, 1-D) when the
+    array is larger than that.  Same arguments, same inputs: two builds can be compared file by file.  With N ranks this is
+    rank 0's call: ``dpoints`` is allreduced over the step's B*N samples, everything else belongs to rank 0's B samples only,
+    so only dumps taken with the same number of ranks compare."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    arrays = {"dpoints": dp, "world": res.world, "sampled": res.sampled, "vertices": res.vertices,
+              "sum_texture": textures[0], "softor_texture": textures[1]}
+    for name, t in arrays.items():
+        if t.numel() > DUMP_SUBSET:
+            idx = torch.randint(0, t.numel(), (DUMP_SUBSET,), generator=torch.Generator().manual_seed(0)).sort().values
+            t, name = t.reshape(-1)[idx.to(t.device)], name + "_subset"
+        np.save(os.path.join(dirname, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def side_configs(ff, device, peak):
     """The other single-GPU BASELINE configs, as short side measurements (CUDA events, medians; inputs resident; a 256 MB buffer is
     rewritten between iterations so that nothing is served from L2).  Not the headline metric."""
@@ -364,8 +392,7 @@ def main_ours(args):
     def one_step(i, rec=None):
         # the public API: randomise B scenes (side stream) | bin + splat forward -> backward against the resident upstream
         # gradients -> fold over the samples + allreduce over the ranks
-        _, dp, _ = step_obj.forward_backward(pattern, upstream=(gS, gO), sample0=i * B * world + first, marks=rec)
-        return dp
+        return step_obj.forward_backward(pattern, upstream=(gS, gO), sample0=i * B * world + first, marks=rec)
 
     def barrier():
         if world > 1:
@@ -390,7 +417,7 @@ def main_ours(args):
     barrier()
     e0.record()
     for i in range(K):
-        one_step(Wm + i, marks[i])
+        _, last_dp, last_res = one_step(Wm + i, marks[i])
     e1.record()
     gc.enable()
     clocks.go()                                            # the device is K steps behind the host here: samples are under load
@@ -399,6 +426,8 @@ def main_ours(args):
     total_ms = max_over_ranks(e0.elapsed_time(e1), device)
     launches = nat.launch_count - l0          # our kernels only (the NCCL allreduce is not counted)
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:     # before the shared-pattern and e2e runs below reuse the step's buffers
+        dump_outputs(args.dump_outputs, last_dp, last_res, step_obj.last[:2])
     ms_step = total_ms / K
     value = B * world * K / (total_ms * 1e-3)
     order = ["start"] + phases[:-1] + ["end"]

@@ -9,17 +9,18 @@ CPU baseline.
 
 Parity status: the reference ships no tests, golden vectors or fixtures
 (SURVEY.md section 4), so parity is *unpinned by the reference itself*.  We pin
-the oracle against the reference's own code executed in the build container:
-``oracle/make_golden.py`` imports ``/root/reference`` (``oracle/ref_loader.py``)
-and writes ``tests/golden/*.npz``; ``tests/test_oracle_golden.py`` checks every
-function here against those fixtures (and against the live reference when it is
-mounted).  Third-party arithmetic that is absent from ``/root/reference`` and not
-installed (kornia 0.7.1 ``gaussian_blur2d``, geomdl 5.3.1 ``NURBS.Curve``) is restated
-from its published algorithm and pinned against independent implementations that ARE
-in the image (OpenCV, scipy): see ``gaussian_blur2d``, ``silhouette`` and the NURBS
-section below.  ``cv2.circle`` is the real OpenCV in the fixtures.
+the oracle against the reference's own code: ``oracle/make_golden.py`` imports a
+checkout of the original Fireflies project named by ``FIREFLIES_REF``
+(``oracle/ref_loader.py``) and writes ``tests/golden/*.npz``;
+``tests/test_oracle_golden.py`` checks every function here against those fixtures
+(and against the live reference when ``FIREFLIES_REF`` is set).  Third-party
+arithmetic that is absent from the reference and not installed (kornia 0.7.1
+``gaussian_blur2d``, geomdl 5.3.1 ``NURBS.Curve``) is restated from its published
+algorithm and pinned against independent implementations that ARE installed
+(OpenCV, scipy): see ``gaussian_blur2d``, ``silhouette`` and the NURBS section
+below.  ``cv2.circle`` is the real OpenCV in the fixtures.
 
-All citations are ``path:line`` relative to ``/root/reference``.
+All citations are ``path:line`` relative to the root of the original Fireflies project.
 """
 from __future__ import annotations
 

@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- writes ``tests/golden/*.npz`` by running the REAL reference
-(``/root/reference``, imported through ``oracle/ref_loader.py``) on CPU.
+(a checkout of the original Fireflies project, imported through ``oracle/ref_loader.py``) on CPU.
 
-Run in the build container only:  ``python oracle/make_golden.py``.
+Run with the reference at hand:  ``FIREFLIES_REF=<checkout> python oracle/make_golden.py``.
 The fixtures pin ``oracle/ff_oracle.py`` (and, on the GPU box, the CUDA path) to outputs of
 the reference's own code, because the reference ships no tests or golden vectors of its own.
 """
@@ -492,6 +492,52 @@ def poisson_cases(ff):
     print("wrote poisson_misc")
 
 
+LIVE_CASES = [(7, [33, 21], 6.0), (40, [96, 64], 20.0), (5, [16, 16], 49.0)]      # (points, texture size, sigma)
+LIVE_ANGLES = [0.0, 0.3, -2.5, 3.14159]
+
+
+def live_reference_outputs(ff):
+    """The reference's outputs that tests/test_oracle_golden.py::test_oracle_equals_live_reference compares the oracle with:
+    dense / baked / full-frame rasterisation on seeded points (texture sizes of one odd, one large and one square case) and the
+    yaw / pitch / roll matrices (the reference always receives an fp32 0-d tensor)."""
+    R, m = ff.graphics.rasterization, ff.utils.math
+    gen = torch.Generator().manual_seed(123)
+    out = {}
+    for i, (n, ts, sigma) in enumerate(LIVE_CASES):
+        pts = torch.rand(n, 2, generator=gen)
+        tsz, sg, c = torch.tensor(ts), torch.tensor([sigma]), f"c{i}_"
+        out.update({c + "points": npy(pts), c + "dense": npy(R.rasterize_points(pts, sigma, tsz, device=CPU)),
+                    c + "baked_sum": npy(R.baked_sum(pts, sg, tsz, device=CPU)),
+                    c + "baked_sum_2": npy(R.baked_sum_2(pts, sg, tsz, device=CPU)),
+                    c + "baked_softor_2": npy(R.baked_softor_2(pts, sg, tsz, device=CPU)),
+                    c + "baked_sum_std3": npy(R.baked_sum(pts, sg, tsz, num_std=3, device=CPU))})
+        if ts[0] == ts[1]:   # the loop-over-points full-frame variants only work on square textures
+            out[c + "points_baked_sum"] = npy(R.rasterize_points_baked_sum(pts, sigma, tsz, device=CPU))
+            out[c + "points_baked_softor"] = npy(R.rasterize_points_baked_softor(pts, sigma, tsz, device=CPU))
+    a32 = [torch.tensor(a) for a in LIVE_ANGLES]
+    for key, fn in (("yaw", m.getYawTransform), ("pitch", m.getPitchTransform), ("roll", m.getRollTransform)):
+        out[key] = np.stack([npy(fn(a, CPU)) for a in a32])
+    return out
+
+
+def live_reference_cases(ff):
+    out = live_reference_outputs(ff)
+    out["c1_dense"], out["c1_dense_stride"] = out["c1_dense"][:, ::2, ::2], np.int64(2)    # every other texel of [40,64,96]: 1 MB -> 250 kB
+    out["source"] = np.array("the original Fireflies code, run by oracle/make_golden.py::live_reference_cases")
+    np.savez_compressed(os.path.join(OUT, "live_reference.npz"), **out)
+    print("wrote live_reference")
+
+
+def reference_api(ff):
+    """Names and positional signatures of the reference package (oracle/ref_loader.py::api) for tests/test_abi_cpu.py."""
+    import json
+    out = {"source": "the original Fireflies tree, read by oracle/make_golden.py::reference_api",
+           **ref_loader.api(os.path.join(ref_loader.REF_ROOT, "fireflies"))}
+    with open(os.path.join(OUT, "reference_api.json"), "w") as f:
+        json.dump(out, f, indent=0, sort_keys=True)
+    print("wrote reference_api")
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
     torch.set_num_threads(8)
@@ -519,6 +565,8 @@ def main():
     perlin_cases(ff)
     curve_cases(ff)
     poisson_cases(ff)
+    live_reference_cases(ff)
+    reference_api(ff)
 
 
 if __name__ == "__main__":

@@ -1,6 +1,7 @@
 """CPU: the C-ABI library builds, loads and exports every symbol ``include/ffb200.h`` declares; ctypes structs
 match the C layouts; the product refuses to run without a GPU instead of falling back."""
 import ctypes as C
+import json
 import os
 import re
 import subprocess
@@ -8,6 +9,8 @@ import sys
 
 import pytest
 import torch
+
+from oracle import ref_loader
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HEADER = os.path.join(ROOT, "include", "ffb200.h")
@@ -109,34 +112,24 @@ def test_api_surface_matches_reference_names():
     assert ff.scene is ff.Scene
 
 
-def _ast_api(root):
-    import ast
-    out = {}
-    for dp, _, files in os.walk(root):
-        for f in files:
-            if not f.endswith(".py"):
-                continue
-            tree = ast.parse(open(os.path.join(dp, f)).read())
-            names = set()
-            for node in tree.body:
-                if isinstance(node, ast.FunctionDef):
-                    names.add(node.name)
-                elif isinstance(node, ast.ClassDef):
-                    names.add(node.name)
-                    names.update(f"{node.name}.{m.name}" for m in node.body if isinstance(m, ast.FunctionDef))
-                elif isinstance(node, ast.Assign):
-                    names.update(t.id for t in node.targets if isinstance(t, ast.Name))
-            out[os.path.relpath(os.path.join(dp, f), root)] = names
-    return out
+REFERENCE_API = os.path.join(ROOT, "tests", "golden", "reference_api.json")
+
+
+def reference_apis():
+    """The stored API of the original Fireflies package (``tests/golden/reference_api.json``, see its ``source``) and, when
+    ``FIREFLIES_REF`` names a checkout of the original, the API read from that tree as well."""
+    with open(REFERENCE_API) as f:
+        apis = [("stored", json.load(f))]
+    if ref_loader.available():
+        apis.append(("live", ref_loader.api(os.path.join(ref_loader.REF_ROOT, "fireflies"))))
+    return apis
 
 
 def test_every_reference_definition_has_a_counterpart_or_a_documented_reason():
-    """File by file, name by name (AST walk of both trees): everything the reference defines exists here under the same
-    module path and name, except the list below -- each entry is out of scope for a stated reason (DESIGN.md section 7)."""
-    ref_root = "/root/reference/fireflies"
-    if not os.path.isdir(ref_root):
-        pytest.skip("reference tree not mounted")
-    ref, ours = _ast_api(ref_root), _ast_api(os.path.join(ROOT, "fireflies_b200"))
+    """File by file, name by name (AST walk of this package against the reference's): everything the reference defines exists
+    here under the same module path and name, except the list below -- each entry is out of scope for a stated reason
+    (DESIGN.md section 7)."""
+    ours = ref_loader.api(os.path.join(ROOT, "fireflies_b200"))["names"]
     allowed_files = {
         "entity/flame.py": "FLAME shape model: external package + weights",
         "entity/shape.py": "NotImplementedError stub in the reference",
@@ -148,15 +141,16 @@ def test_every_reference_definition_has_a_counterpart_or_a_documented_reason():
         "entity/mesh.py": {"Mesh.randomize"},                 # inherited: Transformable.randomize composes T, R and (for meshes) S in one launch
         "projection/laser.py": {"Laser.near_clip", "Laser.far_clip"},     # inherited from Camera
     }
-    missing = {}
-    for rel, names in ref.items():
-        if rel in allowed_files:
-            continue
-        assert rel in ours, f"{rel} has no counterpart"
-        gone = {n for n in names - ours[rel] if not n.startswith("_")} - allowed_names.get(rel, set())
-        if gone:
-            missing[rel] = sorted(gone)
-    assert not missing, missing
+    for source, ref in reference_apis():
+        missing = {}
+        for rel, names in ref["names"].items():
+            if rel in allowed_files:
+                continue
+            assert rel in ours, f"{rel} has no counterpart ({source} reference API)"
+            gone = {n for n in set(names) - set(ours[rel]) if not n.startswith("_")} - allowed_names.get(rel, set())
+            if gone:
+                missing[rel] = sorted(gone)
+        assert not missing, (source, missing)
     import fireflies_b200 as ff
     assert hasattr(ff.entity.Mesh, "randomize") and hasattr(ff.projection.Laser, "near_clip") and hasattr(ff.projection.Laser, "far_clip")
 
@@ -164,36 +158,16 @@ def test_every_reference_definition_has_a_counterpart_or_a_documented_reason():
 def test_signatures_are_prefix_compatible_with_the_reference():
     """Every function / method that exists in both trees takes the reference's positional parameters, same names and order;
     this package only ever appends optional ones (e.g. ``variates=``, ``camera_to_world=``)."""
-    import ast
-    ref_root = "/root/reference/fireflies"
-    if not os.path.isdir(ref_root):
-        pytest.skip("reference tree not mounted")
-
-    def sigs(root):
-        out = {}
-        for dp, _, files in os.walk(root):
-            for f in files:
-                if not f.endswith(".py"):
-                    continue
-                rel = os.path.relpath(os.path.join(dp, f), root)
-                tree = ast.parse(open(os.path.join(dp, f)).read())
-                for node in tree.body:
-                    fns = [("", node)] if isinstance(node, ast.FunctionDef) else (
-                        [(node.name + ".", m) for m in node.body if isinstance(m, ast.FunctionDef)] if isinstance(node, ast.ClassDef) else [])
-                    for prefix, fn in fns:
-                        names = [a.arg for a in fn.args.posonlyargs + fn.args.args]
-                        out[(rel, prefix + fn.name)] = (names, len(names) - len(fn.args.defaults))
-        return out
-
-    ref, ours = sigs(ref_root), sigs(os.path.join(ROOT, "fireflies_b200"))
-    both = [k for k in ref if k in ours]
-    assert len(both) >= 200
-    for k in both:
-        (rn, rreq), (on, oreq) = ref[k], ours[k]
-        if k == ("entity/curve.py", "Curve.fromObj"):
-            continue
-        assert on[:len(rn)] == rn, (k, rn, on)
-        assert oreq <= rreq, (k, "more required parameters than the reference")
+    ours = ref_loader.api(os.path.join(ROOT, "fireflies_b200"))["signatures"]
+    for source, ref in reference_apis():
+        both = [k for k in ref["signatures"] if k in ours]
+        assert len(both) >= 200, source
+        for k in both:
+            (rn, rreq), (on, oreq) = ref["signatures"][k], ours[k]
+            if k == "entity/curve.py::Curve.fromObj":
+                continue
+            assert on[:len(rn)] == rn, (source, k, rn, on)
+            assert oreq <= rreq, (source, k, "more required parameters than the reference")
 
 
 def test_example_script_imports_without_a_gpu():

@@ -1,5 +1,5 @@
 """CPU: pins ``oracle/ff_oracle.py`` to fixtures generated from the real reference
-(``oracle/make_golden.py``), and to the live reference when ``/root/reference`` is mounted."""
+(``oracle/make_golden.py``), and also to the live reference when ``FIREFLIES_REF`` names a checkout of it."""
 import random
 
 import numpy as np
@@ -212,31 +212,33 @@ def test_postprocess(golden):
         close(b[r, c], acc, rtol=1e-5, atol=1e-6)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not mounted (GPU box)")
-def test_oracle_equals_live_reference():
-    """Randomised differential check against the reference executed here."""
-    ff = ref_loader.load()
-    R = ff.graphics.rasterization
-    cpu = torch.device("cpu")
-    gen = torch.Generator().manual_seed(123)
-    for (n, ts, sigma) in [(7, [33, 21], 6.0), (40, [96, 64], 20.0), (5, [16, 16], 49.0)]:
-        pts = torch.rand(n, 2, generator=gen)
-        tsz, sg = torch.tensor(ts), torch.tensor([sigma])
-        dense = R.rasterize_points(pts, sigma, tsz, device=cpu)
-        assert torch.equal(O.splat_dense(pts, sigma, ts), dense)
-        close(O.baked_sum(pts, sigma, ts), R.baked_sum(pts, sg, tsz, device=cpu), atol=1e-6)
-        close(O.baked_sum(pts, sigma, ts, transposed=True), R.baked_sum_2(pts, sg, tsz, device=cpu), atol=1e-6)
-        close(O.baked_softor(pts, sigma, ts), R.baked_softor_2(pts, sg, tsz, device=cpu), atol=1e-6)
-        close(O.baked_sum(pts, sigma, ts, num_std=3), R.baked_sum(pts, sg, tsz, num_std=3, device=cpu), atol=1e-6)
-        if ts[0] == ts[1]:   # the loop-over-points full-frame variants only work on square textures
-            close(O.reduce_sum(dense), R.rasterize_points_baked_sum(pts, sigma, tsz, device=cpu), atol=1e-5)
-            close(O.softor(dense), R.rasterize_points_baked_softor(pts, sigma, tsz, device=cpu), atol=1e-6)
-    m = ff.utils.math
-    for a in [0.0, 0.3, -2.5, 3.14159]:
-        a32 = torch.tensor(a)        # the reference always receives an fp32 0-d tensor
-        assert torch.equal(O.yaw(a32), m.getYawTransform(a32, cpu))
-        assert torch.equal(O.pitch(a32), m.getPitchTransform(a32, cpu))
-        assert torch.equal(O.roll(a32), m.getRollTransform(a32, cpu))
+def test_oracle_equals_live_reference(golden):
+    """Differential check on seeded inputs against the reference's outputs stored in ``tests/golden/live_reference.npz``
+    (see its ``source``) and, when ``FIREFLIES_REF`` names a checkout of the original, against the reference executed here."""
+    from oracle import make_golden
+    sources = [("stored", golden("live_reference"))]
+    if ref_loader.available():
+        sources.append(("live", make_golden.live_reference_outputs(ref_loader.load())))
+    for source, ref in sources:
+        for i, (n, ts, sigma) in enumerate(make_golden.LIVE_CASES):
+            c = f"c{i}_"
+            pts = T(ref[c + "points"])
+            assert pts.shape == (n, 2), source
+            dense = O.splat_dense(pts, sigma, ts)
+            st = int(ref.get(c + "dense_stride", 1))                     # the stored [40,64,96] stack keeps every other texel
+            assert np.array_equal(dense.numpy()[:, ::st, ::st], ref[c + "dense"]), (source, i)
+            close(O.baked_sum(pts, sigma, ts), ref[c + "baked_sum"], atol=1e-6)
+            close(O.baked_sum(pts, sigma, ts, transposed=True), ref[c + "baked_sum_2"], atol=1e-6)
+            close(O.baked_softor(pts, sigma, ts), ref[c + "baked_softor_2"], atol=1e-6)
+            close(O.baked_sum(pts, sigma, ts, num_std=3), ref[c + "baked_sum_std3"], atol=1e-6)
+            if ts[0] == ts[1]:   # the loop-over-points full-frame variants only work on square textures
+                close(O.reduce_sum(dense), ref[c + "points_baked_sum"], atol=1e-5)
+                close(O.softor(dense), ref[c + "points_baked_softor"], atol=1e-6)
+        for j, a in enumerate(make_golden.LIVE_ANGLES):
+            a32 = torch.tensor(a)        # the reference always receives an fp32 0-d tensor
+            assert np.array_equal(O.yaw(a32).numpy(), ref["yaw"][j]), (source, a)
+            assert np.array_equal(O.pitch(a32).numpy(), ref["pitch"][j]), (source, a)
+            assert np.array_equal(O.roll(a32).numpy(), ref["roll"][j]), (source, a)
 
 
 # ---- line / depth rasterisers (SURVEY 8(f) row 2) ---------------------------------------------------------
