@@ -36,15 +36,10 @@ constexpr int WROWS = 8;      // rows per warp
 constexpr int CTA = 256;      // 8 warps: 2 column halves x 4 row groups
 constexpr int CHUNK = 128;    // candidate records staged per pass
 constexpr int KCACHE = 6;     // cached g slots per warp in the backward (8 rows x 32 lanes each; dynamic smem)
-#ifndef FFB_PREP_CTA
-#define FFB_PREP_CTA 1024
-#endif
-constexpr int PREP_CTA = FFB_PREP_CTA;
+constexpr int PREP_CTA = 1024;
+constexpr int PREP_MINB = 1;
 constexpr int WT = 16;        // warp tile side of the warp-tile kernels (ffb_splat_wt.cuh)
-#ifndef FFB_WCH
-#define FFB_WCH 16
-#endif
-constexpr int WCH = FFB_WCH;  // candidates a warp stages at once; longer super-tile lists go to the overflow kernels.  Measured at 12 (25 resident
+constexpr int WCH = 16;       // candidates a warp stages at once; longer super-tile lists go to the overflow kernels.  Measured at 12 (25 resident
                               // backward warps instead of 22, but 3 % of the super tiles overflow): forward 0.403 / backward 0.625 ms against 0.382 / 0.614
 static_assert(WCH <= 16 && WCH % 4 == 0, "ballot masks hold 16 bits per tile; the staging structs are 16-byte aligned per WCH rows");
 
@@ -279,10 +274,7 @@ __device__ __forceinline__ float origin_axis_f(float P, int baked, int half) {
 // path (a list entry is a copy of its record), and the random 32-byte record reads of the emit phase were the kernel's
 // long-scoreboard stalls (profiles/r01n: issue 41 %, long scoreboard 51 % of the stall samples)
 template <bool FAST, bool SREC = false>
-#ifndef FFB_PREP_MINB
-#define FFB_PREP_MINB 1
-#endif
-__global__ void __launch_bounds__(PREP_CTA, FFB_PREP_MINB) prepare_kernel(PrepParams q) {
+__global__ void __launch_bounds__(PREP_CTA, PREP_MINB) prepare_kernel(PrepParams q) {
     extern __shared__ __align__(16) int sm[];
     const int band_tiles = q.band_rows * q.tgx;
     int* cnt = sm;                 // [band_tiles] counts, then exclusive offsets
@@ -646,7 +638,7 @@ struct RasterParams {
     const float* g_sum; const float* g_softor;    // backward
     float* d_pts;
     int eager;                // backward: request a super tile's first upstream boxes before its candidate list is known (dense patterns)
-    int log_tgx, log_T;       // log2 of tgx and T when both are powers of two (item decode of the persistent backward by shifts), else -1
+    int log_tgx, log_T;       // log2 of tgx and T when both are powers of two (item decode of the chunked backward by shifts), else -1
     float* loss;              // fused L1 backward: per-sample mean |softor - sum| (accumulated)
     float loss_inv;           // 1 / (ts0 * ts1)
 };
@@ -904,12 +896,11 @@ static WtConsts wt_consts(const ffb_splat_desc* d, const Plan& p) {
     fc.ho = (float)p.H_o + 0.5f;
     fc.c1 = 1.00000011920928955078125f;      // 1 + 2^-23
     // backward tile culling: a tile whose nearest texel centre has g < 1e-7 is skipped.  Measured at config 3 against fp64
-    // (scripts/grad_precision.py, scripts/gpu_cull.sh): error relative to the gradient norm 5.2e-7 at 1e-7 and 5.3e-7 at 1e-9 (the
+    // (scripts/grad_precision.py): error relative to the gradient norm 5.2e-7 at 1e-7 and 5.3e-7 at 1e-9 (the
     // round-1 threshold) -- below the kernels' own rounding -- and 8.2e-7 at 1e-6; 7 % fewer (candidate, tile) visits than at 1e-9.
     // Worst case (upstream of one sign, dropped ring all on one side): 170 texels x 3.5e-7 against one-sided sums of ~20, 1e-5 of a
     // non-cancelling gradient's norm = a tenth of the parity tolerance.
     fc.disc2 = (float)((double)d->sigma * sqrt(16.11809565095832));       // (d2 / sigma)^2 = ln(1e7)
-    if (const char* e = getenv("FFB_BWD_CULL_LN")) fc.disc2 = (float)((double)d->sigma * sqrt(atof(e)));   // dev switch: ln(1 / threshold)
     fc.disc2_f = (float)((double)d->sigma * sqrt(17.5) * 1.02);           // same margin as the exact soft-OR no-op radius h_o (make_plan)
     fc.near2 = (float)((double)d->sigma * sqrt(5.545177444479562));       // (d2 / sigma)^2 = ln(2^8)
     fc.s2 = (float)(sqrt(1.4426950408889634) / (double)d->sigma);
@@ -955,26 +946,27 @@ static int launch_fwd_tma(K kernel, KO overflow, const RasterParams& q, const Wt
     return 0;
 }
 
-// TMA-fed backward over the same strip grid (tensor maps of the upstream arrays as kernel parameters)
+// tensor maps of the upstream arrays (kernel parameters of the TMA-fed backward kernels)
 struct BwdMaps {
     CUtensorMap gs, go, sv, ot;
 };
+// TMA-fed backward over the same strip grid
 template <typename K, typename KO>
 static int launch_bwd_tma(K kernel, KO overflow, const RasterParams& q, const WtConsts& fc, const OvfParams& o, int B, cudaStream_t st,
-                          const BwdMaps& m, size_t stage_bytes, size_t smem_ovf, int nbuf = 3) {
+                          const BwdMaps& m, size_t stage_bytes, size_t smem_ovf) {
     const unsigned gy = (unsigned)((q.tgy + WB_WARPS * WT_S - 1) / (WB_WARPS * WT_S));
     if (B > 65535 || gy > 65535) return fail_arg(FFB_E_LIMIT, "splat: B or the tile rows exceed the grid limit (65535)");
-    const size_t smem = (size_t)WB_WARPS * nbuf * TMA_TILE_BYTES + 64 + stage_bytes * WB_WARPS;
+    const size_t smem = (size_t)WB_WARPS * 3 * TMA_TILE_BYTES + 64 + stage_bytes * WB_WARPS;
     if (smem > 48 * 1024) FFB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (smem_ovf > 48 * 1024) FFB_CUDA(cudaFuncSetAttribute(overflow, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ovf));
-    kernel<<<dim3((unsigned)q.tgx, gy, (unsigned)B), WB_CTA, smem, st>>>(q, fc, m.gs, m.go, m.sv, m.ot);
+    kernel<<<dim3((unsigned)q.tgx, gy, (unsigned)B), WB_CTA, smem, st>>>(q, fc, m.gs, m.go, m.sv);
     FFB_CUDA(cudaGetLastError());
     overflow<<<kNumSMs, WT_CTA, smem_ovf, st>>>(q, fc, o);
     FFB_CUDA(cudaGetLastError());
     return 0;
 }
 
-__device__ unsigned st_counters[64];      // work counters of the persistent backward launches in flight (ffb_splat_st.cuh)
+__device__ unsigned st_counters[64];      // work counters of the loss-mode backward launches in flight (ffb_splat_st.cuh)
 
 // One zeroed counter per launch: a slot of the per-device pool, handed out round-robin across ALL instantiations and streams (64
 // launches may be in flight; a launch lasts milliseconds), zeroed on the launching stream.
@@ -990,56 +982,52 @@ static int st_counter_slot(cudaStream_t st, unsigned** counter) {
     return 0;
 }
 
-// super-tile backward (ffb_splat_st.cuh): persistent one-warp CTAs walking the (super tile, sample) items for dense patterns,
-// one one-warp CTA per item otherwise
-template <typename KP, typename K, typename KO>
-static int launch_bwd_st(KP persistent, K oneshot, KO overflow, const RasterParams& q, const WtConsts& fc, const OvfParams& o, int B,
-                         cudaStream_t st, const BwdMaps& m, size_t smem, size_t smem_ovf, bool prefer_persistent = false) {
+// super-tile backward (ffb_splat_st.cuh) for dense patterns (q.eager), then the overflow kernel; splat_bwd_stp's item loop with the
+// two-stage request pipeline.
+//   chunk > 0 (plain mode, 8): a one-warp CTA walks `chunk` consecutive (super tile, sample) items; the hardware block scheduler
+//     balances the 131 k CTAs of a config-3 launch.  1.91 ms per 256 samples inside the bench step against 2.05 for the one-shot form
+//     (whose warp slots stay empty ~2 of every ~9 us) and 2.6-2.7 for the counter form (profiles/r02x/forms.log);
+//   chunk == 0 (loss mode): 148 x 22 resident warps claim items from a global counter.  The fused L1 step measured 4.03 ms end to end
+//     against 4.07 with chunks of 4 and 4.18 with chunks of 8 (B200 at 1000 W, 5 alternating rounds of bench.py --steps 20).
+template <typename K, typename KO>
+static int launch_bwd_stp(K kernel, KO overflow, const RasterParams& q, const WtConsts& fc, const OvfParams& o, int B, cudaStream_t st,
+                          const BwdMaps& m, size_t smem, size_t smem_ovf, int chunk) {
     if (B > 65535 || q.tgy > 65535) return fail_arg(FFB_E_LIMIT, "splat: B or the tile rows exceed the grid limit (65535)");
-    if (smem_ovf > 48 * 1024) FFB_CUDA(cudaFuncSetAttribute(overflow, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ovf));
     const long long items = (long long)q.T * B;
-    // Three launch forms of the same item loop (dense patterns; sparse ones -- !q.eager -- always take the one-shot kernel):
-    //   chunk   (default): a one-warp CTA walks FFB_SPLAT_BWD_CHUNK (8) consecutive items with the two-stage request pipeline of the
-    //           persistent kernel; the hardware block scheduler balances the 131 k CTAs of a config-3 launch.  1.91 ms per 256 samples
-    //           inside the bench step against 2.05 for the one-shot form (whose warp slots stay empty ~2 of every ~9 us) and 2.6-2.7 for
-    //           the counter form (scripts/gpu_forms.sh, profiles/r02x/forms.log);
-    //   counter (FFB_SPLAT_BWD_PERSIST=1): 148 x 20 resident warps claim items from a global counter.  Fastest of the three in
-    //           isolation until the chunks came (1.96 ms), but the slowest inside the step (2.07-2.24 ms next to 1.98 for the chunks,
-    //           profiles/r02x/forms.log) -- kept for the fused-loss mode, where it is the fastest;
-    //   oneshot (FFB_SPLAT_BWD_PERSIST=0): one CTA per item.
-    const char* e = getenv("FFB_SPLAT_BWD_PERSIST");
-    int chunk = prefer_persistent ? 0 : 8;
-    if (e && e[0] == '1') chunk = 0;
-    if (const char* c = getenv("FFB_SPLAT_BWD_CHUNK")) chunk = atoi(c) > 0 ? atoi(c) : 0;   // static chunks of consecutive items per CTA
-    const bool persist = !(e && e[0] == '0') && q.eager != 0;
-    if (persist && items < 0x7fffffffLL) {
-        unsigned* counter = nullptr;
-        if (chunk == 0)
-            if (int rc = st_counter_slot(st, &counter)) return rc;
-        static int occ = 0;                                 // per instantiation (the function is a template)
-        if (occ == 0) {
-            if (smem > 48 * 1024) FFB_CUDA(cudaFuncSetAttribute(persistent, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            FFB_CUDA(cudaFuncSetAttribute(persistent, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-            // queried with the size rounded up to the next KB, which stands in for the 1 KB the system reserves per CTA: with the exact
-            // 10.8 KB of the loss mode the query reported 20 or more CTAs per SM where ncu shows 19 resident (profiles/r02z/ncu_loss_summary.txt),
-            // and 148 CTAs of the counter form started only when the others were done
-            FFB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, persistent, 32, (smem + 1023) & ~(size_t)1023));
-            if (occ < 1) occ = 1;
-        }
-        // 20 resident warps per SM, not the 24 that fit: inside the full step on a board at its power cap 148 x 20 measured
-        // 4.11 ms per step against 4.32 (x 24, with 4.9 ms outliers when the power controller overshoots), 4.32 (x 16), 4.15 for
-        // the one-shot form and 4.41 for round 1's kernel (scripts/bench_ab.py, 5 alternating rounds of 10 steps on one box)
-        // the loss mode (int8 mirrored signs: 22 CTAs per SM fit): 2.31 / 2.26 / 2.22 ms per 256 samples with 19 / 20 / 22 resident warps per SM
-        const int cap_sm = prefer_persistent ? 22 : 20;
-        long long grid = (long long)kNumSMs * (occ < cap_sm ? occ : cap_sm);
-        if (const char* g = getenv("FFB_SPLAT_BWD_GRID")) grid = atoll(g) > 0 ? atoll(g) : grid;
-        if (grid > items) grid = items;
-        if (chunk > 0) grid = (items + chunk - 1) / chunk;
-        persistent<<<(unsigned)grid, 32, smem, st>>>(q, fc, m.gs, m.go, m.sv, m.ot, (int)items, counter, chunk);
-    } else {
-        if (smem > 48 * 1024) FFB_CUDA(cudaFuncSetAttribute(oneshot, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        oneshot<<<dim3((unsigned)q.tgx, (unsigned)q.tgy, (unsigned)B), 32, smem, st>>>(q, fc, m.gs, m.go, m.sv, m.ot);
+    if (items > 0x7fff0000LL) return fail_arg(FFB_E_LIMIT, "splat: 2^31 (super tile, sample) items or more in one backward");
+    if (smem_ovf > 48 * 1024) FFB_CUDA(cudaFuncSetAttribute(overflow, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ovf));
+    static int occ = 0;                                     // per instantiation (the function is a template): queried on every call, the fused L1 step ran 4.15-4.27 ms end to end instead of 4.01-4.05
+    if (occ == 0) {
+        if (smem > 48 * 1024) FFB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        FFB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+        // queried with the size rounded up to the next KB, which stands in for the 1 KB the system reserves per CTA: with the exact size
+        // the query reported more CTAs per SM than ncu showed resident (profiles/r02z/ncu_loss_summary.txt), and 148 CTAs of the counter
+        // form started only when the others were done
+        FFB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, 32, (smem + 1023) & ~(size_t)1023));
+        if (occ < 1) occ = 1;
     }
+    unsigned* counter = nullptr;
+    long long grid = chunk > 0 ? (items + chunk - 1) / chunk : 0;
+    if (chunk == 0) {
+        if (int rc = st_counter_slot(st, &counter)) return rc;
+        // 22 resident warps per SM: 2.31 / 2.26 / 2.22 ms per 256 samples with 19 / 20 / 22
+        grid = (long long)kNumSMs * (occ < 22 ? occ : 22);
+        if (grid > items) grid = items;
+    }
+    kernel<<<(unsigned)grid, 32, smem, st>>>(q, fc, m.gs, m.go, m.sv, m.ot, (int)items, counter, chunk);
+    FFB_CUDA(cudaGetLastError());
+    overflow<<<kNumSMs, WT_CTA, smem_ovf, st>>>(q, fc, o);
+    FFB_CUDA(cudaGetLastError());
+    return 0;
+}
+// super-tile backward for sparse patterns: one one-warp CTA of splat_bwd_st per (super tile, sample), then the overflow kernel
+template <typename K, typename KO>
+static int launch_bwd_st(K kernel, KO overflow, const RasterParams& q, const WtConsts& fc, const OvfParams& o, int B, cudaStream_t st,
+                         const BwdMaps& m, size_t smem, size_t smem_ovf) {
+    if (B > 65535 || q.tgy > 65535) return fail_arg(FFB_E_LIMIT, "splat: B or the tile rows exceed the grid limit (65535)");
+    if (smem > 48 * 1024) FFB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (smem_ovf > 48 * 1024) FFB_CUDA(cudaFuncSetAttribute(overflow, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ovf));
+    kernel<<<dim3((unsigned)q.tgx, (unsigned)q.tgy, (unsigned)B), 32, smem, st>>>(q, fc, m.gs, m.go);
     FFB_CUDA(cudaGetLastError());
     overflow<<<kNumSMs, WT_CTA, smem_ovf, st>>>(q, fc, o);
     FFB_CUDA(cudaGetLastError());
@@ -1461,74 +1449,62 @@ extern "C" int ffb_splat_bwd(const ffb_splat_desc* d, const float* pts, const vo
         const WtConsts fc = wt_consts(d, p);
         const int B = d->B;
         const OvfParams ov = {q.ovf, q.ovf + 1, B};
-        q.saved_softor = g_softor ? saved_softor : nullptr;
-        if (!p.mask_o) {
-            // production path: super-tile kernel, whole 64x16 blocks of the upstream arrays through TMA (needs 16-byte aligned
-            // bases and row pitches).  The soft-OR product is rebuilt unless FFB_SPLAT_BWD_SAVED=1 asks for the forward's output.
-            const char* e = getenv("FFB_SPLAT_NO_TMA");
-            const char* e2 = getenv("FFB_SPLAT_BWD_ST");
-            const char* e3 = getenv("FFB_SPLAT_BWD_SAVED");
-            const bool use_saved = q.saved_softor && e3 && e3[0] == '1';
-            BwdMaps m;
-            bool ok = !(e && e[0] == '1') && !(e2 && e2[0] == '0');
-            const uint64_t t0 = (uint64_t)d->ts0, t1 = (uint64_t)d->ts1;
+        const char* e = getenv("FFB_SPLAT_NO_TMA");         // tests: force the plain-load kernels
+        const bool tma_ok = !(e && e[0] == '1');
+        const uint64_t t0 = (uint64_t)d->ts0, t1 = (uint64_t)d->ts1;
+        BwdMaps m;
+        if (g_softor && p.mask_o) {
+            // soft-OR window tighter than its no-op radius: upstream 16x16 tiles through TMA, the soft-OR product read back from the
+            // forward's output when it is given, rebuilt otherwise
+            q.saved_softor = saved_softor;
+            bool ok = tma_ok && tma::encode_f32_3d(&m.go, g_softor, t0, t1, (uint64_t)B, WT, WT, CU_TENSOR_MAP_SWIZZLE_NONE);
+            if (ok && saved_softor) ok = tma::encode_f32_3d(&m.sv, saved_softor, t0, t1, (uint64_t)B, WT, WT, CU_TENSOR_MAP_SWIZZLE_NONE);
+            if (ok && g_sum)
+                ok = sum_transposed ? tma::encode_f32_3d(&m.gs, g_sum, t1, t0, (uint64_t)B, WT, WT, CU_TENSOR_MAP_SWIZZLE_64B)
+                                    : tma::encode_f32_3d(&m.gs, g_sum, t0, t1, (uint64_t)B, WT, WT, CU_TENSOR_MAP_SWIZZLE_NONE);
+            if (ok) {
+                if (!saved_softor) m.sv = m.go;             // unused maps still have to be valid kernel parameters
+                if (!g_sum) m.gs = m.go;
+#define FFB_TMA1(S, T, V) launch_bwd_tma(splat_bwd_tma<S, true, T, V>, splat_bwd_ovf<S, true, T, true, V>, q, fc, ov, B, st, m, \
+                                         sizeof(WarpStage<2, true, false, 1>), sizeof(WarpStage<2, true, false, 1>) * WT_WARPS)
+#define FFB_TMA(S, T) (saved_softor ? FFB_TMA1(S, T, true) : FFB_TMA1(S, T, false))
+                if (g_sum) return sum_transposed ? FFB_TMA(true, true) : FFB_TMA(true, false);
+                return FFB_TMA(false, false);
+#undef FFB_TMA
+#undef FFB_TMA1
+            }
+        } else {
+            // production path: super-tile kernel, whole 64x16 blocks of the upstream arrays through TMA (needs 16-byte aligned bases and
+            // row pitches).  The soft-OR product is rebuilt from the candidates (saved_softor is not read), as is the overflow kernel's.
+            bool ok = tma_ok;
             if (ok && g_softor) ok = tma::encode_f32_3d(&m.go, g_softor, t0, t1, (uint64_t)B, 2 * WT, WT, CU_TENSOR_MAP_SWIZZLE_128B);
-            if (ok && use_saved) ok = tma::encode_f32_3d(&m.sv, q.saved_softor, t0, t1, (uint64_t)B, 2 * WT, WT, CU_TENSOR_MAP_SWIZZLE_128B);
             if (ok && g_sum)
                 ok = sum_transposed ? tma::encode_f32_3d(&m.gs, g_sum, t1, t0, (uint64_t)B, WT, 2 * WT, CU_TENSOR_MAP_SWIZZLE_64B)
                                     : tma::encode_f32_3d(&m.gs, g_sum, t0, t1, (uint64_t)B, 2 * WT, WT, CU_TENSOR_MAP_SWIZZLE_128B);
             if (ok) {
                 if (!g_softor) m.go = m.gs;                 // unused maps still have to be valid kernel parameters
-                if (!use_saved) m.sv = g_softor ? m.go : m.gs;
                 if (!g_sum) m.gs = m.go;
-                m.ot = m.go;
+                m.sv = m.ot = m.go;
                 const size_t so = sizeof(WarpStage<1, true, false, 1>) * WT_WARPS;
-                if (!use_saved) q.saved_softor = nullptr;   // the overflow kernel rebuilds the product as well
                 // the sum window's truncation is dropped where every truncated texel has g < 2^-22 (its share of d/dP is below 1e-6):
                 // the gradient of the sum is then one addend of the same FFMA2 instead of two mask computations per visit
-                const char* e4 = getenv("FFB_SPLAT_BWD_MASK");
                 const double edge = (double)p.H_s * (double)p.H_s / (double)d->sigma;
-                const bool msk = g_sum && (e4 ? e4[0] == '1' : edge * edge < 15.25);
-#define FFB_ST0(S, O, T, K, V) launch_bwd_st(splat_bwd_stp<S, O, T, K, V ? ST_SAVED : ST_REBUILD>, splat_bwd_st<S, O, T, K, V ? ST_SAVED : ST_REBUILD>, \
-                                             splat_bwd_ovf<S, O, T, false, V>, q, fc, ov, B, st, m, (size_t)StSmem<S, O, T, V ? ST_SAVED : ST_REBUILD>::bytes, so)
-#define FFB_ST1(S, O, T, V) (msk ? FFB_ST0(S, O, T, true, V) : FFB_ST0(S, O, T, false, V))
-#define FFB_ST(S, O, T) (use_saved ? FFB_ST1(S, O, T, true) : FFB_ST1(S, O, T, false))
+                const bool msk = g_sum && edge * edge < 15.25;
+#define FFB_ST0(S, O, T, K)                                                                                                          \
+    (q.eager ? launch_bwd_stp(splat_bwd_stp<S, O, T, K, ST_REBUILD>, splat_bwd_ovf<S, O, T, false, false>, q, fc, ov, B, st, m,       \
+                              (size_t)StSmem<S, O, T, ST_REBUILD>::bytes, so, 8)                                                     \
+             : launch_bwd_st(splat_bwd_st<S, O, T, K>, splat_bwd_ovf<S, O, T, false, false>, q, fc, ov, B, st, m,                    \
+                             (size_t)StSmem<S, O, T, ST_REBUILD>::bytes, so))
+#define FFB_ST(S, O, T) (msk ? FFB_ST0(S, O, T, true) : FFB_ST0(S, O, T, false))
                 if (g_sum && g_softor) return sum_transposed ? FFB_ST(true, true, true) : FFB_ST(true, true, false);
-                if (g_sum) return sum_transposed ? FFB_ST1(true, false, true, false) : FFB_ST1(true, false, false, false);
-                return FFB_ST(false, true, false);
+                if (g_sum) return sum_transposed ? FFB_ST(true, false, true) : FFB_ST(true, false, false);
+                return FFB_ST0(false, true, false, false);
 #undef FFB_ST
-#undef FFB_ST1
 #undef FFB_ST0
             }
         }
-        {
-            // earlier generation (and every case with a masked soft-OR window): upstream 16x16 tiles through TMA
-            const char* e = getenv("FFB_SPLAT_NO_TMA");
-            BwdMaps m;
-            bool ok = !(e && e[0] == '1');
-            const uint64_t t0 = (uint64_t)d->ts0, t1 = (uint64_t)d->ts1;
-            if (ok && g_softor) ok = tma::encode_f32_3d(&m.go, g_softor, t0, t1, (uint64_t)B, WT, WT, CU_TENSOR_MAP_SWIZZLE_NONE);
-            if (ok && q.saved_softor) ok = tma::encode_f32_3d(&m.sv, q.saved_softor, t0, t1, (uint64_t)B, WT, WT, CU_TENSOR_MAP_SWIZZLE_NONE);
-            if (ok && g_sum)
-                ok = sum_transposed ? tma::encode_f32_3d(&m.gs, g_sum, t1, t0, (uint64_t)B, WT, WT, CU_TENSOR_MAP_SWIZZLE_64B)
-                                    : tma::encode_f32_3d(&m.gs, g_sum, t0, t1, (uint64_t)B, WT, WT, CU_TENSOR_MAP_SWIZZLE_NONE);
-            if (ok) {
-                if (!g_softor) m.go = m.gs;                 // unused maps still have to be valid kernel parameters
-                if (!q.saved_softor) m.sv = g_softor ? m.go : m.gs;
-                if (!g_sum) m.gs = m.go;
-                m.ot = m.go;
-#define FFB_TMA1(S, O, T, M, V) launch_bwd_tma(splat_bwd_tma<S, O, T, M, V>, splat_bwd_ovf<S, O, T, M, V>, q, fc, ov, B, st, m, \
-                                               sizeof(WarpStage<M ? 2 : 1, true, false, 1>), sizeof(WarpStage<M ? 2 : 1, true, false, 1>) * WT_WARPS)
-#define FFB_TMA2(S, O, T, M) (q.saved_softor ? FFB_TMA1(S, O, T, M, true) : FFB_TMA1(S, O, T, M, false))
-#define FFB_TMA(S, O, T) (p.mask_o ? FFB_TMA2(S, O, T, true) : FFB_TMA2(S, O, T, false))
-                if (g_sum && g_softor) return sum_transposed ? FFB_TMA(true, true, true) : FFB_TMA(true, true, false);
-                if (g_sum) return sum_transposed ? FFB_TMA1(true, false, true, false, false) : FFB_TMA1(true, false, false, false, false);
-                return FFB_TMA(false, true, false);
-#undef FFB_TMA
-#undef FFB_TMA2
-#undef FFB_TMA1
-            }
-        }
+        // plain-load fallback: textures the TMA unit cannot describe (unaligned base, sides not multiples of 4)
+        q.saved_softor = g_softor ? saved_softor : nullptr;
 #define FFB_BWD1(S, O, T, M, V) launch_wt(splat_bwd_wt<S, O, T, M, V>, splat_bwd_ovf<S, O, T, M, V>, q, fc, ov, B, st, WB_CTA, \
                                           sizeof(WarpStage<M ? 2 : 1, true, true, 1>) * WB_WARPS, sizeof(WarpStage<M ? 2 : 1, true, false, 1>) * WT_WARPS)
 #define FFB_BWD2(S, O, T, M) (q.saved_softor ? FFB_BWD1(S, O, T, M, true) : FFB_BWD1(S, O, T, M, false))
@@ -1561,58 +1537,34 @@ extern "C" int ffb_splat_bwd_l1(const ffb_splat_desc* d, const float* pts, const
     if (!p.fast || p.mask_o) return fail_arg(FFB_E_UNSUPPORTED, "splat_bwd_l1: needs the warp-tile path (texture larger than the footprints, exact soft-OR window)");
     RasterParams q;
     fill_raster(d, p, workspace, q);
-    q.g_sum = out_sum; q.g_softor = out_softor; q.saved_softor = out_softor; q.d_pts = d_pts;
+    q.g_sum = out_sum; q.g_softor = out_softor; q.d_pts = d_pts;
     q.loss = loss_out; q.loss_inv = 1.0f / ((float)d->ts0 * (float)d->ts1);
     cudaStream_t st = as_stream(stream);
     const int B = d->B;
+    // the super-tile kernel in its loss mode: whole 64x16 blocks of the forward's outputs, two request rounds per item when the sum is
+    // stored transposed (mirrored index -> signs in shared memory, then own index)
     BwdMaps m;
     const uint64_t t0 = (uint64_t)d->ts0, t1 = (uint64_t)d->ts1;
-    bool ok = tma::encode_f32_3d(&m.go, out_softor, t0, t1, (uint64_t)B, WT, WT, CU_TENSOR_MAP_SWIZZLE_NONE);
-    if (ok) ok = sum_transposed ? tma::encode_f32_3d(&m.sv, out_sum, t1, t0, (uint64_t)B, WT, WT, CU_TENSOR_MAP_SWIZZLE_NONE)
-                                : tma::encode_f32_3d(&m.sv, out_sum, t0, t1, (uint64_t)B, WT, WT, CU_TENSOR_MAP_SWIZZLE_NONE);
-    if (ok && sum_transposed) {
-        ok = tma::encode_f32_3d(&m.gs, out_sum, t1, t0, (uint64_t)B, WT, WT, CU_TENSOR_MAP_SWIZZLE_64B) &&
-             tma::encode_f32_3d(&m.ot, out_softor, t0, t1, (uint64_t)B, WT, WT, CU_TENSOR_MAP_SWIZZLE_64B);
-    } else if (ok) {
-        m.gs = m.sv; m.ot = m.go;
-    }
+    bool ok = tma::encode_f32_3d(&m.go, out_softor, t0, t1, (uint64_t)B, 2 * WT, WT, CU_TENSOR_MAP_SWIZZLE_128B);
+    if (ok) ok = sum_transposed ? tma::encode_f32_3d(&m.gs, out_sum, t1, t0, (uint64_t)B, 2 * WT, WT, CU_TENSOR_MAP_SWIZZLE_128B)
+                                : tma::encode_f32_3d(&m.gs, out_sum, t0, t1, (uint64_t)B, 2 * WT, WT, CU_TENSOR_MAP_SWIZZLE_128B);
+    if (ok && sum_transposed)
+        ok = tma::encode_f32_3d(&m.sv, out_sum, t1, t0, (uint64_t)B, WT, 2 * WT, CU_TENSOR_MAP_SWIZZLE_64B) &&
+             tma::encode_f32_3d(&m.ot, out_softor, t0, t1, (uint64_t)B, WT, 2 * WT, CU_TENSOR_MAP_SWIZZLE_64B);
+    else if (ok) { m.sv = m.gs; m.ot = m.go; }
     if (!ok) return fail_arg(FFB_E_UNSUPPORTED, "splat_bwd_l1: textures must be 16-byte aligned with sides that are multiples of 4 (TMA)");
     FFB_CUDA(cudaMemsetAsync(d_pts, 0, (size_t)B * d->N * 2 * sizeof(float), st));
     FFB_CUDA(cudaMemsetAsync(loss_out, 0, (size_t)B * sizeof(float), st));
     const WtConsts fc = wt_consts(d, p);
     const OvfParams ov = {q.ovf, q.ovf + 1, B};
-    const size_t stage = sizeof(WarpStage<1, true, false, 1>);
-    {
-        // production path: the super-tile kernel in its loss mode (whole 64x16 blocks of the forward's outputs, two request rounds per
-        // item: mirrored index -> signs in shared memory, then own index).  Measured 0.676 ms per 64 samples against 0.695 ms for
-        // splat_bwd_tma<LOSS> (profiles/r02q; 2000 against 2630 warp instructions per item); FFB_SPLAT_L1_ST=0 selects the latter.
-        const char* e2 = getenv("FFB_SPLAT_L1_ST");
-        BwdMaps n;
-        bool ok2 = !(e2 && e2[0] == '0');
-        if (ok2) ok2 = tma::encode_f32_3d(&n.go, out_softor, t0, t1, (uint64_t)B, 2 * WT, WT, CU_TENSOR_MAP_SWIZZLE_128B);
-        if (ok2) ok2 = sum_transposed ? tma::encode_f32_3d(&n.gs, out_sum, t1, t0, (uint64_t)B, 2 * WT, WT, CU_TENSOR_MAP_SWIZZLE_128B)
-                                      : tma::encode_f32_3d(&n.gs, out_sum, t0, t1, (uint64_t)B, 2 * WT, WT, CU_TENSOR_MAP_SWIZZLE_128B);
-        if (ok2 && sum_transposed)
-            ok2 = tma::encode_f32_3d(&n.sv, out_sum, t1, t0, (uint64_t)B, WT, 2 * WT, CU_TENSOR_MAP_SWIZZLE_64B) &&
-                  tma::encode_f32_3d(&n.ot, out_softor, t0, t1, (uint64_t)B, WT, 2 * WT, CU_TENSOR_MAP_SWIZZLE_64B);
-        else if (ok2) { n.sv = n.gs; n.ot = n.go; }
-        if (ok2) {
-            const char* e4 = getenv("FFB_SPLAT_BWD_MASK");
-            const double edge = (double)p.H_s * (double)p.H_s / (double)d->sigma;
-            const bool msk = e4 ? e4[0] == '1' : edge * edge < 15.25;
-            q.eager = 1;                                    // the loss needs every texel: every item requests its blocks
-#define FFB_SL(T, K) launch_bwd_st(splat_bwd_stp<true, true, T, K, ST_LOSS>, splat_bwd_st<true, true, T, K, ST_LOSS>, \
-                                   splat_bwd_ovf<true, true, T, false, true, true>, q, fc, ov, B, st, n, (size_t)StSmem<true, true, T, ST_LOSS>::bytes, stage * WT_WARPS, true)
-            if (sum_transposed) return msk ? FFB_SL(true, true) : FFB_SL(true, false);
-            return msk ? FFB_SL(false, true) : FFB_SL(false, false);
+    const size_t so = sizeof(WarpStage<1, true, false, 1>) * WT_WARPS;
+    const double edge = (double)p.H_s * (double)p.H_s / (double)d->sigma;     // sum-window mask as in ffb_splat_bwd
+    const bool msk = edge * edge < 15.25;
+#define FFB_SL(T, K) launch_bwd_stp(splat_bwd_stp<true, true, T, K, ST_LOSS>, splat_bwd_ovf<true, true, T, false, true, true>, q, fc, ov, B, st, m, \
+                                    (size_t)StSmem<true, true, T, ST_LOSS>::bytes, so, 0)
+    if (sum_transposed) return msk ? FFB_SL(true, true) : FFB_SL(true, false);
+    return msk ? FFB_SL(false, true) : FFB_SL(false, false);
 #undef FFB_SL
-        }
-    }
-    if (sum_transposed)
-        return launch_bwd_tma(splat_bwd_tma<true, true, true, false, true, true>, splat_bwd_ovf<true, true, true, false, true, true>, q, fc, ov,
-                              B, st, m, stage, stage * WT_WARPS, 4);
-    return launch_bwd_tma(splat_bwd_tma<true, true, false, false, true, true>, splat_bwd_ovf<true, true, false, false, true, true>, q, fc, ov,
-                          B, st, m, stage, stage * WT_WARPS, 3);
 }
 
 extern "C" int ffb_reduce_over_samples(const float* in, int32_t B, int64_t row_elems, float* out, void* stream) {

@@ -29,44 +29,25 @@
 // candidate -- 8.4 KB of shared memory per warp, 24 resident warps instead of 19.
 #pragma once
 
-#ifndef FFB_ST_MINB
-#define FFB_ST_MINB 22                    // register target of the allocation (80 registers: up to 24 one-warp CTAs per SM fit, 8.5 KB of shared memory + 1 KB reserved each); measured 0.526 / 0.542 / 0.823 ms per 64 samples at 22 / 20 / 24
-#endif
-#ifndef FFB_ST_PAIR
-#define FFB_ST_PAIR 1                     // two-candidate tiles: exclusive products are the other candidate's factor (no pass 1, no reciprocal)
-#endif
-#ifndef FFB_ST_EXACT
-#define FFB_ST_EXACT 0                    // 1: distances as exact differences scaled afterwards (three more packed multiplies per visit); 0: differences of
-#endif                                    // pre-scaled tile-relative coordinates (operands rounded to ~3e-7 before the subtraction)
-#ifndef FFB_ST_TRIPLE
-#define FFB_ST_TRIPLE 1                   // three-candidate tiles: all exponentials in registers, exclusive products are the other two factors
-#endif
-#ifndef FFB_ST_SIGN8
-#define FFB_ST_SIGN8 1                    // loss mode: mirrored signs as int8 (1 KB per warp, 22 resident warps) instead of bf16 (2.5 KB, 19)
-#endif
-#ifndef FFB_ST_DYN
-#define FFB_ST_DYN 1                      // persistent kernel: items claimed from a global counter (1) or walked with a fixed stride (0)
-#endif
-
+constexpr int ST_MINB = 22;               // register target of the allocation (80 registers: up to 24 one-warp CTAs per SM fit, 8.5 KB of shared memory + 1 KB reserved each); measured 0.526 / 0.542 / 0.823 ms per 64 samples at 22 / 20 / 24
 constexpr int ST_BOX = 4 * WT * WT * 4;   // one 64x16 fp32 block = 4 KB
 
-enum StMode { ST_REBUILD = 0, ST_SAVED = 1, ST_LOSS = 2 };
+enum StMode { ST_REBUILD, ST_LOSS };
 
 template <bool SUM, bool SOFTOR, bool SUM_T, int MODE>
 struct StSmem {
-    static constexpr int n_box = MODE == ST_LOSS ? 2 : ((SOFTOR ? 1 : 0) + (SUM ? 1 : 0) + ((SOFTOR && MODE == ST_SAVED) ? 1 : 0));
+    static constexpr int n_box = MODE == ST_LOSS ? 2 : ((SOFTOR ? 1 : 0) + (SUM ? 1 : 0));
     static constexpr int off_go = 0;                                   // LOSS: the soft-OR output at the tile's own index
     static constexpr int off_gs = MODE == ST_LOSS ? ST_BOX : (SOFTOR ? ST_BOX : 0);       // LOSS: the sum output at the tile's own index (as stored)
-    static constexpr int off_sv = 2 * ST_BOX;                          // SAVED: forward's soft-OR output
     // LOSS + SUM_T: the same two boxes first hold the outputs at the MIRRORED index (soft-OR in off_go, sum in off_gs, {16,32} boxes),
-    // from which the lane keeps two sign bits per texel, and then the outputs at the tile's own index
+    // from which the lane keeps one sign per texel, and then the outputs at the tile's own index
     static constexpr int off_bar = n_box * ST_BOX;
     static constexpr int off_rec = off_bar + 16;
     static constexpr int off_idx = off_rec + WCH * 16;
-    // LOSS + SUM_T: -sign(softor - sum) at the mirrored index, [column 64][row 16]: int8 with a 16-byte pitch (FFB_ST_SIGN8), or the sign
-    // as bf16 (-1, 0, +1) with a 40-byte pitch
+    // LOSS + SUM_T: -sign(softor - sum) at the mirrored index, [column 64][row 16] as int8 with a 16-byte pitch (1 KB per warp: 22 resident
+    // warps per SM, where the sign as bf16 with a 40-byte pitch took 2.5 KB and allowed 19)
     static constexpr int off_sgn = off_idx + WCH * 4;
-    static constexpr int sgn_pitch = FFB_ST_SIGN8 ? 16 : 40;
+    static constexpr int sgn_pitch = 16;
     static constexpr int bytes = off_sgn + ((MODE == ST_LOSS && SUM_T) ? 4 * WT * sgn_pitch : 0);
 };
 
@@ -82,7 +63,7 @@ struct StLane {
 __device__ __forceinline__ StLane st_lane(int lane, const WtConsts& fc) {
     StLane ln;
     const int qy = lane & 7, cg = lane >> 3;
-    const float sc = FFB_ST_EXACT ? 1.f : fc.r1;
+    const float sc = fc.r1;
     ln.rabs = make_float2((float)qy * sc, (float)(qy + 8) * sc);
     ln.cbs = (float)(4 * cg) * sc;
     ln.nat_e = (unsigned)(qy * 128 + ((cg ^ qy) << 4));
@@ -105,7 +86,6 @@ template <bool MSK>
 __device__ __forceinline__ StRow st_row(const float4 rc, const StLane& ln, const WtConsts& fc) {
     StRow r;
     r.dys = __fadd2_rn(ln.rabs, bc(-rc.y));
-    if (FFB_ST_EXACT) r.dys = __fmul2_rn(r.dys, bc(fc.r1));
     r.dy2 = __fmul2_rn(r.dys, r.dys);
     r.pa = r.pb = true;
     if (MSK) {
@@ -123,10 +103,6 @@ __device__ __forceinline__ StCol st_col(const float4 rc, const StTileCols& tc, c
     StCol c;
     c.dxs[0] = __fadd2_rn(tc.c01, bc(-rc.x));
     c.dxs[1] = __fadd2_rn(tc.c23, bc(-rc.x));
-    if (FFB_ST_EXACT) {
-        c.dxs[0] = __fmul2_rn(c.dxs[0], bc(fc.r1));
-        c.dxs[1] = __fmul2_rn(c.dxs[1], bc(fc.r1));
-    }
     if (MSK) {
 #pragma unroll
         for (int p = 0; p < 2; ++p) {
@@ -356,11 +332,11 @@ __device__ __forceinline__ void st_weigh_triple(unsigned rec, StPend& pd, float&
 }
 
 // ---- staging: one candidate per lane -> tile masks (ballots) and 16-byte records {(P0 - c0) r1, (P1 - r0) r1, (P0 - f0) r1, (P1 - f1) r1} ----
-__device__ __forceinline__ WtMasks st_stage(const RasterParams& q, const WtConsts& fc, bool grad, int bin, int beg, int n, int c0, int r0, int lane,
+__device__ __forceinline__ WtMasks st_stage(const RasterParams& q, const WtConsts& fc, int bin, int beg, int n, int c0, int r0, int lane,
                                             float4* rec, int* idx) {
     const float r0f = (float)r0, c0f = (float)c0;
     bool ta[4] = {false, false, false, false}, na[4] = {false, false, false, false};
-    if (grad && lane < n) {
+    if (lane < n) {
         const float4 ea = __ldg(reinterpret_cast<const float4*>(q.entries + (size_t)bin * q.cap + beg + lane));
         const uint4 eb = __ldg(reinterpret_cast<const uint4*>(q.entries + (size_t)bin * q.cap + beg + lane) + 1);
         const int clo = (int)(eb.y & 0xffff) - c0, chi = (int)(eb.y >> 16) - c0;
@@ -376,8 +352,7 @@ __device__ __forceinline__ WtMasks st_stage(const RasterParams& q, const WtConst
             ta[i] = clo < WT * i + WT && chi > WT * i && rr <= fc.disc2;
             na[i] = ta[i] && rr < fc.near2;
         }
-        const float sc = FFB_ST_EXACT ? 1.f : fc.r1;
-        rec[lane] = make_float4(px * sc, py * sc, (ea.x - ea.z) * fc.r1, (ea.y - ea.w) * fc.r1);
+        rec[lane] = make_float4(px * fc.r1, py * fc.r1, (ea.x - ea.z) * fc.r1, (ea.y - ea.w) * fc.r1);
         idx[lane] = (int)eb.z;
     }
     WtMasks mk;
@@ -389,10 +364,10 @@ __device__ __forceinline__ WtMasks st_stage(const RasterParams& q, const WtConst
 }
 
 // LOSS + SUM_T, first request round: the boxes hold the forward's outputs at the mirrored index ({16,32} boxes: [column 64][row 16]).
-// sign(softor - sum) of all 1024 texels goes to shared memory as bf16 (-1, 0, +1): lane L takes columns L and L + 32 -- four
+// -sign(softor - sum) of all 1024 texels goes to shared memory as int8 (-1, 0, +1): lane L takes columns L and L + 32 -- four
 // conflict-free LDS.128 per array and column (the 64-byte swizzle spreads the eight lanes of a phase over all banks), packed
-// subtractions, and one 8-byte store per four rows.  The consumer mapping (rows q, q + 8; columns 4 cg ..) reads them back with
-// conflict-free 16-bit loads.  (A first version kept two bits per texel in registers: 64 scalar loads and ~350 instructions per item.)
+// subtractions, and one 4-byte store per four rows.  The consumer mapping (rows q, q + 8; columns 4 cg ..) reads them back with
+// conflict-free 8-bit loads.  (A first version kept two bits per texel in registers: 64 scalar loads and ~350 instructions per item.)
 __device__ __forceinline__ unsigned st_sign_bf16x2(const float2 d) {
     // (sign(d.y) as bf16) << 16 | (sign(d.x) as bf16): the high halves of the two floats are d truncated to bf16 (zero only for a zero or
     // flushed difference), and sign(x) = min(max(x * 2^127, -1), 1) in packed bf16 -- four instructions per texel pair where the
@@ -415,16 +390,12 @@ __device__ __forceinline__ void st_loss_signs(unsigned sbase, int lane) {
             const float4 o = st_lds128(a + L::off_go), m = st_lds128(a + L::off_gs);
             const unsigned w0 = st_sign_bf16x2(__fadd2_rn(make_float2(o.x, o.y), neg2(make_float2(m.x, m.y))));
             const unsigned w1 = st_sign_bf16x2(__fadd2_rn(make_float2(o.z, o.w), neg2(make_float2(m.z, m.w))));
-            if (FFB_ST_SIGN8) {
-                // four bf16 signs -> four int8 of the NEGATED sign (what the consumer needs): top bytes 0x3f / 0xbf / 0x00 (0x80 for -0)
-                unsigned T;
-                asm("prmt.b32 %0, %1, %2, 0x7531;" : "=r"(T) : "r"(w0), "r"(w1));
-                const unsigned nz = T & 0x01010101u, sg = (T >> 7) & nz;
-                const unsigned out = (nz * 0xffu) ^ (sg * 0xfeu);                          // +1 -> 0xff, -1 -> 0x01, 0 -> 0x00
-                asm volatile("st.shared.u32 [%0], %1;" ::"r"(sbase + L::off_sgn + (unsigned)c * L::sgn_pitch + (unsigned)ch * 4u), "r"(out) : "memory");
-            } else {
-                asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(sbase + L::off_sgn + (unsigned)c * L::sgn_pitch + (unsigned)ch * 8u), "r"(w0), "r"(w1) : "memory");
-            }
+            // four bf16 signs -> four int8 of the NEGATED sign (what the consumer needs): top bytes 0x3f / 0xbf / 0x00 (0x80 for -0)
+            unsigned T;
+            asm("prmt.b32 %0, %1, %2, 0x7531;" : "=r"(T) : "r"(w0), "r"(w1));
+            const unsigned nz = T & 0x01010101u, sg = (T >> 7) & nz;
+            const unsigned out = (nz * 0xffu) ^ (sg * 0xfeu);                          // +1 -> 0xff, -1 -> 0x01, 0 -> 0x00
+            asm volatile("st.shared.u32 [%0], %1;" ::"r"(sbase + L::off_sgn + (unsigned)c * L::sgn_pitch + (unsigned)ch * 4u), "r"(out) : "memory");
         }
     }
 }
@@ -433,11 +404,6 @@ __device__ __forceinline__ float st_lds_s8(unsigned a) {
     asm volatile("ld.shared.s8 %0, [%1];" : "=r"(v) : "r"(a));
     return (float)v;
 }
-__device__ __forceinline__ float st_lds_bf16(unsigned a) {
-    unsigned short v;
-    asm volatile("ld.shared.u16 %0, [%1];" : "=h"(v) : "r"(a));
-    return __uint_as_float((unsigned)v << 16);
-}
 
 // one 16x16 tile of the resident super tile: upstream values of the lane's 8 texels from shared memory, then the tile's candidates
 template <bool SUM, bool SOFTOR, bool SUM_T, bool MSK, int MODE>
@@ -445,7 +411,6 @@ __device__ __forceinline__ void st_tile(unsigned sbase, int j, unsigned tm, unsi
                                         float& lacc, const StLane& ln, int lane, const WtConsts& fc) {
     typedef StSmem<SUM, SOFTOR, SUM_T, MODE> L;
     constexpr bool LOSS = MODE == ST_LOSS;
-    constexpr bool SAVED = MODE == ST_SAVED && SOFTOR;
     const unsigned nb = (ln.nat_e ^ ((unsigned)(j & 1) << 6)) + (unsigned)(j >> 1) * (ST_BOX / 2);
     float2 gs[4], gp[4];
     auto ld_nat = [&](int off, float2 (&v)[4]) {
@@ -479,29 +444,20 @@ __device__ __forceinline__ void st_tile(unsigned sbase, int j, unsigned tm, unsi
         if (tm == 0u) return;
         if (SUM_T) {
             // d loss / d sum at this texel = -sign(softor - sum) at the mirrored texel (st_loss_signs)
-            const unsigned t = sbase + L::off_sgn + (unsigned)(WT * j + 4 * (lane >> 3)) * L::sgn_pitch + (FFB_ST_SIGN8 ? 1u : 2u) * (unsigned)(lane & 7);
+            const unsigned t = sbase + L::off_sgn + (unsigned)(WT * j + 4 * (lane >> 3)) * L::sgn_pitch + (unsigned)(lane & 7);
 #pragma unroll
             for (int v = 0; v < 4; ++v) {
-                const unsigned a = t + (unsigned)(2 * (v & 1)) * L::sgn_pitch + (v >> 1) * (FFB_ST_SIGN8 ? 8u : 16u);
-                if (FFB_ST_SIGN8) gs[v] = make_float2(st_lds_s8(a), st_lds_s8(a + L::sgn_pitch));
-                else gs[v] = make_float2(-st_lds_bf16(a), -st_lds_bf16(a + L::sgn_pitch));
+                const unsigned a = t + (unsigned)(2 * (v & 1)) * L::sgn_pitch + (v >> 1) * 8u;
+                gs[v] = make_float2(st_lds_s8(a), st_lds_s8(a + L::sgn_pitch));
             }
         }
     } else {
         if (SUM) { if (SUM_T) ld_tr(L::off_gs, gs); else ld_nat(L::off_gs, gs); }
-        if (SOFTOR) {
-            ld_nat(L::off_go, gp);
-            if (SAVED && !one) {
-                float2 sv[4];
-                ld_nat(L::off_sv, sv);
-#pragma unroll
-                for (int v = 0; v < 4; ++v) gp[v] = __fmul2_rn(gp[v], make_float2(1.f - sv[v].x, 1.f - sv[v].y));
-            }
-        }
+        if (SOFTOR) ld_nat(L::off_go, gp);
     }
     StTileCols tc;
     {
-        const float sc = FFB_ST_EXACT ? 1.f : fc.r1;
+        const float sc = fc.r1;
         const float cfs = fmaf((float)j, (float)WT * sc, ln.cbs);
         tc.c01 = make_float2(cfs, cfs + sc);
         tc.c23 = make_float2(cfs + 2.f * sc, cfs + 3.f * sc);
@@ -511,11 +467,11 @@ __device__ __forceinline__ void st_tile(unsigned sbase, int j, unsigned tm, unsi
         return;
     }
     const int cands = __popc(tm);
-    if (FFB_ST_PAIR && MODE != ST_SAVED && cands == 2) {
+    if (cands == 2) {                                       // exclusive products are the other candidate's factor (no pass 1, no reciprocal)
         st_weigh_pair<SUM, MSK>(rec, pd, accr, tm, tc, ln, lane, fc, gs, gp);
         return;
     }
-    if (FFB_ST_TRIPLE && MODE != ST_SAVED && cands == 3) {
+    if (cands == 3) {
         st_weigh_triple<SUM, MSK>(rec, pd, accr, tm, tc, ln, lane, fc, gs, gp);
         return;
     }
@@ -533,12 +489,10 @@ __device__ __forceinline__ void st_tile(unsigned sbase, int j, unsigned tm, unsi
         st_weigh<SUM, SOFTOR, MSK, 1>(rec, pd, accr, tm & ~nm, tc, ln, lane, fc, gs, gp);
         return;
     }
-    unsigned rest = tm;
-    if (MODE == ST_REBUILD) {
-        // pass 1 over all candidates but one, whose exponentials then serve both passes: its exclusive product is the product so far
-        // (no reciprocal), and its factor completes the product for the others
-        const unsigned low = tm & (0u - tm);
-        rest = tm ^ low;
+    // pass 1 over all candidates but one, whose exponentials then serve both passes: its exclusive product is the product so far
+    // (no reciprocal), and its factor completes the product for the others
+    const unsigned low = tm & (0u - tm), rest = tm ^ low;
+    {
         float2 p[4] = {bc(1.f), bc(1.f), bc(1.f), bc(1.f)};
         st_prod(rec, rest, tc, ln, fc, p);
         int k;
@@ -575,7 +529,6 @@ __device__ __forceinline__ void st_issue_half(unsigned char* st_smem, uint64_t* 
                                               const CUtensorMap* tm_go, const CUtensorMap* tm_sv, const CUtensorMap* tm_ot, bool mirrored = false) {
     typedef StSmem<SUM, SOFTOR, SUM_T, MODE> L;
     constexpr bool LOSS = MODE == ST_LOSS;
-    constexpr bool SAVED = MODE == ST_SAVED && SOFTOR;
     if (tma::elect_one()) {
         const int ch = c0 + 2 * WT * h, o = h * (ST_BOX / 2);
         tma::mbar_expect_tx(bar, (unsigned)(L::n_box * ST_BOX / 2));
@@ -589,7 +542,6 @@ __device__ __forceinline__ void st_issue_half(unsigned char* st_smem, uint64_t* 
             if (SUM_T && !LOSS) tma::load_3d(st_smem + L::off_gs + o, tm_gs, bar, r0, ch, b);
             else tma::load_3d(st_smem + L::off_gs + o, tm_gs, bar, ch, r0, b);
         }
-        if (SAVED) tma::load_3d(st_smem + L::off_sv + o, tm_sv, bar, ch, r0, b);
     }
 }
 
@@ -606,22 +558,19 @@ __device__ __forceinline__ void st_flush(const RasterParams& q, float kh, const 
     }
 }
 
-// MODE ST_REBUILD / ST_SAVED: tm_gs = upstream sum gradient ([ts1,ts0] boxes {32,16}, or [ts0,ts1] boxes {16,32} when SUM_T),
-// tm_go = upstream soft-OR gradient, tm_sv = forward's soft-OR output (SAVED).
+// MODE ST_REBUILD: tm_gs = upstream sum gradient ([ts1,ts0] boxes {32,16}, or [ts0,ts1] boxes {16,32} when SUM_T), tm_go = upstream
+// soft-OR gradient; the soft-OR product is rebuilt from the candidates.
 // MODE ST_LOSS: upstream gradients of mean|softor - sum| formed from the forward's outputs (rasterization.py:589-599):
 // tm_go = soft-OR output, tm_gs = sum output addressed like the soft-OR output (its own index: [ts0,ts1] read as stored),
 // and for SUM_T tm_sv / tm_ot = sum / soft-OR outputs as {16,32} boxes at the mirrored index (a first request round into the same
-// two boxes: 8.5 KB of shared memory per warp like the other modes, where four resident boxes allowed only 13 warps per SM).
+// two boxes: 8.5 KB of shared memory per warp like the other mode, where four resident boxes allowed only 13 warps per SM).
 //
-// One-shot form: one one-warp CTA per (super tile, sample); nothing is requested for super tiles without candidates unless the
-// pattern is dense (q.eager).  Used for sparse patterns, where most super tiles are empty.
-template <bool SUM, bool SOFTOR, bool SUM_T, bool MSK, int MODE>
-__global__ void __launch_bounds__(32, FFB_ST_MINB) splat_bwd_st(RasterParams q, WtConsts fc, const __grid_constant__ CUtensorMap tm_gs,
-                                                                const __grid_constant__ CUtensorMap tm_go,
-                                                                const __grid_constant__ CUtensorMap tm_sv,
-                                                                const __grid_constant__ CUtensorMap tm_ot) {
-    typedef StSmem<SUM, SOFTOR, SUM_T, MODE> L;
-    constexpr bool LOSS = MODE == ST_LOSS;
+// One-shot form (sparse patterns, !q.eager, where most super tiles are empty; ST_REBUILD only): one one-warp CTA per (super tile,
+// sample), and nothing is requested for super tiles without candidates.
+template <bool SUM, bool SOFTOR, bool SUM_T, bool MSK>
+__global__ void __launch_bounds__(32, ST_MINB) splat_bwd_st(RasterParams q, WtConsts fc, const __grid_constant__ CUtensorMap tm_gs,
+                                                            const __grid_constant__ CUtensorMap tm_go) {
+    typedef StSmem<SUM, SOFTOR, SUM_T, ST_REBUILD> L;
     extern __shared__ __align__(1024) unsigned char st_smem[];
     const int lane = threadIdx.x;
     const int bx = blockIdx.x, sty = blockIdx.y, b = blockIdx.z;
@@ -636,56 +585,32 @@ __global__ void __launch_bounds__(32, FFB_ST_MINB) splat_bwd_st(RasterParams q, 
         tma::fence_mbar_init();
     }
     __syncwarp();
-    constexpr bool TWO = LOSS && SUM_T;                     // two request rounds: mirrored index (sign bits), then own index
-    auto issue = [&](bool mirrored) {                       // converged warp
-        st_issue_half<SUM, SOFTOR, SUM_T, MODE>(st_smem, bar, 0, c0, r0, b, &tm_gs, &tm_go, &tm_sv, &tm_ot, mirrored);
-        st_issue_half<SUM, SOFTOR, SUM_T, MODE>(st_smem, bar + 1, 1, c0, r0, b, &tm_gs, &tm_go, &tm_sv, &tm_ot, mirrored);
-    };
-    const bool eager = LOSS || q.eager;
-    if (eager) issue(TWO);
     const int* toff = q.tile_off + (size_t)bin * (q.T + 1) + (size_t)sty * q.tgx + bx;
     const int beg = __ldg(toff), n = __ldg(toff + 1) - beg;
-    const bool grad = n > 0 && n <= WCH;                   // empty: no gradient work; longer lists: overflow kernel
-    if (!grad && !LOSS) {
-        if (eager) {                                        // requested, not needed: the boxes must land before the CTA's shared memory goes away
-            tma::mbar_wait(bar, 0);
-            tma::mbar_wait(bar + 1, 0);
-        }
-        return;
-    }
-    if (!eager) issue(false);
+    if (n <= 0 || n > WCH) return;                          // empty: no gradient work; longer lists: overflow kernel
+    st_issue_half<SUM, SOFTOR, SUM_T, ST_REBUILD>(st_smem, bar, 0, c0, r0, b, &tm_gs, &tm_go, nullptr, nullptr);
+    st_issue_half<SUM, SOFTOR, SUM_T, ST_REBUILD>(st_smem, bar + 1, 1, c0, r0, b, &tm_gs, &tm_go, nullptr, nullptr);
     const StLane ln = st_lane(lane, fc);
     const unsigned sbase = tma::smem_u32(st_smem);
-    if (TWO) {
-        tma::mbar_wait(bar, 0);
-        tma::mbar_wait(bar + 1, 0);
-        st_loss_signs<L>(sbase, lane);
-        __syncwarp();                                       // the signs are in shared memory: the boxes may be overwritten
-        issue(false);
-    }
-    const WtMasks mk = st_stage(q, fc, grad, bin, beg, n, c0, r0, lane, rec, idx);
+    const WtMasks mk = st_stage(q, fc, bin, beg, n, c0, r0, lane, rec, idx);
     StPend pd = {0.f, 0.f, 0};
     float accr = 0.f;                                       // lane (k, h): d/dp_h of candidate k, summed over the super tile
-    float lacc = 0.f;                                       // LOSS: this lane's share of sum |softor - sum|
+    float lacc = 0.f;
     __syncwarp();
-    unsigned tbits = mk.tb01, nbits = mk.nb01;             // tile masks shifted out as the tiles go by (all zero without candidates)
+    unsigned tbits = mk.tb01, nbits = mk.nb01;             // tile masks shifted out as the tiles go by
 #pragma unroll 1
     for (int j = 0; j < 4; ++j) {
-        if (j == 0) tma::mbar_wait(bar, TWO ? 1u : 0u);
+        if (j == 0) tma::mbar_wait(bar, 0);
         if (j == 2) {
-            tma::mbar_wait(bar + 1, TWO ? 1u : 0u);
+            tma::mbar_wait(bar + 1, 0);
             tbits = mk.tb23; nbits = mk.nb23;
         }
         const unsigned tm = tbits & 0xffffu, nm = nbits & 0xffffu;
         tbits >>= 16; nbits >>= 16;
-        if (!LOSS && tm == 0u) continue;
-        st_tile<SUM, SOFTOR, SUM_T, MSK, MODE>(sbase, j, tm, nm, sbase + L::off_rec, pd, accr, lacc, ln, lane, fc);
+        if (tm == 0u) continue;
+        st_tile<SUM, SOFTOR, SUM_T, MSK, ST_REBUILD>(sbase, j, tm, nm, sbase + L::off_rec, pd, accr, lacc, ln, lane, fc);
     }
-    if (grad) st_flush(q, st_scale(q, fc, lane) * (LOSS ? q.loss_inv : 1.f), pd, accr, lane, n, b, idx);
-    if (LOSS) {
-        lacc = warp_sum(lacc);
-        if (lane == 0) atomicAdd(q.loss + b, lacc * q.loss_inv);
-    }
+    st_flush(q, st_scale(q, fc, lane), pd, accr, lane, n, b, idx);
 }
 
 // Pipelined item loop (dense patterns: nearly every super tile has candidates).  The one-shot kernel keeps only ~19 of its 24 warp slots
@@ -693,10 +618,9 @@ __global__ void __launch_bounds__(32, FFB_ST_MINB) splat_bwd_st(RasterParams q, 
 // dependent global loads (list bounds, then records) before it can do anything.  Here a warp walks several (super tile, sample) items:
 // the two halves of the upstream blocks sit behind one mbarrier each, and the next item's left half is requested as soon as tiles 0
 // and 1 of the current one are done, its right half after tiles 2 and 3 -- the same 8 KB of shared memory hold a two-stage pipeline.
-// The next item's list bounds are loaded a whole item ahead, its records are pulled into L1 half an item ahead.  Two ways to hand out
-// the items (launch_bwd_st): chunk > 0 -- the CTA walks `chunk` consecutive items and exits, the hardware block scheduler balances the
-// launch (the default, chunk = 8); chunk == 0 -- 148 x 20 resident warps claim items from a global counter, two items ahead (the
-// fused-loss mode).
+// The next item's list bounds are loaded a whole item ahead, its records are pulled into L1 half an item ahead.  The mode decides how
+// the items are handed out (launch_bwd_stp): ST_REBUILD -- the CTA walks `chunk` consecutive items and exits, the hardware block
+// scheduler balances the launch; ST_LOSS -- resident warps claim items from a global counter, two items ahead.
 struct StItem {
     int b, sty, bx;
 };
@@ -718,19 +642,17 @@ __device__ __forceinline__ StItem st_decode(const RasterParams& q, int it, float
     return s;
 }
 template <bool SUM, bool SOFTOR, bool SUM_T, bool MSK, int MODE>
-__global__ void __launch_bounds__(32, FFB_ST_MINB) splat_bwd_stp(RasterParams q, WtConsts fc, const __grid_constant__ CUtensorMap tm_gs,
-                                                                 const __grid_constant__ CUtensorMap tm_go,
-                                                                 const __grid_constant__ CUtensorMap tm_sv,
-                                                                 const __grid_constant__ CUtensorMap tm_ot, int n_items, unsigned* counter, int chunk) {
+__global__ void __launch_bounds__(32, ST_MINB) splat_bwd_stp(RasterParams q, WtConsts fc, const __grid_constant__ CUtensorMap tm_gs,
+                                                             const __grid_constant__ CUtensorMap tm_go,
+                                                             const __grid_constant__ CUtensorMap tm_sv,
+                                                             const __grid_constant__ CUtensorMap tm_ot, int n_items, unsigned* counter, int chunk) {
     typedef StSmem<SUM, SOFTOR, SUM_T, MODE> L;
     constexpr bool LOSS = MODE == ST_LOSS;
     extern __shared__ __align__(1024) unsigned char st_smem[];
     const int lane = threadIdx.x;
-    const int G = (int)gridDim.x;
-    // chunk > 0: a CTA walks `chunk` consecutive items (no counter; the hardware scheduler balances the CTAs); chunk == 0: persistent
-    int it = chunk > 0 ? (int)blockIdx.x * chunk : (int)blockIdx.x;
+    int it = LOSS ? (int)blockIdx.x : (int)blockIdx.x * chunk;
     if (it >= n_items) return;
-    if (chunk > 0) n_items = min(n_items, it + chunk);
+    if (!LOSS) n_items = min(n_items, it + chunk);
     uint64_t* bar = reinterpret_cast<uint64_t*>(st_smem + L::off_bar);
     float4* rec = reinterpret_cast<float4*>(st_smem + L::off_rec);
     int* idx = reinterpret_cast<int*>(st_smem + L::off_idx);
@@ -742,21 +664,19 @@ __global__ void __launch_bounds__(32, FFB_ST_MINB) splat_bwd_stp(RasterParams q,
     __syncwarp();
     const float inv_T = 1.0f / (float)q.T, inv_tgx = 1.0f / (float)q.tgx;
     auto toff_of = [&](const StItem& s) { return q.tile_off + (size_t)(q.shared_pattern ? 0 : s.b) * (q.T + 1) + (size_t)s.sty * q.tgx + s.bx; };
-    // claims an item: the first G items are the CTAs' own indices, the counter hands out the rest.  One lane asks (claim_ask) at the start
-    // of an item; the warp picks the answer up (claim_get) at its end, a whole item of work later.
-    const bool dyn = FFB_ST_DYN && chunk == 0;
+    // LOSS claims items: the first gridDim.x items are the CTAs' own indices, the counter hands out the rest.  One lane asks (claim_ask)
+    // at the start of an item; the warp picks the answer up (claim_get) at its end, a whole item of work later.
     auto claim_ask = [&]() {
         unsigned v = 0;
-        if (dyn && lane == 0) v = atomicAdd(counter, 1u);
+        if (LOSS && lane == 0) v = atomicAdd(counter, 1u);
         return v;
     };
-    auto claim_get = [&](unsigned v) { return (int)__shfl_sync(0xffffffffu, v, 0) + G; };
+    auto claim_get = [&](unsigned v) { return (int)__shfl_sync(0xffffffffu, v, 0) + (int)gridDim.x; };
     constexpr bool TWO = LOSS && SUM_T;                     // two request rounds per item: mirrored index (sign bits), then own index
     StItem cur = st_decode(q, it, inv_T, inv_tgx);
     st_issue_half<SUM, SOFTOR, SUM_T, MODE>(st_smem, bar, 0, cur.bx * (4 * WT), cur.sty * WT, cur.b, &tm_gs, &tm_go, &tm_sv, &tm_ot, TWO);
     st_issue_half<SUM, SOFTOR, SUM_T, MODE>(st_smem, bar + 1, 1, cur.bx * (4 * WT), cur.sty * WT, cur.b, &tm_gs, &tm_go, &tm_sv, &tm_ot, TWO);
-    const int step = chunk > 0 ? 1 : G;
-    int nit = dyn ? claim_get(claim_ask()) : it + step;      // the item after this one
+    int nit = LOSS ? claim_get(claim_ask()) : it + 1;        // the item after this one
     int beg, end;
     {
         const int* t = toff_of(cur);
@@ -780,7 +700,7 @@ __global__ void __launch_bounds__(32, FFB_ST_MINB) splat_bwd_stp(RasterParams q,
         const int n = end - beg, c0 = cur.bx * (4 * WT), r0 = cur.sty * WT;
         const bool grad = n > 0 && n <= WCH;               // empty: no gradient work; longer lists: overflow kernel
         if (TWO) {
-            // round 1 (requested during the previous item): outputs at the mirrored index -> two sign bits per texel; then round 2, the
+            // round 1 (requested during the previous item): outputs at the mirrored index -> one sign per texel; then round 2, the
             // outputs at the item's own index, lands while the candidates are staged.  Each barrier completes twice per item, so
             // the mirrored round always waits on parity 0 and the own round on parity 1.
             tma::mbar_wait(bar, 0);
@@ -792,7 +712,7 @@ __global__ void __launch_bounds__(32, FFB_ST_MINB) splat_bwd_stp(RasterParams q,
         }
         WtMasks mk;
         mk.tb01 = mk.tb23 = mk.nb01 = mk.nb23 = 0u;
-        if (grad) mk = st_stage(q, fc, true, q.shared_pattern ? 0 : cur.b, beg, n, c0, r0, lane, rec, idx);
+        if (grad) mk = st_stage(q, fc, q.shared_pattern ? 0 : cur.b, beg, n, c0, r0, lane, rec, idx);
         StPend pd = {0.f, 0.f, 0};
         float accr = 0.f, lacc = 0.f;
         __syncwarp();
@@ -824,7 +744,7 @@ __global__ void __launch_bounds__(32, FFB_ST_MINB) splat_bwd_stp(RasterParams q,
             if (lane == 0) atomicAdd(q.loss + cur.b, lacc * q.loss_inv);
         }
         if (!more) break;
-        it = nit; nit = dyn ? claim_get(asked) : nit + step; cur = nx; beg = nbeg; end = nend;
+        it = nit; nit = LOSS ? claim_get(asked) : nit + 1; cur = nx; beg = nbeg; end = nend;
         phase ^= 1u;
         __syncwarp();                                       // records and point indices of this item are dead
     }

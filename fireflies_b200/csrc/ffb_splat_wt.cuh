@@ -35,67 +35,21 @@
 //     this file, which walk the binning kernel's overflow list with the same device functions in chunks of 16.
 #pragma once
 
-#ifndef FFB_WT_S
-#define FFB_WT_S 1                        // backward: 0.624 / 0.658 / 0.654 / 0.651 ms per 64 samples at 1 / 2 / 3 / 4 (locality of the CTAs in flight beats the
-#endif                                    // cross-super-tile prefetch a longer strip allows)
-constexpr int WT_S = FFB_WT_S;            // vertically adjacent super tiles per warp (<= 16: one lane pair per super tile holds its list bounds)
-#ifndef FFB_RASTER_G
-#define FFB_RASTER_G 1
-#endif
-#ifndef FFB_WF_S
-#define FFB_WF_S 1
-#endif
-constexpr int WF_S = FFB_WF_S;            // ... in the TMA-store forward.  Measured per 64 samples (256-thread CTAs): 0.422 / 0.419 / 0.475 / 0.541 /
+constexpr int WT_S = 1;                   // vertically adjacent super tiles per warp (<= 16: one lane pair per super tile holds its list bounds).  Backward:
+                                          // 0.624 / 0.658 / 0.654 / 0.651 ms per 64 samples at 1 / 2 / 3 / 4 (locality of the CTAs in flight beats the
+                                          // cross-super-tile prefetch a longer strip allows)
+constexpr int WF_S = 1;                   // ... in the TMA-store forward.  Measured per 64 samples (256-thread CTAs): 0.422 / 0.419 / 0.475 / 0.541 /
                                           // 0.587 ms at 1 / 2 / 4 / 8 / 16: with short strips the CTAs in flight (scheduled column block first) write a
                                           // narrow band of texture rows at any time, and DRAM sees whole rows complete together
 constexpr int WT_CTA = 256;               // forward / overflow kernels: 8 warps x 4 super tiles (64 x 16 texels each) = 64 x 512 texels
 constexpr int WT_WARPS = WT_CTA / 32;
-#ifndef FFB_WF_CTA
-#define FFB_WF_CTA 64
-#endif
-constexpr int WF_CTA = FFB_WF_CTA;        // TMA-store forward (measured at one super tile per warp: 0.386 / 0.379 / 0.378 ms at 128 / 64 / 32 threads)
+constexpr int WF_CTA = 64;                // TMA-store forward (measured at one super tile per warp: 0.386 / 0.379 / 0.378 ms at 128 / 64 / 32 threads)
 constexpr int WF_WARPS = WF_CTA / 32;
-#ifndef FFB_WF_MINB
-#define FFB_WF_MINB (1024 / FFB_WF_CTA)   // 32 warps per SM at 64 registers
-#endif
-#ifndef FFB_FWD_ELECT
-#define FFB_FWD_ELECT 1                   // forward TMA stores / bulk-group waits under elect.sync (the same leader every time) instead of lane == 0 (A/B knob)
-#endif
-#ifndef FFB_TMA_ELECT
-#define FFB_TMA_ELECT 1                   // backward TMA requests under elect.sync instead of lane == 0 (A/B knob)
-#endif
-#ifndef FFB_WB_CTA
-#define FFB_WB_CTA 32
-#endif
-constexpr int WB_CTA = FFB_WB_CTA;        // backward: one warp per CTA (measured 0.67 ms vs 0.70 ms at 64 / 128 threads: a strip's slot frees the moment it ends; the forward prefers 8 warps)
+constexpr int WF_MINB = 1024 / WF_CTA;    // 32 warps per SM at 64 registers
+constexpr int WB_CTA = 32;                // backward: one warp per CTA (measured 0.67 ms vs 0.70 ms at 64 / 128 threads: a strip's slot frees the moment it ends; the forward prefers 8 warps)
 constexpr int WB_WARPS = WB_CTA / 32;
-#ifndef FFB_FFS_LOOP
-#define FFB_FFS_LOOP 1                    // 1: walk a tile's candidate mask with ffs (two XU-pipe ops per candidate); 0: test bit k of the mask for k < n
-#endif
-#ifndef FFB_BWD_SKIP
-#define FFB_BWD_SKIP 0                    // backward: skip 16x4 row groups outside a candidate's row span (measured slower: the branches cost more than the skipped MUFUs)
-#endif
-#ifndef FFB_BWD_DISC
-#define FFB_BWD_DISC 1                    // backward: drop (candidate, tile) pairs whose nearest texel is beyond the radius where g < 1e-7 (wt_consts)
-#endif
-#ifndef FFB_ACC_FOLD
-#define FFB_ACC_FOLD 0                    // backward: fold the parked partial sums once more (1 KB less shared memory per warp, one more shuffle per candidate tile)
-#endif
-#ifndef FFB_BWD_STAGED
-#define FFB_BWD_STAGED 1                  // backward inner loop staged over the four row groups (MUFU latencies overlap)
-#endif
-#ifndef FFB_FWD_DISC
-#define FFB_FWD_DISC 1                    // forward: drop (candidate, tile) pairs whose nearest texel is beyond the radius where g <= 2^-25
-#endif
-#ifndef FFB_BWD_FAR
-#define FFB_BWD_FAR 1                     // backward: tiles where every g < 2^-8 take 1/(1-g) = 1 + g + g^2 (+O(g^3) < 6e-8) on the FMA pipe instead of MUFU.RCP
-#endif
-#ifndef FFB_FWD_MINB
-#define FFB_FWD_MINB 4                    // resident CTAs per SM the register allocation aims for
-#endif
-#ifndef FFB_BWD_MINB
-#define FFB_BWD_MINB (FFB_WB_CTA == 32 ? 22 : 768 / FFB_WB_CTA)   // 22-24 warps per SM: what 80 registers and ~10 KB of shared memory per warp allow
-#endif
+constexpr int FWD_MINB = 4;               // resident CTAs per SM the register allocation aims for
+constexpr int BWD_MINB = 22;              // 22-24 warps per SM: what 80 registers and ~10 KB of shared memory per warp allow
 
 constexpr int TMA_TILE_BYTES = WT * WT * 4;   // one 16x16 fp32 tile as a TMA box
 
@@ -153,7 +107,7 @@ struct WarpStage {
     float4 tabB4[TABB == 2 ? WCH : 1][WT / 2];   // dy (2 rows), soft-OR row mask (2 rows)
     float2 tabB2[TABB == 1 ? WCH : 1][WT / 2];   // dy (2 rows)
     uint4 raw[NRAW][2 * WCH];             // candidate records as fetched by cp.async
-    float acc[ACC ? WCH : 1][FFB_ACC_FOLD ? 17 : 33];   // backward: parked d/dP partial sums (first half: d/dp0, second: d/dp1), row padded
+    float acc[ACC ? WCH : 1][33];   // backward: parked d/dP partial sums (first half: d/dp0, second: d/dp1), row padded
     float tin[TIN ? 2 : 1][TIN ? WT : 1][TIN ? 24 : 4];   // backward: upstream soft-OR gradient / saved output tile, rows padded to 24 (bank-conflict free)
 };
 
@@ -232,34 +186,30 @@ __device__ __forceinline__ WtMasks stage_regs(Stage& s, const EntryRegs& e, int 
             ta[i] = clo < WT * i + WT && chi > WT * i;
             if (rlo < 4 * i + 4 && rhi > 4 * i) gm |= 1u << i;
         }
-        if (ACC ? FFB_BWD_DISC : FFB_FWD_DISC) {
-            // backward: a tile whose nearest texel centre has g < 1e-7 contributes nothing measurable to d/dP (weights
-            // g * d2 * (c - P)); corner tiles of the square window go.  Forward: the radius is where g <= 2^-25, i.e. where
-            // the soft-OR factor 1 - g is exactly 1 and a sum term is below 3e-8 (half an ulp of a texel value of 0.5; the
-            // reference's own dense and baked sums differ by 2.4e-7).
-            const float ry = fmaxf(fmaxf(r0f - e.a.y, e.a.y - (r0f + (float)(WT - 1))), 0.f);
-            const float ry2 = ry * ry;
+        // backward: a tile whose nearest texel centre has g < 1e-7 contributes nothing measurable to d/dP (weights
+        // g * d2 * (c - P)); corner tiles of the square window go.  Forward: the radius is where g <= 2^-25, i.e. where
+        // the soft-OR factor 1 - g is exactly 1 and a sum term is below 3e-8 (half an ulp of a texel value of 0.5; the
+        // reference's own dense and baked sums differ by 2.4e-7).
+        const float ry = fmaxf(fmaxf(r0f - e.a.y, e.a.y - (r0f + (float)(WT - 1))), 0.f);
+        const float ry2 = ry * ry;
 #pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const float xl = (float)(c0 + WT * i);
-                const float rx = fmaxf(fmaxf(xl - e.a.x, e.a.x - (xl + (float)(WT - 1))), 0.f);
-                const float rr = fmaf(rx, rx, ry2);
-                ta[i] = ta[i] && rr <= (ACC ? fc.disc2 : fc.disc2_f);
-                na[i] = ta[i] && (!FFB_BWD_FAR || rr < fc.near2);
-            }
+        for (int i = 0; i < 4; ++i) {
+            const float xl = (float)(c0 + WT * i);
+            const float rx = fmaxf(fmaxf(xl - e.a.x, e.a.x - (xl + (float)(WT - 1))), 0.f);
+            const float rr = fmaf(rx, rx, ry2);
+            ta[i] = ta[i] && rr <= (ACC ? fc.disc2 : fc.disc2_f);
+            na[i] = ta[i] && rr < fc.near2;
         }
         s.cand[lane] = make_float4(e.a.x, e.a.z, __uint_as_float(e.b.z), __uint_as_float(gm));
         s.prow[lane] = make_float2(e.a.y, e.a.w);
     }
-    if (ACC) {
-        if (FFB_ACC_FOLD) { if (lane < 16) for (int k = 0; k < n; ++k) s.acc[k][lane] = 0.f; }
-        else for (int k = 0; k < n; ++k) s.acc[k][lane] = 0.f;
-    }
+    if (ACC)
+        for (int k = 0; k < n; ++k) s.acc[k][lane] = 0.f;
     WtMasks m;
     m.tb01 = __ballot_sync(0xffffffffu, ta[0]) | (__ballot_sync(0xffffffffu, ta[1]) << 16);
     m.tb23 = __ballot_sync(0xffffffffu, ta[2]) | (__ballot_sync(0xffffffffu, ta[3]) << 16);
     m.nb01 = m.tb01; m.nb23 = m.tb23;
-    if (ACC && FFB_BWD_DISC && FFB_BWD_FAR) {
+    if (ACC) {
         m.nb01 = __ballot_sync(0xffffffffu, na[0]) | (__ballot_sync(0xffffffffu, na[1]) << 16);
         m.nb23 = __ballot_sync(0xffffffffu, na[2]) | (__ballot_sync(0xffffffffu, na[3]) << 16);
     }
@@ -401,14 +351,9 @@ template <bool SUM, bool SOFTOR, bool MASK_O, typename Stage>
 __device__ __forceinline__ void accumulate_tile(const Stage& st, unsigned tm, int n, float cf, int h, const WtConsts& fc,
                                                 float2 (&acc_s)[4], float2 (&acc_p)[4]) {
     constexpr bool SCALED = StageTraits<Stage>::acc;                                  // backward stages hold d^2 * s2
-#if FFB_FFS_LOOP
     while (tm) {                                                                      // warp-uniform
         const int k = __ffs(tm) - 1;
         tm &= tm - 1;
-#else
-    for (int k = 0; k < n; ++k) {
-        if (!((tm >> k) & 1u)) continue;                                              // warp-uniform
-#endif
         const float2 cd = *reinterpret_cast<const float2*>(&st.cand[k]);
         const float dx = cf - cd.x;
         const float dx2 = SCALED ? __fmul_rn(dx, dx) * fc.s2 : __fmul_rn(dx, dx);
@@ -471,16 +416,7 @@ struct Strip {
 template <int WARPS, int S = WT_S>
 __device__ __forceinline__ bool strip_init(Strip& s, const RasterParams& q) {
     s.b = blockIdx.z;
-    // CTA rasterisation: the hardware issues CTAs with blockIdx.x fastest; FFB_RASTER_G > 1 walks bands of G CTA rows
-    // column block by column block instead (G vertically adjacent CTAs, then the next column block)
-    int bx = blockIdx.x, by = blockIdx.y;
-    if (FFB_RASTER_G > 1) {
-        const int lin = blockIdx.y * gridDim.x + blockIdx.x, per = FFB_RASTER_G * gridDim.x;
-        const int band = lin / per, r = lin - band * per;
-        const int g = min(FFB_RASTER_G, (int)gridDim.y - band * FFB_RASTER_G);
-        by = band * FFB_RASTER_G + r % g;
-        bx = r / g;
-    }
+    const int bx = blockIdx.x, by = blockIdx.y;
     s.bin = q.shared_pattern ? 0 : s.b;
     s.lane = threadIdx.x & 31;
     // one-warp CTAs: the warp index is the constant 0, which keeps the row coordinate of the TMA boxes in uniform registers
@@ -497,7 +433,7 @@ __device__ __forceinline__ bool strip_init(Strip& s, const RasterParams& q) {
 }
 
 template <bool SUM, bool SOFTOR, bool SUM_T, bool MASK_O>
-__global__ void __launch_bounds__(WT_CTA, FFB_FWD_MINB) splat_fwd_wt(RasterParams q, WtConsts fc) {
+__global__ void __launch_bounds__(WT_CTA, FWD_MINB) splat_fwd_wt(RasterParams q, WtConsts fc) {
     typedef WarpStage<MASK_O ? 2 : 0> Stage;
     __shared__ Stage stage[WT_WARPS];
     Strip sp;
@@ -542,7 +478,7 @@ __global__ void __launch_bounds__(WT_CTA, FFB_FWD_MINB) splat_fwd_wt(RasterParam
 // per output: no per-lane addresses, no edge path (the TMA unit clips boxes at the texture border).  In splat_fwd_wt
 // the stores and their address arithmetic were 130 of the ~340 instructions per tile.
 template <bool SUM, bool SOFTOR, bool SUM_T, bool MASK_O>
-__global__ void __launch_bounds__(WF_CTA, FFB_WF_MINB) splat_fwd_tma(RasterParams q, WtConsts fc, const __grid_constant__ CUtensorMap tm_s,
+__global__ void __launch_bounds__(WF_CTA, WF_MINB) splat_fwd_tma(RasterParams q, WtConsts fc, const __grid_constant__ CUtensorMap tm_s,
                                                                       const __grid_constant__ CUtensorMap tm_o) {
     typedef WarpStage<MASK_O ? 2 : 0> Stage;
     extern __shared__ __align__(1024) unsigned char wt_smem_ftma[];
@@ -578,7 +514,7 @@ __global__ void __launch_bounds__(WF_CTA, FFB_WF_MINB) splat_fwd_tma(RasterParam
 #pragma unroll
                 for (int i = 0; i < 4; ++i) { acc_s[i] = bc(0.f); acc_p[i] = bc(1.f); }
                 accumulate_tile<SUM, SOFTOR, MASK_O>(st, tile_mask(mk, j), n, (float)(ct + w.lc), w.h, fc, acc_s, acc_p);
-                if (FFB_FWD_ELECT ? tma::elect_one() : sp.lane == 0) tma::store_wait_read<0>();   // the previous tile's boxes have left the buffers
+                if (tma::elect_one()) tma::store_wait_read<0>();   // the previous tile's boxes have left the buffers
                 __syncwarp();
                 if (SOFTOR) {
 #pragma unroll
@@ -593,7 +529,7 @@ __global__ void __launch_bounds__(WF_CTA, FFB_WF_MINB) splat_fwd_tma(RasterParam
                 }
                 tma::fence_async_smem();
                 __syncwarp();
-                if (FFB_FWD_ELECT ? tma::elect_one() : sp.lane == 0) {
+                if (tma::elect_one()) {
                     if (SOFTOR) tma::store_3d(&tm_o, tout, ct, w.r0, w.b);
                     if (SUM) {
                         if (SUM_T) tma::store_3d(&tm_s, tout + TMA_TILE_BYTES, w.r0, ct, w.b);
@@ -605,7 +541,7 @@ __global__ void __launch_bounds__(WF_CTA, FFB_WF_MINB) splat_fwd_tma(RasterParam
         }
         n = nn;
     }
-    if (FFB_FWD_ELECT ? tma::elect_one() : sp.lane == 0) tma::store_wait_read<0>();   // shared memory must outlive the last boxes
+    if (tma::elect_one()) tma::store_wait_read<0>();   // shared memory must outlive the last boxes
 }
 
 // Backward.  dL/dg = gS * m_s + gO * m_o * prod / (1 - g) per (texel, point); dg/dP = 4 g d2 (c - P) / sigma^2.
@@ -618,29 +554,17 @@ __global__ void __launch_bounds__(WF_CTA, FFB_WF_MINB) splat_fwd_tma(RasterParam
 template <bool SUM, bool SOFTOR, bool MASK_O, bool FARV, typename Stage>
 __device__ __forceinline__ void weigh_tile(Stage& st, unsigned tm, int n, float cf, int h, int lane, const WtConsts& fc,
                                            const float2 (&gs)[4], const float2 (&gp)[4]) {
-#if FFB_FFS_LOOP
     while (tm) {
         const int k = __ffs(tm) - 1;
         tm &= tm - 1;
-#else
-    for (int k = 0; k < n; ++k) {
-        if (!((tm >> k) & 1u)) continue;
-#endif
-#if FFB_BWD_SKIP
-        const float4 cd = st.cand[k];
-        const unsigned gm = __float_as_uint(cd.w);
-#else
         const float2 cd = *reinterpret_cast<const float2*>(&st.cand[k]);
-        const unsigned gm = 15u;
-#endif
         const float dx = cf - cd.x;
         const float dx2 = __fmul_rn(dx, dx) * fc.s2;
         const float ec = fabsf(cf - cd.y);
         const bool pcs = ec <= fc.hs, pco = ec <= fc.ho;
         const float4* tA = &st.tabA[k][h];
         float2 a0 = bc(0.f), a1 = bc(0.f);
-#if FFB_BWD_STAGED
-        if (!MASK_O && !FFB_BWD_SKIP) {
+        if (!MASK_O) {
             // staged over the four row groups: all exponentials, then all reciprocals, then the FMA tail -- the special-function
             // latencies overlap instead of being waited for group by group (the ncu source view showed ~400 stall samples on
             // every first consumer of a MUFU result in the group-serial schedule)
@@ -687,10 +611,8 @@ __device__ __forceinline__ void weigh_tile(Stage& st, unsigned tm, int n, float 
                 a1 = __ffma2_rn(wgt, dy, a1);
             }
         } else
-#endif
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
-            if (FFB_BWD_SKIP && !(gm & (1u << i))) continue;                          // warp-uniform
             const float4 A = tA[2 * i];
             float4 Bq;
             if (MASK_O) Bq = st.tabB4[k][2 * i + h];
@@ -725,13 +647,7 @@ __device__ __forceinline__ void weigh_tile(Stage& st, unsigned tm, int n, float 
         }
         const float s0 = a0.x + a0.y, s1 = a1.x + a1.y;
         const float keep = h ? s1 : s0, give = h ? s0 : s1;
-#if FFB_ACC_FOLD
-        float v = keep + __shfl_xor_sync(0xffffffffu, give, 16);        // lanes 0-15: d/dp0 parts, 16-31: d/dp1 parts
-        v += __shfl_xor_sync(0xffffffffu, v, 8);                        // pairs folded: half the parking space
-        if (!(lane & 8)) st.acc[k][(lane & 7) + 8 * (lane >> 4)] += v;
-#else
         st.acc[k][lane] += keep + __shfl_xor_sync(0xffffffffu, give, 16);
-#endif
     }
 }
 
@@ -740,11 +656,10 @@ template <typename Stage>
 __device__ __forceinline__ void flush_warp(const Stage& st, int n, int h, int lc, float kh, float* __restrict__ dp) {
     __syncwarp();
     if (lc < n) {
-        constexpr int NP = FFB_ACC_FOLD ? 8 : 16;
-        const float* a = &st.acc[lc][NP * h];
+        const float* a = &st.acc[lc][16 * h];
         float x = 0.f, y = 0.f;
 #pragma unroll
-        for (int j = 0; j < NP; j += 2) { x += a[j]; y += a[j + 1]; }
+        for (int j = 0; j < 16; j += 2) { x += a[j]; y += a[j + 1]; }
         const float val = (x + y) * kh;
         if (val != 0.f) atomicAdd(dp + (size_t)__float_as_int(st.cand[lc].z) * 2, val);
     }
@@ -811,7 +726,7 @@ __device__ __forceinline__ void stage_tile_async(float (&buf)[WT][24], const flo
 }
 
 template <bool SUM, bool SOFTOR, bool SUM_T, bool MASK_O, bool SAVED>
-__global__ void __launch_bounds__(WB_CTA, FFB_BWD_MINB) splat_bwd_wt(RasterParams q, WtConsts fc) {
+__global__ void __launch_bounds__(WB_CTA, BWD_MINB) splat_bwd_wt(RasterParams q, WtConsts fc) {
     typedef WarpStage<MASK_O ? 2 : 1, true, true, 1> Stage;
     extern __shared__ __align__(16) unsigned char wt_smem[];
     Strip sp;
@@ -899,8 +814,8 @@ __global__ void __launch_bounds__(WB_CTA, FFB_BWD_MINB) splat_bwd_wt(RasterParam
                     for (int i = 0; i < 4; ++i) gp[i] = __fmul2_rn(gp[i], prod[i]);
                 }
                 const unsigned nm = near_mask(mk, j);
-                weigh_tile<SUM, SOFTOR, MASK_O, false>(st, (MASK_O || !FFB_BWD_FAR) ? tm : nm, n, cf, w.h, sp.lane, fc, gs, gp);
-                if (!MASK_O && FFB_BWD_FAR) weigh_tile<SUM, SOFTOR, MASK_O, true>(st, tm & ~nm, n, cf, w.h, sp.lane, fc, gs, gp);
+                weigh_tile<SUM, SOFTOR, MASK_O, false>(st, MASK_O ? tm : nm, n, cf, w.h, sp.lane, fc, gs, gp);
+                if (!MASK_O) weigh_tile<SUM, SOFTOR, MASK_O, true>(st, tm & ~nm, n, cf, w.h, sp.lane, fc, gs, gp);
             }
             flush_warp(st, n, w.h, w.lc, kh, dp);
             have = next_live;
@@ -911,7 +826,8 @@ __global__ void __launch_bounds__(WB_CTA, FFB_BWD_MINB) splat_bwd_wt(RasterParam
     }
 }
 
-// TMA-fed backward.  The ncu source view of splat_bwd_wt showed ~200 instructions of per-tile overhead around ~290 of
+// TMA-fed backward for soft-OR windows tighter than their no-op radius (every other case takes the super-tile kernel,
+// ffb_splat_st.cuh).  The ncu source view of splat_bwd_wt showed ~200 instructions of per-tile overhead around ~290 of
 // splat arithmetic: at an 80-register budget the compiler re-derives block / lane coordinates and the 64-bit addresses
 // of three arrays for every 16x16 tile.  Here the address generation belongs to the TMA unit: lane 0 issues one
 // cp.async.bulk.tensor box {16, 16, 1} per upstream array and tile (coordinates (column, row, sample); texels beyond
@@ -920,25 +836,17 @@ __global__ void __launch_bounds__(WB_CTA, FFB_BWD_MINB) splat_bwd_wt(RasterParam
 // 64-byte swizzle so that a lane's (column, row pair) reads are conflict free; no shuffles are needed any more.
 // One 3 KB buffer set per warp: a tile's values move to registers first, then the next tile's boxes are requested and
 // land while this tile is computed.
-//
-// LOSS: the upstream gradients are those of mean|softor - sum| (torch.nn.L1Loss on the two reductions as stored,
-// rasterization.py:589-599) and are formed here from the forward's outputs instead of being read: tm_go / tm_sv are
-// the soft-OR / sum outputs at the tile's own index, and -- when the sum is stored transposed ([ts0, ts1], square
-// textures) -- tm_gs / tm_ot the sum / soft-OR outputs at the mirrored index, which is where this tile's sum texels
-// meet their partners.  Every tile of the strip is visited (the loss needs all texels); super tiles without a
-// usable candidate list only contribute to the loss.
-template <bool SUM, bool SOFTOR, bool SUM_T, bool MASK_O, bool SAVED, bool LOSS = false>
-__global__ void __launch_bounds__(WB_CTA, FFB_BWD_MINB) splat_bwd_tma(RasterParams q, WtConsts fc, const __grid_constant__ CUtensorMap tm_gs,
-                                                                      const __grid_constant__ CUtensorMap tm_go,
-                                                                      const __grid_constant__ CUtensorMap tm_sv,
-                                                                      const __grid_constant__ CUtensorMap tm_ot) {
-    typedef WarpStage<MASK_O ? 2 : 1, true, false, 1> Stage;
-    constexpr int NBUF = (LOSS && SUM_T) ? 4 : 3;
+template <bool SUM, bool SOFTOR, bool SUM_T, bool SAVED>
+__global__ void __launch_bounds__(WB_CTA, BWD_MINB) splat_bwd_tma(RasterParams q, WtConsts fc, const __grid_constant__ CUtensorMap tm_gs,
+                                                                  const __grid_constant__ CUtensorMap tm_go,
+                                                                  const __grid_constant__ CUtensorMap tm_sv) {
+    typedef WarpStage<2, true, false, 1> Stage;
+    constexpr int NBUF = 3;
     extern __shared__ __align__(1024) unsigned char wt_smem_tma[];
     Strip sp;
     if (!strip_init<WB_WARPS>(sp, q)) return;
     const int wid = WB_WARPS == 1 ? 0 : (int)(threadIdx.x >> 5);
-    unsigned char* tin = wt_smem_tma + wid * (NBUF * TMA_TILE_BYTES);            // [go | saved | gs | (LOSS) ot], 1 KB each, 1 KB aligned
+    unsigned char* tin = wt_smem_tma + wid * (NBUF * TMA_TILE_BYTES);            // [go | saved | gs], 1 KB each, 1 KB aligned
     uint64_t* bar = reinterpret_cast<uint64_t*>(wt_smem_tma + WB_WARPS * NBUF * TMA_TILE_BYTES) + wid;
     Stage& st = reinterpret_cast<Stage*>(wt_smem_tma + WB_WARPS * NBUF * TMA_TILE_BYTES + 64)[wid];
     const Entry* entries = q.entries + (size_t)sp.bin * q.cap;
@@ -954,26 +862,16 @@ __global__ void __launch_bounds__(WB_CTA, FFB_BWD_MINB) splat_bwd_tma(RasterPara
     __syncwarp();
     unsigned phase = 0;
     bool have = false;                                      // tile 0 of the current super tile is already in flight
-    constexpr unsigned kBytes = (unsigned)TMA_TILE_BYTES * (LOSS ? (SUM_T ? 4 : 2) : ((SOFTOR ? (SAVED ? 2 : 1) : 0) + (SUM ? 1 : 0)));
-    float lacc = 0.f;                                       // LOSS: this lane's share of sum |softor - sum|
+    constexpr unsigned kBytes = (unsigned)TMA_TILE_BYTES * ((SOFTOR ? (SAVED ? 2 : 1) : 0) + (SUM ? 1 : 0));
     // natural tiles: texel (row 4i + 2h + j, column lc) at float (4i + j) * 16 + nat_off
     const float* nat = reinterpret_cast<const float*>(tin) + (2 * w.h) * WT + w.lc;
     // transposed tile (64-byte swizzle: 16-byte chunk index ^= (column >> 1) & 3): rows 4i + 2h + {0, 1} of column lc
     const unsigned tr_base = (unsigned)(2 * TMA_TILE_BYTES + w.lc * 64 + 8 * w.h), tr_x = (unsigned)((w.lc >> 1) & 3) << 4;
 
     auto issue = [&](int r0, int j) {                      // called by the converged warp
-        if (FFB_TMA_ELECT ? tma::elect_one() : sp.lane == 0) {
+        if (tma::elect_one()) {
             const int ct = w.c0 + WT * j;
             tma::mbar_expect_tx(bar, kBytes);
-            if (LOSS) {
-                tma::load_3d(tin, &tm_go, bar, ct, r0, w.b);
-                tma::load_3d(tin + TMA_TILE_BYTES, &tm_sv, bar, ct, r0, w.b);
-                if (SUM_T) {
-                    tma::load_3d(tin + 2 * TMA_TILE_BYTES, &tm_gs, bar, r0, ct, w.b);
-                    tma::load_3d(tin + 3 * TMA_TILE_BYTES, &tm_ot, bar, r0, ct, w.b);
-                }
-                return;
-            }
             if (SOFTOR) {
                 tma::load_3d(tin, &tm_go, bar, ct, r0, w.b);
                 if (SAVED) tma::load_3d(tin + TMA_TILE_BYTES, &tm_sv, bar, ct, r0, w.b);
@@ -984,11 +882,9 @@ __global__ void __launch_bounds__(WB_CTA, FFB_BWD_MINB) splat_bwd_tma(RasterPara
             }
         }
     };
-    const unsigned inv_bits = __float_as_uint(q.loss_inv);
-    auto sgn = [&](float d) { return sign_times(d, inv_bits); };
-    // dense patterns (or the loss mode, which visits every tile): the first tile's boxes are requested before the list bounds and
-    // the candidate records arrive -- three dependent memory latencies at the head of a warp's life become one
-    if (LOSS || q.eager) {
+    // dense patterns: the first tile's boxes are requested before the list bounds and the candidate records arrive -- three
+    // dependent memory latencies at the head of a warp's life become one
+    if (q.eager) {
         issue(sp.sty0 * WT, 0);
         have = true;
     }
@@ -1004,44 +900,24 @@ __global__ void __launch_bounds__(WB_CTA, FFB_BWD_MINB) splat_bwd_tma(RasterPara
             nn = __shfl_sync(0xffffffffu, sp.tv, 2 * s + 3) - nb;
             prefetch_entries(st.raw[0], entries + nb, nn <= WCH ? nn : 0, sp.lane);
         }
-        const bool next_live = LOSS ? (s + 1 < sp.nst) : (nn > 0 && nn <= WCH);
-        const bool grad = n > 0 && n <= WCH;               // empty: no gradient work; larger lists: overflow kernel
-        if (LOSS || grad) {
+        const bool next_live = nn > 0 && nn <= WCH;
+        if (n > 0 && n <= WCH) {                           // empty: no gradient work; larger lists: overflow kernel
             w.r0 = (sp.sty0 + s) * WT;
             if (!have) issue(w.r0, 0);
-            WtMasks mk;
-            mk.tb01 = mk.tb23 = mk.nb01 = mk.nb23 = 0u;
-            if (grad) mk = stage_regs(st, e, n, w.c0, (float)w.r0, fc, sp.lane);
+            const WtMasks mk = stage_regs(st, e, n, w.c0, (float)w.r0, fc, sp.lane);
 #pragma unroll 1
             for (int j = 0; j < 4; ++j) {
                 float2 gs[4], gp[4];
                 tma::mbar_wait(bar, phase);
                 phase ^= 1u;
-                if (LOSS) {
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        const float2 o = make_float2(nat[(4 * i) * WT], nat[(4 * i + 1) * WT]);
-                        const float2 sm = make_float2(nat[WT * WT + (4 * i) * WT], nat[WT * WT + (4 * i + 1) * WT]);
-                        const float dx_ = o.x - sm.x, dy_ = o.y - sm.y;
-                        lacc += fabsf(dx_) + fabsf(dy_);
-                        const float2 sg = make_float2(sgn(dx_), sgn(dy_));
-                        gp[i] = __fmul2_rn(sg, make_float2(1.f - o.x, 1.f - o.y));
-                        if (SUM_T) {
-                            const float2 st_ = *reinterpret_cast<const float2*>(tin + (tr_base + (tr_x ^ (unsigned)(i << 4))));
-                            const float2 ot_ = *reinterpret_cast<const float2*>(tin + TMA_TILE_BYTES + (tr_base + (tr_x ^ (unsigned)(i << 4))));
-                            gs[i] = make_float2(-sgn(ot_.x - st_.x), -sgn(ot_.y - st_.y));
-                        } else {
-                            gs[i] = neg2(sg);
-                        }
-                    }
-                } else if (SOFTOR) {
+                if (SOFTOR) {
 #pragma unroll
                     for (int i = 0; i < 4; ++i) {
                         gp[i] = make_float2(nat[(4 * i) * WT], nat[(4 * i + 1) * WT]);
                         if (SAVED) gp[i] = __fmul2_rn(gp[i], make_float2(1.f - nat[WT * WT + (4 * i) * WT], 1.f - nat[WT * WT + (4 * i + 1) * WT]));
                     }
                 }
-                if (SUM && !LOSS) {
+                if (SUM) {
 #pragma unroll
                     for (int i = 0; i < 4; ++i) {
                         if (SUM_T) gs[i] = *reinterpret_cast<const float2*>(tin + (tr_base + (tr_x ^ (unsigned)(i << 4))));
@@ -1052,22 +928,19 @@ __global__ void __launch_bounds__(WB_CTA, FFB_BWD_MINB) splat_bwd_tma(RasterPara
                 // next tile (of this super tile, or tile 0 of the next one) in flight while this one is computed
                 if (j < 3) issue(w.r0, j + 1);
                 else if (next_live) issue(w.r0 + WT, 0);
-                if (LOSS && !grad) continue;
                 const unsigned tm = tile_mask(mk, j);
                 const float cf = (float)(w.c0 + WT * j + w.lc);
                 if (SOFTOR && !SAVED) {                    // pass 1 (only without the saved output): per-texel product of (1 - g)
                     float2 prod[4], unused[4];
 #pragma unroll
                     for (int i = 0; i < 4; ++i) prod[i] = bc(1.f);
-                    accumulate_tile<false, true, MASK_O>(st, tm, n, cf, w.h, fc, unused, prod);
+                    accumulate_tile<false, true, true>(st, tm, n, cf, w.h, fc, unused, prod);
 #pragma unroll
                     for (int i = 0; i < 4; ++i) gp[i] = __fmul2_rn(gp[i], prod[i]);
                 }
-                const unsigned nm = near_mask(mk, j);
-                weigh_tile<SUM, SOFTOR, MASK_O, false>(st, (MASK_O || !FFB_BWD_FAR) ? tm : nm, n, cf, w.h, sp.lane, fc, gs, gp);
-                if (!MASK_O && FFB_BWD_FAR) weigh_tile<SUM, SOFTOR, MASK_O, true>(st, tm & ~nm, n, cf, w.h, sp.lane, fc, gs, gp);
+                weigh_tile<SUM, SOFTOR, true, false>(st, tm, n, cf, w.h, sp.lane, fc, gs, gp);
             }
-            if (grad) flush_warp(st, n, w.h, w.lc, kh, dp);
+            flush_warp(st, n, w.h, w.lc, kh, dp);
             have = next_live;
         } else {
             if (have) {                                     // requested eagerly, not needed: let the boxes land before the buffers go away
@@ -1077,10 +950,6 @@ __global__ void __launch_bounds__(WB_CTA, FFB_BWD_MINB) splat_bwd_tma(RasterPara
             have = false;
         }
         n = nn;
-    }
-    if (LOSS) {
-        lacc = warp_sum(lacc);
-        if (sp.lane == 0) atomicAdd(q.loss + sp.b, lacc * q.loss_inv);
     }
 }
 

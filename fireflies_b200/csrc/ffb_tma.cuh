@@ -4,7 +4,6 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 #include <string.h>
 
 namespace ffb {
@@ -82,14 +81,8 @@ inline bool encode_f32_3d(CUtensorMap* map, const float* base, uint64_t d0, uint
     cuuint64_t gstr[2] = {d0 * 4, d0 * d1 * 4};
     cuuint32_t box[3] = {b0, b1, 1};
     cuuint32_t estr[3] = {1, 1, 1};
-    CUtensorMapL2promotion promo = CU_TENSOR_MAP_L2_PROMOTION_L2_128B;
-    if (const char* e = getenv("FFB_TMA_L2")) {           // A/B knob: L2 promotion of the tile boxes (0 / 64 / 128 / 256 bytes)
-        const int v = atoi(e);
-        promo = v == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : v == 64 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
-              : v == 256 ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B : CU_TENSOR_MAP_L2_PROMOTION_L2_128B;
-    }
     return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-               swizzle, promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+               swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
 }  // namespace tma

@@ -92,7 +92,8 @@ class _SplatPlan:
 
     def backward(self, points, g_sum, g_softor, sum_transposed: bool, saved_softor=None, out=None) -> torch.Tensor:
         """``saved_softor``: the forward's soft-OR output (what autograd saves for ``prod``'s backward); the production kernel
-        rebuilds the per-texel product instead (8 instead of 12 B/texel) unless ``FFB_SPLAT_BWD_SAVED=1``.  ``out``: optional
+        rebuilds the per-texel product instead (8 instead of 12 B/texel) and reads it only for soft-OR windows tighter than
+        their no-op radius and for textures the TMA unit cannot describe.  ``out``: optional
         ``[B,N,2]`` tensor to write into."""
         d_pts = out if out is not None else torch.empty((self.B, self.N, 2), dtype=torch.float32, device=points.device)
         nat.check(nat.lib().ffb_splat_bwd(C.byref(self.desc), points.data_ptr(), self.ws.data_ptr(), nat.ptr(g_sum),

@@ -1,6 +1,6 @@
 #!/bin/bash
 # compute-sanitizer over the GPU parity tests: memcheck, racecheck (shared-memory hazards) and synccheck on the parity files (the
-# full-size config-3 case excluded: minutes under the tools); the splat file twice, with the one-shot and the persistent backward.
+# full-size config-3 case excluded: minutes under the tools).
 # Usage: gpurun --timeout 1200 -- bash scripts/gpu_sanitize.sh [tag]
 set -u
 OUT=gpurun_out/${1:-sanitize}
@@ -15,5 +15,3 @@ run() {   # tool, log name, test files, extra env
 run memcheck memcheck "$SMALL tests/test_configs_gpu.py"
 run racecheck racecheck "$SMALL"
 run synccheck synccheck "$SMALL"
-run memcheck memcheck_persistent "tests/test_splat_gpu.py" FFB_SPLAT_BWD_PERSIST=1
-run racecheck racecheck_persistent "tests/test_splat_gpu.py" FFB_SPLAT_BWD_PERSIST=1

@@ -49,10 +49,10 @@ tol = 1e-4 * ref.abs() + 1e-4 * ref.norm(dim=1, keepdim=True)
 def report(name, d):
     e = (d.double() - ref).abs() / tol
     print(f"{name:22s}: max {float(e.max()):.4f}  rms {float((e * e).mean().sqrt()):.4f}  (tolerance units);  rel-to-norm {float((d.double() - ref).norm() / ref.norm()):.3e}")
-variants = [("st rebuild", dict()), ("st rebuild masked", dict(FFB_SPLAT_BWD_MASK="1")), ("st saved", dict(FFB_SPLAT_BWD_SAVED="1")),
-            ("old saved", dict(FFB_SPLAT_BWD_ST="0")), ("old rebuild", dict(FFB_SPLAT_BWD_ST="0", NOSAVED="1")), ("general kernels", dict(GENERAL="1"))]
+variants = [("st rebuild", dict()), ("plain-load saved", dict(FFB_SPLAT_NO_TMA="1")), ("plain-load rebuild", dict(FFB_SPLAT_NO_TMA="1", NOSAVED="1")),
+            ("general kernels", dict(GENERAL="1"))]
 for name, kw in variants:
-    for k in ("FFB_SPLAT_BWD_MASK", "FFB_SPLAT_BWD_SAVED", "FFB_SPLAT_BWD_ST"): os.environ.pop(k, None)
+    os.environ.pop("FFB_SPLAT_NO_TMA", None)
     for k, v in kw.items():
         if k.startswith("FFB"): os.environ[k] = v
     if "GENERAL" in kw:
@@ -63,6 +63,7 @@ for name, kw in variants:
     else:
         d = plan.backward(p1, gS.unsqueeze(0).contiguous(), gO.unsqueeze(0).contiguous(), False, None if "NOSAVED" in kw else O_)[0]
     report(name, d)
+os.environ.pop("FFB_SPLAT_NO_TMA", None)
 # the oracle's own fp32 autograd for scale
 sys.path.insert(0, ".")
 from oracle import ff_oracle as O

@@ -19,47 +19,27 @@ def t(fn, n=3):
     for _ in range(n): fn()
     e1.record(); torch.cuda.synchronize()
     return e0.elapsed_time(e1) / n
-def env(**kw):
-    for k, v in kw.items():
-        if v is None: os.environ.pop(k, None)
-        else: os.environ[k] = v
 hw = ts[0] * ts[1]
 tp = t(lambda: R._SplatPlan(ptsB, B, 100.0, ts[0], ts[1], 4, 5))
 tf = t(lambda: plan.forward(ptsB, True, True, True))
 S_, O_ = plan.forward(ptsB, True, True, True)
 res = {}
-for name, kw in [("st_rebuild", dict(FFB_SPLAT_BWD_ST=None, FFB_SPLAT_BWD_SAVED=None, FFB_SPLAT_BWD_PERSIST="1")),
-                 ("st_oneshot", dict(FFB_SPLAT_BWD_ST=None, FFB_SPLAT_BWD_SAVED=None, FFB_SPLAT_BWD_PERSIST=None)),
-                 ("st_chunk2", dict(FFB_SPLAT_BWD_PERSIST="1", FFB_SPLAT_BWD_CHUNK="2")), ("st_chunk4", dict(FFB_SPLAT_BWD_PERSIST="1", FFB_SPLAT_BWD_CHUNK="4")),
-                 ("st_chunk8", dict(FFB_SPLAT_BWD_PERSIST="1", FFB_SPLAT_BWD_CHUNK="8")),
-                 ("st_saved", dict(FFB_SPLAT_BWD_ST=None, FFB_SPLAT_BWD_SAVED="1", FFB_SPLAT_BWD_PERSIST=None, FFB_SPLAT_BWD_CHUNK=None)),
-                 ("old_saved", dict(FFB_SPLAT_BWD_ST="0", FFB_SPLAT_BWD_SAVED=None)),
-                 ("old_rebuild", dict(FFB_SPLAT_BWD_ST="0", FFB_SPLAT_BWD_SAVED=None))]:
-    env(**kw)
-    sv = None if name == "old_rebuild" else O_
-    tb = t(lambda: plan.backward(ptsB, gS, gO, True, sv))
-    res[name] = (tb, plan.backward(ptsB, gS, gO, True, sv))
+for name, eager in (("st_chunk8", "1"), ("st_oneshot", "0")):
+    os.environ["FFB_SPLAT_EAGER"] = eager
+    tb = t(lambda: plan.backward(ptsB, gS, gO, True, O_))
+    res[name] = (tb, plan.backward(ptsB, gS, gO, True, O_))
     print(f"bwd {name:12s}: {tb:.3f} ms  ({B*8*hw/tb/1e6:.0f} GB/s algorithmic, frac {B*8*hw/tb/1e6/6458.4:.3f})")
-env(FFB_SPLAT_BWD_ST=None, FFB_SPLAT_BWD_SAVED=None)
-ref = res["old_rebuild"][1]
-for k, (_, d) in res.items():
-    print(f"  {k:12s} vs old_rebuild: max|diff| {float((d - ref).abs().max()):.3e} of {float(ref.abs().max()):.3e}; rel-to-norm {float((d - ref).norm() / ref.norm()):.3e}")
+os.environ.pop("FFB_SPLAT_EAGER", None)
+ref = res["st_chunk8"][1]
+d = res["st_oneshot"][1]
+print(f"  st_oneshot vs st_chunk8: max|diff| {float((d - ref).abs().max()):.3e} of {float(ref.abs().max()):.3e}; rel-to-norm {float((d - ref).norm() / ref.norm()):.3e}")
 # natural-layout sum gradient and single-reduction variants
 gSn = gS.transpose(1, 2).contiguous()
 for name, fn in [("nat sum+softor", lambda: plan.backward(ptsB, gSn, gO, False)), ("sum only T", lambda: plan.backward(ptsB, gS, None, True)),
                  ("softor only", lambda: plan.backward(ptsB, None, gO, False))]:
-    env(FFB_SPLAT_BWD_ST=None); tn = t(fn); dn = fn()
-    env(FFB_SPLAT_BWD_ST="0"); to = t(fn); do = fn()
-    env(FFB_SPLAT_BWD_ST=None)
-    print(f"bwd {name:15s}: st {tn:.3f} ms, old {to:.3f} ms; rel diff {float((dn - do).norm() / do.norm()):.3e}")
-for nm_, st_ in (("st", None), ("old", "0")):
-    env(FFB_SPLAT_L1_ST=st_)
-    tl = t(lambda: plan.backward_l1(ptsB, S_, O_, True))
-    ll, dl = plan.backward_l1(ptsB, S_, O_, True)
-    if st_ is None: l_new, d_new = ll, dl
-    print(f"fused L1 backward ({nm_}): {tl:.3f} ms ({B*8*hw/tl/1e6:.0f} GB/s algorithmic)")
-env(FFB_SPLAT_L1_ST=None)
-print(f"  L1 st vs old: loss rel {float((l_new - ll).abs().max() / ll.abs().max()):.2e}, grad rel-to-norm {float((d_new - dl).norm() / dl.norm()):.3e}")
-tb = res["st_rebuild"][0]
+    print(f"bwd {name:15s}: {t(fn):.3f} ms")
+tl = t(lambda: plan.backward_l1(ptsB, S_, O_, True))
+print(f"fused L1 backward (st): {tl:.3f} ms ({B*8*hw/tl/1e6:.0f} GB/s algorithmic)")
+tb = res["st_chunk8"][0]
 print(f"B={B} prepare {tp:.3f} ms  fwd {tf:.3f} ms ({B*8*hw/tf/1e6:.0f} GB/s)  bwd {tb:.3f} ms ({B*8*hw/tb/1e6:.0f} GB/s)"
       f"  fwd+bwd per sample {(tf+tb)/B*1e3:.2f} us -> {B/(tf+tb)*1e3:.0f} samples/s, roofline frac {(B*(16*hw+16*N)/((tp+tf+tb)*1e-3))/6458.4e9:.3f}")

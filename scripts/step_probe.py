@@ -14,7 +14,7 @@ gS = torch.randn(B, 2048, 2048, device=dev); gO = torch.randn(B, 2048, 2048, dev
 scene = bench.build_scene(ff, dev); sb = scene.batch(seed=1)
 step = ff.PatternStep(4096, (2048, 2048), 100.0, B, scene_batch=sb, device=dev)
 def run(tag, rnd, **env):
-    for k in ("FFB_SPLAT_BWD_PERSIST",): os.environ.pop(k, None)
+    os.environ.pop("FFB_SPLAT_EAGER", None)
     os.environ.update(env)
     ms = []
     for i in range(8):
@@ -26,9 +26,9 @@ def run(tag, rnd, **env):
     print(f"{tag:34s} prepare {t[0]:.3f} fwd {t[1]:.3f} bwd {t[2]:.3f} fold {t[3]:.3f} total {t[4]:.3f}")
 run("PatternStep + randomize", True)
 run("PatternStep, no randomize", False)
-run("PatternStep + randomize, one-shot", True, FFB_SPLAT_BWD_PERSIST="0")
-run("PatternStep, no randomize, one-shot", False, FFB_SPLAT_BWD_PERSIST="0")
-os.environ.pop("FFB_SPLAT_BWD_PERSIST", None)
+run("PatternStep + randomize, one-shot", True, FFB_SPLAT_EAGER="0")
+run("PatternStep, no randomize, one-shot", False, FFB_SPLAT_EAGER="0")
+os.environ.pop("FFB_SPLAT_EAGER", None)
 # hand-assembled like the round-1 bench
 ev = lambda: torch.cuda.Event(enable_timing=True)
 for rnd in (True, False):

@@ -15,14 +15,10 @@ for ns, no in ((4, 5), (0, 0), (3, 2)):
         anas = [O.splat_grad_analytic(pts[b], sigma, ts, wS[b] if ws else None, wO[b] if wo else None, ns or None, no or None) for b in range(B)]
         plan = R._SplatPlan(pts.cuda(), B, sigma, ts[0], ts[1], ns, no)
         s, o = plan.forward(pts.cuda(), ws, wo, False)
-        for env in ({}, {"FFB_SPLAT_BWD_ST": "0"}):
-            for k in ("FFB_SPLAT_BWD_ST",): os.environ.pop(k, None)
-            os.environ.update(env)
-            for saved in ((None, o) if wo else (None,)):
-                g = plan.backward(pts.cuda(), wS.cuda() if ws else None, wO.cuda() if wo else None, False, saved).cpu().double()
-                worst = 0.0
-                for b in range(B):
-                    ana = anas[b]; nrm = ana.norm(dim=1, keepdim=True)
-                    worst = max(worst, float(((g[b] - ana).abs() / (1e-4 * ana.abs() + 1e-4 * nrm + 1e-12)).max()))
-                print(f"ns {ns} no {no} sum {int(ws)} softor {int(wo)} {'old' if env else 'st '} saved {saved is not None}: max {worst:.3f} tol units")
-os.environ.pop("FFB_SPLAT_BWD_ST", None)
+        for saved in ((None, o) if wo else (None,)):
+            g = plan.backward(pts.cuda(), wS.cuda() if ws else None, wO.cuda() if wo else None, False, saved).cpu().double()
+            worst = 0.0
+            for b in range(B):
+                ana = anas[b]; nrm = ana.norm(dim=1, keepdim=True)
+                worst = max(worst, float(((g[b] - ana).abs() / (1e-4 * ana.abs() + 1e-4 * nrm + 1e-12)).max()))
+            print(f"ns {ns} no {no} sum {int(ws)} softor {int(wo)} saved {saved is not None}: max {worst:.3f} tol units")

@@ -258,41 +258,38 @@ def test_large_grid_takes_the_banded_binning(R, monkeypatch):
     close(res[0][0][0, r0:r0 + 64, c0:c0 + 64].cpu(), want)
 
 
-def test_saturated_softor_backward(R, monkeypatch):
+def test_saturated_softor_backward(R):
     """220 points inside a 20x20 texel patch at sigma = 100: the soft-OR saturates (prod(1 - g) runs from 1e-40 to 1e-2 across the
-    patch), every super tile overflows.  The production backward rebuilds the product like torch.prod's backward; the earlier
-    generation reads the forward's output back (prod = 1 - O, an fp32 difference that loses the product's bits where O -> 1).  Both
-    against the fp64 closed form, per component."""
+    patch), every super tile overflows.  The production backward rebuilds the product like torch.prod's backward.  A soft-OR window
+    tighter than its no-op radius (num_std 2) takes the round-1 kernel, which reads the forward's output back when it is given
+    (prod = 1 - O, an fp32 difference that loses the product's bits where O -> 1) and rebuilds the product otherwise.  All against
+    the fp64 closed form, per component."""
     gen = torch.Generator().manual_seed(21)
     ts, sigma = [160, 160], 100.0
     pts = torch.cat([(70.0 + 20.0 * torch.rand(220, 2, generator=gen)) / 160.0, torch.rand(24, 2, generator=gen)])
     wS, wO = torch.randn(ts[1], ts[0], generator=gen), torch.randn(ts[1], ts[0], generator=gen)
-    ana = O.splat_grad_analytic(pts, sigma, ts, wS, wO, 4, 5)
-    so = O.baked_softor(pts, sigma, ts)
-    assert float((1 - so).min()) < 1e-6 and float(so.max()) == 1.0            # the case does saturate
-    p1 = pts.cuda().unsqueeze(0).contiguous()
-    plan = R._SplatPlan(p1, 1, sigma, ts[0], ts[1], 4, 5)
-    s, o = plan.forward(p1, True, True, False)
-    close(o[0], so)
     gs, go = wS.cuda().unsqueeze(0).contiguous(), wO.cuda().unsqueeze(0).contiguous()
-    close_grad(plan.backward(p1, gs, go, False, o)[0], ana)                    # production: product rebuilt (saved output ignored)
-    monkeypatch.setenv("FFB_SPLAT_BWD_SAVED", "1")
-    close_grad(plan.backward(p1, gs, go, False, o)[0], ana)                    # super-tile kernel reading 1 - O
-    monkeypatch.setenv("FFB_SPLAT_BWD_ST", "0")
-    close_grad(plan.backward(p1, gs, go, False, o)[0], ana)                    # earlier generation, saved output
-    close_grad(plan.backward(p1, gs, go, False)[0], ana)                       # earlier generation, product rebuilt
+    p1 = pts.cuda().unsqueeze(0).contiguous()
+    for no in (5, 2):                                                          # exact soft-OR window / masked (round-1 kernel)
+        ana = O.splat_grad_analytic(pts, sigma, ts, wS, wO, 4, no)
+        so = O.baked_softor(pts, sigma, ts, num_std=no)
+        assert float((1 - so).min()) < 1e-6 and float(so.max()) == 1.0        # the case does saturate
+        plan = R._SplatPlan(p1, 1, sigma, ts[0], ts[1], 4, no)
+        s, o = plan.forward(p1, True, True, False)
+        close(o[0], so)
+        close_grad(plan.backward(p1, gs, go, False, o)[0], ana)                # saved output (ignored by the production kernel)
+        close_grad(plan.backward(p1, gs, go, False)[0], ana)                   # product rebuilt
     # a milder pattern where no list overflows (the main kernels, not the overflow kernels, see the saturation)
-    monkeypatch.delenv("FFB_SPLAT_BWD_SAVED"); monkeypatch.delenv("FFB_SPLAT_BWD_ST")
     gen = torch.Generator().manual_seed(22)
     pts2 = torch.cat([(40.0 + 80.0 * torch.rand(14, 2, generator=gen)) / 160.0 for _ in range(1)] + [(78.0 + 4.0 * torch.rand(2, 2, generator=gen)) / 160.0])
     pts2 = torch.cat([pts2, pts2[:8] + 0.004])                                 # near-coincident pairs: 1 - g small where it matters
-    ana2 = O.splat_grad_analytic(pts2, 400.0, ts, wS, wO, 4, 5)
     q1 = pts2.cuda().unsqueeze(0).contiguous()
-    plan2 = R._SplatPlan(q1, 1, 400.0, ts[0], ts[1], 4, 5)
-    _, o2 = plan2.forward(q1, True, True, False)
-    close_grad(plan2.backward(q1, gs, go, False, o2)[0], ana2)
-    monkeypatch.setenv("FFB_SPLAT_BWD_ST", "0")
-    close_grad(plan2.backward(q1, gs, go, False, o2)[0], ana2)
+    for no in (5, 2):
+        ana2 = O.splat_grad_analytic(pts2, 400.0, ts, wS, wO, 4, no)
+        plan2 = R._SplatPlan(q1, 1, 400.0, ts[0], ts[1], 4, no)
+        _, o2 = plan2.forward(q1, True, True, False)
+        close_grad(plan2.backward(q1, gs, go, False, o2)[0], ana2)
+        close_grad(plan2.backward(q1, gs, go, False)[0], ana2)
 
 
 def test_batched_and_shared_patterns(R):
@@ -455,14 +452,14 @@ def test_tma_and_plain_kernels_agree(R, monkeypatch):
 
 
 def test_backward_launch_forms(R, monkeypatch):
-    """The dense-pattern backward has three launch forms of one item loop: chunks of consecutive items per CTA (default 8; 7 leaves a
-    ragged last chunk of the 128 items), resident warps with a work counter, one CTA per item.  Each against the fp64 closed form,
-    with given upstream gradients and through the fused L1 loss."""
+    """The super-tile backward has two launch forms for given upstream gradients: chunks of 8 consecutive items per one-warp CTA
+    (dense patterns, FFB_SPLAT_EAGER=1; 5 x 17 super tiles x 2 samples = 170 items leave a ragged last chunk) and one CTA per item
+    (sparse patterns, FFB_SPLAT_EAGER=0).  The fused L1 loss mode always takes a third: resident warps claiming items from a work
+    counter.  Each against the fp64 closed form."""
     gen = torch.Generator().manual_seed(77)
-    B, ts, sigma = 2, [256, 256], 49.0
+    B, ts, sigma = 2, [260, 260], 49.0
     pts = (torch.rand(B, 120, 2, generator=gen) * 0.96 + 0.02)
     gS, gO = torch.randn(B, ts[0], ts[1], generator=gen), torch.randn(B, ts[1], ts[0], generator=gen)
-    monkeypatch.setenv("FFB_SPLAT_EAGER", "1")            # dense-pattern path whatever the density heuristic says
     plan = R._SplatPlan(pts.cuda(), B, sigma, ts[0], ts[1], 4, 5)
     s, o = plan.forward(pts.cuda(), True, True, True)
     ana, ana_l1, loss_ref = [], [], []
@@ -472,11 +469,8 @@ def test_backward_launch_forms(R, monkeypatch):
         sg = torch.sign(diff) / diff.numel()
         ana_l1.append(O.splat_grad_analytic(pts[b], sigma, ts, (-sg).T, sg, 4, 5))
         loss_ref.append(diff.abs().double().mean())
-    for form in ({}, {"FFB_SPLAT_BWD_CHUNK": "7"}, {"FFB_SPLAT_BWD_PERSIST": "1"}, {"FFB_SPLAT_BWD_PERSIST": "0"}):
-        for k in ("FFB_SPLAT_BWD_CHUNK", "FFB_SPLAT_BWD_PERSIST"):
-            monkeypatch.delenv(k, raising=False)
-        for k, v in form.items():
-            monkeypatch.setenv(k, v)
+    for eager in ("1", "0"):
+        monkeypatch.setenv("FFB_SPLAT_EAGER", eager)       # whatever the density heuristic says
         d = plan.backward(pts.cuda(), gS.cuda(), gO.cuda(), True).cpu()
         fused = plan.backward_l1(pts.cuda(), s, o, True)
         assert fused is not None
@@ -498,7 +492,9 @@ def test_every_kernel_variant(R, want, sum_t):
     wS = torch.randn(B, ts[0], ts[1], generator=gen) if sum_t else torch.randn(B, ts[1], ts[0], generator=gen)
     wO = torch.randn(B, ts[1], ts[0], generator=gen)
     ws, wo = "sum" in want, "softor" in want
-    for ns, no in ((4, 5), (0, 0), (3, 2)):                # baked footprints / dense semantics / a soft-OR window tighter than its no-op radius (MASK_O kernels)
+    # baked footprints / dense semantics / a soft-OR window tighter than its no-op radius (MASK_O kernels) / a sum window whose truncation
+    # matters (MSK super-tile kernels; also the sum-only backward of (3, 2))
+    for ns, no in ((4, 5), (0, 0), (3, 2), (3, 5)):
         plan = R._SplatPlan(pts.cuda(), B, sigma, ts[0], ts[1], ns, no)
         s, o = plan.forward(pts.cuda(), ws, wo, sum_t)
         grads = []
