@@ -7,13 +7,15 @@
 //   + the torch autograd of those w.r.t. `points`.
 //
 // Design (HBM-bound gather, no tensor cores -- nothing here is a contraction):
-//   * prepare: one CTA per sample bins its N points into texture tiles (count / scan / fill in shared
-//     memory, lists sorted so accumulation order is deterministic) and writes one 32-byte record per
-//     point: scaled position + the integer clip windows of both reductions.  Two tilings: 16x16 warp
-//     tiles with 16-byte list entries for the warp-tile kernels (ffb_splat_wt.cuh, the production path
-//     whenever the texture is larger than the footprints), 64x32 CTA tiles with index lists for the
-//     general kernels below (textures smaller than a footprint, where the reference's slice clipping
-//     is not a plain intersection).
+//   * prepare: one CTA per sample bins its N points into texture tiles, lists sorted by point index so
+//     accumulation order is deterministic.  Two tilings: 64x16 super tiles with 32-byte list entries for
+//     the warp-tile kernels (ffb_splat_wt.cuh, the production path whenever the texture is larger than
+//     the footprints), 64x32 CTA tiles with index lists for the general kernels below (textures smaller
+//     than a footprint, where the reference's slice clipping is not a plain intersection).  The
+//     warp-tile path bins with the one-pass kernel (slot lists and records in shared memory; the whole
+//     grid at once or in bands of tile rows); count / scan / fill with one 32-byte record per point in
+//     the workspace (scaled position + the integer clip windows of both reductions) is its form for
+//     large N and the general path's only form.
 //   * general forward: one CTA per (tile, sample).  Each warp owns 8 rows x 32 columns, a lane owns one column
 //     (8 texels in registers).  Candidate records are staged in shared memory; rows outside a point's
 //     window are skipped with warp-uniform branches, so only the column overhang is wasted work.  Every
@@ -252,28 +254,76 @@ __device__ __forceinline__ PointRec make_rec(const PrepParams& q, float x, float
 }
 
 // window origin of the warp-tile kernels' Chebyshev masks along one axis: the reference's (unclipped) slice start
-// floor(P - half) plus half for a baked window (rasterization.py:186), floor(P) otherwise; clamped to int16.
-__device__ __forceinline__ int origin_axis(float P, int baked, int half) {
-    const float fo = floorf(baked ? P - (float)half : P);
-    if (!(fo > -30000.f && fo < 30000.f)) return fo > 0.f ? 32767 : -32768;
-    return (int)fo + (baked ? half : 0);
-}
-
-// the same value as a float without the integer round trip (|result| < 2^24: fo + half is exact); seven instructions instead of ~25,
-// which mattered where every lane of the one-pass kernel's emit loop evaluates it twice per super tile
+// floor(P - half) plus half for a baked window (rasterization.py:186), floor(P) otherwise; clamped to int16.  Integer valued and
+// exact in fp32 (|result| < 2^24).
 __device__ __forceinline__ float origin_axis_f(float P, int baked, int half) {
     const float fo = floorf(baked ? P - (float)half : P);
     if (!(fo > -30000.f && fo < 30000.f)) return fo > 0.f ? 32767.f : -32768.f;
     return baked ? fo + (float)half : fo;
 }
 
-// One CTA per binned pattern instance.  FAST: 64x16 super tiles, 32-byte entries; otherwise 64x32 CTA tiles,
-// index lists.  The tile grid is processed in bands of whole tile rows so that the
-// counters fit in shared memory for any texture size.
-// SREC (FAST only): the point records live in shared memory instead of the workspace -- only this kernel reads them in the fast
-// path (a list entry is a copy of its record), and the random 32-byte record reads of the emit phase were the kernel's
-// long-scoreboard stalls (profiles/r01n: issue 41 %, long scoreboard 51 % of the stall samples)
-template <bool FAST, bool SREC = false>
+// list entry {p0, p1, f0, f1 | ur, uc, idx, 0} as two 128-bit stores
+__device__ __forceinline__ void store_entry(Entry* dst, float p0, float p1, uint32_t ur, uint32_t uc, unsigned idx, int baked, int half) {
+    uint4* d = reinterpret_cast<uint4*>(dst);
+    d[0] = make_uint4(__float_as_uint(p0), __float_as_uint(p1), __float_as_uint(origin_axis_f(p0, baked, half)),
+                      __float_as_uint(origin_axis_f(p1, baked, half)));
+    d[1] = make_uint4(ur, uc, idx, 0u);
+}
+
+// the reference's slice triples of point n ([Bp][N][2][2][3])
+__device__ __forceinline__ void store_windows(const PrepParams& q, int bin, int n, const int (&win)[12]) {
+    int* w = q.windows + ((size_t)bin * q.N + n) * 12;
+#pragma unroll
+    for (int k = 0; k < 12; ++k) w[k] = win[k];
+}
+
+// Batcher's odd-even merge sort on 16 registers (63 compare-exchanges, 0-1 principle checked exhaustively): a quarter of the
+// instructions of ranking by counting; empty slots (INT_MAX) sink to the end
+__device__ __forceinline__ void sort16(int (&l)[16]) {
+#define FFB_CE(a, c) { const int lo_ = min(l[a], l[c]), hi_ = max(l[a], l[c]); l[a] = lo_; l[c] = hi_; }
+    FFB_CE(0,1) FFB_CE(2,3) FFB_CE(0,2) FFB_CE(1,3) FFB_CE(1,2) FFB_CE(4,5) FFB_CE(6,7) FFB_CE(4,6) FFB_CE(5,7) FFB_CE(5,6)
+    FFB_CE(0,4) FFB_CE(2,6) FFB_CE(2,4) FFB_CE(1,5) FFB_CE(3,7) FFB_CE(3,5) FFB_CE(1,2) FFB_CE(3,4) FFB_CE(5,6)
+    FFB_CE(8,9) FFB_CE(10,11) FFB_CE(8,10) FFB_CE(9,11) FFB_CE(9,10) FFB_CE(12,13) FFB_CE(14,15) FFB_CE(12,14) FFB_CE(13,15) FFB_CE(13,14)
+    FFB_CE(8,12) FFB_CE(10,14) FFB_CE(10,12) FFB_CE(9,13) FFB_CE(11,15) FFB_CE(11,13) FFB_CE(9,10) FFB_CE(11,12) FFB_CE(13,14)
+    FFB_CE(0,8) FFB_CE(4,12) FFB_CE(4,8) FFB_CE(2,10) FFB_CE(6,14) FFB_CE(6,10) FFB_CE(2,4) FFB_CE(6,8) FFB_CE(10,12)
+    FFB_CE(1,9) FFB_CE(5,13) FFB_CE(5,9) FFB_CE(3,11) FFB_CE(7,15) FFB_CE(7,11) FFB_CE(3,5) FFB_CE(7,9) FFB_CE(11,13)
+    FFB_CE(1,2) FFB_CE(3,4) FFB_CE(5,6) FFB_CE(7,8) FFB_CE(9,10) FFB_CE(11,12) FFB_CE(13,14)
+#undef FFB_CE
+}
+
+// exclusive scan of cnt[0, nt) by the whole CTA (two levels of warp shuffles): thread tid owns [beg, end) and gets base plus the
+// counts before beg.  base is read after the scan's barriers.
+__device__ __forceinline__ int block_exclusive_scan(const int* cnt, int nt, int* warp_tot, const int& base, int& beg, int& end) {
+    const int tid = threadIdx.x;
+    const int per = (nt + PREP_CTA - 1) / PREP_CTA;
+    beg = min(tid * per, nt); end = min(beg + per, nt);
+    int local = 0;
+    for (int i = beg; i < end; ++i) local += cnt[i];
+    int incl = local;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        int v = __shfl_up_sync(0xffffffffu, incl, o);
+        if ((tid & 31) >= o) incl += v;
+    }
+    if ((tid & 31) == 31) warp_tot[tid >> 5] = incl;
+    __syncthreads();
+    if (tid < 32) {
+        int v = warp_tot[tid], sc = v;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            int t = __shfl_up_sync(0xffffffffu, sc, o);
+            if (tid >= o) sc += t;
+        }
+        warp_tot[tid] = sc - v;
+    }
+    __syncthreads();
+    return base + warp_tot[tid >> 5] + incl - local;
+}
+
+// One CTA per binned pattern instance: count / scan / fill with the records in the workspace.  FAST: 64x16 super tiles, 32-byte
+// entries (what the warp-tile path runs when the one-pass kernel's shared arrays do not fit); otherwise 64x32 CTA tiles, index
+// lists.  The tile grid is processed in bands of whole tile rows so that the counters fit in shared memory for any texture size.
+template <bool FAST>
 __global__ void __launch_bounds__(PREP_CTA, PREP_MINB) prepare_kernel(PrepParams q) {
     extern __shared__ __align__(16) int sm[];
     const int band_tiles = q.band_rows * q.tgx;
@@ -283,31 +333,19 @@ __global__ void __launch_bounds__(PREP_CTA, PREP_MINB) prepare_kernel(PrepParams
     __shared__ int band_base;
     const int bin = blockIdx.x, tid = threadIdx.x;
     const float* pts = q.pts + (long long)bin * q.stride;
-    PointRec* recs = SREC ? reinterpret_cast<PointRec*>(sm + ((2 * band_tiles + 3) & ~3)) : q.recs + (size_t)bin * q.N;
+    PointRec* recs = q.recs + (size_t)bin * q.N;
     int* tile_off = q.tile_off + (size_t)bin * (q.T + 1);
     int* list = q.list + (size_t)bin * q.cap;          // FAST: unsorted scratch; otherwise the final index lists
     Entry* entries = q.entries + (FAST ? (size_t)bin * q.cap : 0);
+    const bool bs = q.baked_s != 0;
+    const int baked = (bs || !q.baked_o) ? (int)bs : 1, half = (bs || !q.baked_o) ? q.half_s : q.half_o;
 
     // records (+ the reference's slice triples)
     for (int n = tid; n < q.N; n += PREP_CTA) {
         const float2 xy = reinterpret_cast<const float2*>(pts)[n];
         int win[12];
-        PointRec rec = make_rec(q, xy.x, xy.y, q.windows ? win : nullptr);
-        if (FAST) {
-            // the warp-tile kernels need {p0, p1, window origin, union spans}: keep exactly that in the record's first 24 bytes
-            // (the reduction windows sc / sr / oc / orow are only read by the general kernels), so a list entry is a copy
-            const bool bs = q.baked_s != 0;
-            const int baked = (bs || !q.baked_o) ? (int)bs : 1, half = (bs || !q.baked_o) ? q.half_s : q.half_o;
-            rec.sc = __float_as_uint((float)origin_axis(rec.p0, baked, half));
-            rec.sr = __float_as_uint((float)origin_axis(rec.p1, baked, half));
-            rec.oc = rec.ur; rec.orow = rec.uc;
-        }
-        recs[n] = rec;
-        if (q.windows) {
-            int* w = q.windows + ((size_t)bin * q.N + n) * 12;
-#pragma unroll
-            for (int k = 0; k < 12; ++k) w[k] = win[k];
-        }
+        recs[n] = make_rec(q, xy.x, xy.y, q.windows ? win : nullptr);
+        if (q.windows) store_windows(q, bin, n, win);
     }
     if (tid == 0) band_base = 0;
     __syncthreads();
@@ -329,30 +367,8 @@ __global__ void __launch_bounds__(PREP_CTA, PREP_MINB) prepare_kernel(PrepParams
         }
         __syncthreads();
         // 2. exclusive scan over the band's tiles
-        const int per = (nt + PREP_CTA - 1) / PREP_CTA;
-        const int beg = min(tid * per, nt), end = min(beg + per, nt);
-        int local = 0;
-        for (int i = beg; i < end; ++i) local += cnt[i];
-        int incl = local;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            int v = __shfl_up_sync(0xffffffffu, incl, o);
-            if ((tid & 31) >= o) incl += v;
-        }
-        if ((tid & 31) == 31) warp_tot[tid >> 5] = incl;
-        __syncthreads();
-        if (tid < 32) {
-            int v = warp_tot[tid], sc = v;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                int t = __shfl_up_sync(0xffffffffu, sc, o);
-                if (tid >= o) sc += t;
-            }
-            warp_tot[tid] = sc - v;     // exclusive
-        }
-        __syncthreads();
-        const int base0 = band_base;
-        int run = base0 + warp_tot[tid >> 5] + incl - local;
+        int beg, end;
+        int run = block_exclusive_scan(cnt, nt, warp_tot, band_base, beg, end);
         for (int i = beg; i < end; ++i) {
             const int c = cnt[i];
             cnt[i] = run; cur[i] = run; tile_off[t0 + i] = run;
@@ -380,29 +396,16 @@ __global__ void __launch_bounds__(PREP_CTA, PREP_MINB) prepare_kernel(PrepParams
             const int b = cnt[t], e = min(cur[t], q.cap);
             if (FAST && e - b <= WCH) {
                 // the common case: the whole list in registers (one load per element instead of one per comparison -- the
-                // per-lane scattered re-reads were the kernel's L1 wavefront budget), rank by counting, entries written in order
+                // per-lane scattered re-reads were the kernel's L1 wavefront budget), sorted there, entries written in order
                 int l[16];
 #pragma unroll
                 for (int i = 0; i < 16; ++i) l[i] = (i < WCH && b + i < e) ? list[b + i] : 0x7fffffff;
-                // Batcher's odd-even merge sort on the 16 registers (63 compare-exchanges, 0-1 principle checked exhaustively):
-                // a quarter of the instructions of ranking by counting; empty slots (INT_MAX) sink to the end
-#define FFB_CE(a, c) { const int lo_ = min(l[a], l[c]), hi_ = max(l[a], l[c]); l[a] = lo_; l[c] = hi_; }
-                FFB_CE(0,1) FFB_CE(2,3) FFB_CE(0,2) FFB_CE(1,3) FFB_CE(1,2) FFB_CE(4,5) FFB_CE(6,7) FFB_CE(4,6) FFB_CE(5,7) FFB_CE(5,6)
-                FFB_CE(0,4) FFB_CE(2,6) FFB_CE(2,4) FFB_CE(1,5) FFB_CE(3,7) FFB_CE(3,5) FFB_CE(1,2) FFB_CE(3,4) FFB_CE(5,6)
-                FFB_CE(8,9) FFB_CE(10,11) FFB_CE(8,10) FFB_CE(9,11) FFB_CE(9,10) FFB_CE(12,13) FFB_CE(14,15) FFB_CE(12,14) FFB_CE(13,15) FFB_CE(13,14)
-                FFB_CE(8,12) FFB_CE(10,14) FFB_CE(10,12) FFB_CE(9,13) FFB_CE(11,15) FFB_CE(11,13) FFB_CE(9,10) FFB_CE(11,12) FFB_CE(13,14)
-                FFB_CE(0,8) FFB_CE(4,12) FFB_CE(4,8) FFB_CE(2,10) FFB_CE(6,14) FFB_CE(6,10) FFB_CE(2,4) FFB_CE(6,8) FFB_CE(10,12)
-                FFB_CE(1,9) FFB_CE(5,13) FFB_CE(5,9) FFB_CE(3,11) FFB_CE(7,15) FFB_CE(7,11) FFB_CE(3,5) FFB_CE(7,9) FFB_CE(11,13)
-                FFB_CE(1,2) FFB_CE(3,4) FFB_CE(5,6) FFB_CE(7,8) FFB_CE(9,10) FFB_CE(11,12) FFB_CE(13,14)
-#undef FFB_CE
+                sort16(l);
 #pragma unroll
                 for (int i = 0; i < WCH; ++i) {
-                    if (b + i < e) {                          // entry = {p0, p1, f0, f1 | ur, uc, idx, 0}: two 128-bit words of the record
-                        const uint4* r = reinterpret_cast<const uint4*>(recs + l[i]);
-                        const uint4 a = r[0], c = r[1];
-                        uint4* dst = reinterpret_cast<uint4*>(entries + b + i);
-                        dst[0] = a;
-                        dst[1] = make_uint4(c.x, c.y, (unsigned)l[i], 0u);
+                    if (b + i < e) {
+                        const PointRec& r = recs[l[i]];
+                        store_entry(entries + b + i, r.p0, r.p1, r.ur, r.uc, (unsigned)l[i], baked, half);
                     }
                 }
             } else if (FAST) {
@@ -411,11 +414,8 @@ __global__ void __launch_bounds__(PREP_CTA, PREP_MINB) prepare_kernel(PrepParams
                     const int v = list[i];
                     int rank = 0;
                     for (int j = b; j < e; ++j) rank += list[j] < v;
-                    const uint4* r = reinterpret_cast<const uint4*>(recs + v);
-                    const uint4 a = r[0], c = r[1];
-                    uint4* dst = reinterpret_cast<uint4*>(entries + b + rank);
-                    dst[0] = a;
-                    dst[1] = make_uint4(c.x, c.y, (unsigned)v, 0u);
+                    const PointRec& r = recs[v];
+                    store_entry(entries + b + rank, r.p0, r.p1, r.ur, r.uc, (unsigned)v, baked, half);
                 }
             } else {
                 for (int i = b + 1; i < e; ++i) {
@@ -471,11 +471,7 @@ __global__ void __maxnreg__(48) prepare_onepass_kernel(PrepParams q) {
         const PointRec rec = make_rec(q, xy.x, xy.y, q.windows ? win : nullptr);
         const Rec16 r = Rec16{rec.p0, rec.p1, rec.ur, rec.uc};
         recs[n] = r;
-        if (q.windows) {
-            int* w = q.windows + ((size_t)bin * q.N + n) * 12;
-#pragma unroll
-            for (int k = 0; k < 12; ++k) w[k] = win[k];
-        }
+        if (q.windows) store_windows(q, bin, n, win);
         return r;
     };
     if (BANDED)
@@ -506,29 +502,8 @@ __global__ void __maxnreg__(48) prepare_onepass_kernel(PrepParams q) {
         }
         __syncthreads();
         // 2. exclusive scan over the band's super tiles
-        const int per = (nt + PREP_CTA - 1) / PREP_CTA;
-        const int beg = min(tid * per, nt), end = min(beg + per, nt);
-        int local = 0;
-        for (int i = beg; i < end; ++i) local += cnt[i];
-        int incl = local;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            int v = __shfl_up_sync(0xffffffffu, incl, o);
-            if ((tid & 31) >= o) incl += v;
-        }
-        if ((tid & 31) == 31) warp_tot[tid >> 5] = incl;
-        __syncthreads();
-        if (tid < 32) {
-            int v = warp_tot[tid], sc = v;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                int t = __shfl_up_sync(0xffffffffu, sc, o);
-                if (tid >= o) sc += t;
-            }
-            warp_tot[tid] = sc - v;
-        }
-        __syncthreads();
-        int run = band_base + warp_tot[tid >> 5] + incl - local;
+        int beg, end;
+        int run = block_exclusive_scan(cnt, nt, warp_tot, band_base, beg, end);
         for (int i = beg; i < end; ++i) {
             const int c = cnt[i];
             off[i] = run; tile_off[t0 + i] = run;
@@ -571,10 +546,7 @@ __global__ void __maxnreg__(48) prepare_onepass_kernel(PrepParams q) {
                     int rank = 0;
                     for (int j = b; j < e; ++j) rank += list[j] < v;
                     const Rec16 r = recs[v];
-                    uint4* dst = reinterpret_cast<uint4*>(entries + b + rank);
-                    dst[0] = make_uint4(__float_as_uint(r.p0), __float_as_uint(r.p1), __float_as_uint(origin_axis_f(r.p0, baked, half)),
-                                        __float_as_uint(origin_axis_f(r.p1, baked, half)));
-                    dst[1] = make_uint4(r.ur, r.uc, (unsigned)v, 0u);
+                    store_entry(entries + b + rank, r.p0, r.p1, r.ur, r.uc, (unsigned)v, baked, half);
                 }
             } else if (c > 1) {
                 uint4* row = reinterpret_cast<uint4*>(slot + t * WCH);
@@ -583,16 +555,7 @@ __global__ void __maxnreg__(48) prepare_onepass_kernel(PrepParams q) {
                 int l[16];
 #pragma unroll
                 for (int i = 0; i < 16; ++i) l[i] = i < c ? (int)((w[i >> 1] >> (16 * (i & 1))) & 0xffffu) : 0x7fffffff;
-                // Batcher's odd-even merge sort on the 16 registers (63 compare-exchanges); empty slots (INT_MAX) sink to the end
-#define FFB_CE(a, c_) { const int lo_ = min(l[a], l[c_]), hi_ = max(l[a], l[c_]); l[a] = lo_; l[c_] = hi_; }
-            FFB_CE(0,1) FFB_CE(2,3) FFB_CE(0,2) FFB_CE(1,3) FFB_CE(1,2) FFB_CE(4,5) FFB_CE(6,7) FFB_CE(4,6) FFB_CE(5,7) FFB_CE(5,6)
-            FFB_CE(0,4) FFB_CE(2,6) FFB_CE(2,4) FFB_CE(1,5) FFB_CE(3,7) FFB_CE(3,5) FFB_CE(1,2) FFB_CE(3,4) FFB_CE(5,6)
-            FFB_CE(8,9) FFB_CE(10,11) FFB_CE(8,10) FFB_CE(9,11) FFB_CE(9,10) FFB_CE(12,13) FFB_CE(14,15) FFB_CE(12,14) FFB_CE(13,15) FFB_CE(13,14)
-            FFB_CE(8,12) FFB_CE(10,14) FFB_CE(10,12) FFB_CE(9,13) FFB_CE(11,15) FFB_CE(11,13) FFB_CE(9,10) FFB_CE(11,12) FFB_CE(13,14)
-            FFB_CE(0,8) FFB_CE(4,12) FFB_CE(4,8) FFB_CE(2,10) FFB_CE(6,14) FFB_CE(6,10) FFB_CE(2,4) FFB_CE(6,8) FFB_CE(10,12)
-            FFB_CE(1,9) FFB_CE(5,13) FFB_CE(5,9) FFB_CE(3,11) FFB_CE(7,15) FFB_CE(7,11) FFB_CE(3,5) FFB_CE(7,9) FFB_CE(11,13)
-            FFB_CE(1,2) FFB_CE(3,4) FFB_CE(5,6) FFB_CE(7,8) FFB_CE(9,10) FFB_CE(11,12) FFB_CE(13,14)
-#undef FFB_CE
+                sort16(l);
                 unsigned o[8];
 #pragma unroll
                 for (int i = 0; i < 8; ++i) o[i] = ((unsigned)l[2 * i] & 0xffffu) | ((unsigned)l[2 * i + 1] << 16);
@@ -601,7 +564,7 @@ __global__ void __maxnreg__(48) prepare_onepass_kernel(PrepParams q) {
             }
         }
         __syncthreads();
-        // 5. entries {p0, p1, f0, f1 | ur, uc, idx, 0}: two super tiles per warp step, lane (hp, i) writes entry i of super tile t + hp --
+        // 5. entries: two super tiles per warp step, lane (hp, i) writes entry i of super tile t + hp --
         // 32 contiguous bytes per lane, one contiguous run per warp (consecutive super tiles are consecutive in the entry array)
         const int lane = tid & 31, wid = tid >> 5, i = lane & 15, hp = lane >> 4;
         const int tiles_per_warp = (((nt + 31) / 32) + 1) & ~1;
@@ -612,10 +575,7 @@ __global__ void __maxnreg__(48) prepare_onepass_kernel(PrepParams q) {
             if (c <= WCH && i < c && b + i < q.cap) {
                 const unsigned idx = slot[t * WCH + i];
                 const Rec16 r = recs[idx];
-                uint4* dst = reinterpret_cast<uint4*>(entries + b + i);
-                dst[0] = make_uint4(__float_as_uint(r.p0), __float_as_uint(r.p1), __float_as_uint(origin_axis_f(r.p0, baked, half)),
-                                    __float_as_uint(origin_axis_f(r.p1, baked, half)));
-                dst[1] = make_uint4(r.ur, r.uc, idx, 0u);
+                store_entry(entries + b + i, r.p0, r.p1, r.ur, r.uc, idx, baked, half);
             }
         }
         if (BANDED) __syncthreads();                               // the next band reuses the shared arrays
@@ -1327,43 +1287,35 @@ extern "C" int ffb_splat_prepare(const ffb_splat_desc* d, const float* pts, void
     const size_t smem = (size_t)p.band_rows * p.tgx * 2 * sizeof(int);
     if (p.fast) {
         FFB_CUDA(cudaMemsetAsync(q.ovf, 0, sizeof(int), as_stream(stream)));
-        {
-            // one-pass form: one shared-memory atomic per (point, super tile) pair instead of two.  Whole grid at once when it fits
-            // (config 3: 4096 super tiles + 4096 records = 224 KB), otherwise in bands of tile rows.
-            auto smem_for = [&](size_t tiles) {
-                return ((tiles * 2 + 3) & ~(size_t)3) * sizeof(int) + tiles * WCH * sizeof(unsigned short) + (size_t)d->N * sizeof(Rec16);
-            };
-            const size_t budget = 226 * 1024;
-            const char* e1 = getenv("FFB_PREP_ONEPASS");
-            const bool on = !(e1 && e1[0] == '0') && d->N <= 65535;
-            const char* eb = getenv("FFB_PREP_BAND_ROWS");      // tests: force the banded kernel with this many tile rows per band
-            if (on && !eb && smem_for((size_t)p.T) <= budget) {
-                const size_t sm1 = smem_for((size_t)p.T);
+        // one-pass binning (uint16 slots, so N <= 65535): whole grid at once when it fits (config 3: 4096 super tiles + 4096
+        // records = 224 KB), otherwise in bands of tile rows.  When not even one tile row fits (about 14,400 points), count / scan /
+        // fill with the records in the workspace.
+        auto smem_for = [&](int rows) {
+            const size_t tiles = (size_t)rows * p.tgx;
+            return ((tiles * 2 + 3) & ~(size_t)3) * sizeof(int) + tiles * WCH * sizeof(unsigned short) + (size_t)d->N * sizeof(Rec16);
+        };
+        const size_t budget = 226 * 1024;
+        if (d->N <= 65535 && smem_for(1) <= budget) {
+            const char* eb = getenv("FFB_PREP_BAND_ROWS");      // tests: bin in bands of this many tile rows (at most what fits)
+            const int forced = eb ? atoi(eb) : 0;
+            if (forced <= 0 && smem_for(p.tgy) <= budget) {
+                const size_t sm1 = smem_for(p.tgy);
                 FFB_CUDA(cudaFuncSetAttribute(prepare_onepass_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm1));
                 prepare_onepass_kernel<false><<<p.Bp, PREP_CTA, sm1, as_stream(stream)>>>(q);
                 FFB_CUDA(cudaGetLastError());
                 return 0;
             }
-            if (on && smem_for((size_t)p.tgx) <= budget) {
-                int rows = p.tgy;
-                while (rows > 1 && smem_for((size_t)rows * p.tgx) > budget) rows = (rows + 1) / 2;
-                if (eb && atoi(eb) > 0) rows = atoi(eb) < p.tgy ? atoi(eb) : p.tgy;
-                if (smem_for((size_t)rows * p.tgx) <= budget) {
-                    q.band_rows = rows;
-                    const size_t smb = smem_for((size_t)rows * p.tgx);
-                    FFB_CUDA(cudaFuncSetAttribute(prepare_onepass_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smb));
-                    prepare_onepass_kernel<true><<<p.Bp, PREP_CTA, smb, as_stream(stream)>>>(q);
-                    FFB_CUDA(cudaGetLastError());
-                    return 0;
-                }
-                q.band_rows = p.band_rows;
+            int rows = p.tgy;
+            if (forced > 0) {
+                rows = forced < p.tgy ? forced : p.tgy;
+                while (smem_for(rows) > budget) --rows;
+            } else {
+                while (smem_for(rows) > budget) rows = (rows + 1) / 2;
             }
-        }
-        const size_t smem_rec = (((size_t)p.band_rows * p.tgx * 2 + 3) & ~(size_t)3) * sizeof(int) + (size_t)d->N * sizeof(PointRec);
-        const char* e = getenv("FFB_PREP_SREC");
-        if (smem_rec <= 200 * 1024 && !(e && e[0] == '0')) {        // records in shared memory
-            FFB_CUDA(cudaFuncSetAttribute(prepare_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_rec));
-            prepare_kernel<true, true><<<p.Bp, PREP_CTA, smem_rec, as_stream(stream)>>>(q);
+            q.band_rows = rows;
+            const size_t smb = smem_for(rows);
+            FFB_CUDA(cudaFuncSetAttribute(prepare_onepass_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smb));
+            prepare_onepass_kernel<true><<<p.Bp, PREP_CTA, smb, as_stream(stream)>>>(q);
             FFB_CUDA(cudaGetLastError());
             return 0;
         }

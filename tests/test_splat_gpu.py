@@ -195,27 +195,43 @@ def test_clustered_points_take_the_overflow_path(R, batched):
     close_grad(d[0], ana)
 
 
+def _bin_padded(R, monkeypatch, pts, n_total, band, sigma, ts, gS, gO):
+    """Forward and backward of `pts` padded to `n_total` points with points far off the texture (x = y = -5), appended after the
+    real ones: their windows are empty, so they are never binned and the real points keep their indices -- every candidate list is
+    the same, only N (and with it the binning kernel the library picks) changes.  Returns the sum and soft-OR textures and the
+    gradients of the real points; the pad points' gradients must be exactly 0."""
+    if band:
+        monkeypatch.setenv("FFB_PREP_BAND_ROWS", band)
+    else:
+        monkeypatch.delenv("FFB_PREP_BAND_ROWS", raising=False)
+    n = pts.shape[0]
+    p = torch.cat([pts, torch.full((n_total - n, 2), -5.0)]).cuda()
+    plan = R._SplatPlan(p, 1, sigma, ts[0], ts[1], 4, 5)
+    s, o = plan.forward(p, True, True, False)
+    d = plan.backward(p, gS, gO, False)
+    assert torch.equal(d[:, n:], torch.zeros_like(d[:, n:]))
+    return s.clone(), o.clone(), d[:, :n].clone()
+
+
 @pytest.mark.parametrize("clustered", [False, True])
 def test_binning_forms_agree_bitwise(R, monkeypatch, clustered):
     """The one-pass binning kernel (slot lists in shared memory, warp-wide entry stores; whole grid at once, or in bands of tile rows
-    for grids that do not fit the shared arrays) and the count/scan/fill kernel it replaces
-    order every candidate list by point index, so the outputs are identical to the bit -- also with overflowing lists and
-    with a tile count that is not a multiple of four (shared-memory rows stay 16-byte aligned)."""
+    for grids that do not fit the shared arrays) and the count/scan/fill kernel that takes over when the one-pass kernel's shared
+    arrays do not fit order every candidate list by point index, so the outputs are identical to the bit -- also with overflowing
+    lists and with a tile count that is not a multiple of four (shared-memory rows stay 16-byte aligned)."""
     gen = torch.Generator().manual_seed(5)
     ts, sigma = ([200, 136] if clustered else [328, 200]), 25.0
     pts = torch.rand(400, 2, generator=gen)
     if clustered:
         pts[:150] = 0.45 + 0.1 * pts[:150]
     gS, gO = torch.randn(1, ts[1], ts[0], generator=gen).cuda(), torch.randn(1, ts[1], ts[0], generator=gen).cuda()
-    res = []
-    for flag, band in (("1", None), ("0", None), ("1", "3")):      # one-pass; count / scan / fill; one-pass in bands of 3 tile rows
-        monkeypatch.setenv("FFB_PREP_ONEPASS", flag)
-        if band:
-            monkeypatch.setenv("FFB_PREP_BAND_ROWS", band)
-        plan = R._SplatPlan(pts.cuda(), 1, sigma, ts[0], ts[1], 4, 5)
-        s, o = plan.forward(pts.cuda(), True, True, False)
-        d = plan.backward(pts.cuda(), gS, gO, False)
-        res.append((s.clone(), o.clone(), d.clone()))
+    # the one-pass kernel needs 40 B per super tile of a band + 16 N B of shared memory (WCH = 16 uint16 slots, two int counters)
+    # within 226 KB, and N <= 65535: one tile row of these grids (6 or 4 super tiles) fits up to about 14,400 points
+    forms = ((400, None),       # one-pass, whole grid
+             (400, "3"),        # one-pass in bands of 3 tile rows
+             (15000, None),     # count / scan / fill: 16 * 15000 B = 234 KB of records alone exceed 226 KB
+             (70000, None))     # count / scan / fill: beyond the uint16 slot indices
+    res = [_bin_padded(R, monkeypatch, pts, n, band, sigma, ts, gS, gO) for n, band in forms]
     for other in res[1:]:
         assert torch.equal(res[0][0], other[0]) and torch.equal(res[0][1], other[1])
         # the per-point gradient is a sum of per-tile partials added with float atomics: same terms, arrival order not fixed
@@ -225,18 +241,16 @@ def test_binning_forms_agree_bitwise(R, monkeypatch, clustered):
 
 def test_large_grid_takes_the_banded_binning(R, monkeypatch):
     """4096 x 2048 texels = 8192 super tiles: more than the one-pass binning kernel holds in shared memory at once, so it bins in
-    bands of tile rows (chosen by the library).  Outputs identical to the count / scan / fill kernel's, which the smaller cases pin
-    against the oracle; column sums of the sum texture against the closed form for a few points."""
+    bands of tile rows (chosen by the library).  Outputs identical to the count / scan / fill kernel's (the same points padded past
+    what the one-pass kernel holds), which the smaller cases pin against the oracle; column sums of the sum texture against the
+    closed form for a few points."""
     gen = torch.Generator().manual_seed(19)
     ts, sigma = [4096, 2048], 100.0
     pts = (torch.rand(1500, 2, generator=gen) * 0.98 + 0.01)
     gS, gO = torch.randn(1, ts[1], ts[0], generator=gen).cuda(), torch.randn(1, ts[1], ts[0], generator=gen).cuda()
-    res = []
-    for flag in ("1", "0"):
-        monkeypatch.setenv("FFB_PREP_ONEPASS", flag)
-        plan = R._SplatPlan(pts.cuda(), 1, sigma, ts[0], ts[1], 4, 5)
-        s, o = plan.forward(pts.cuda(), True, True, False)
-        res.append((s.clone(), o.clone(), plan.backward(pts.cuda(), gS, gO, False).clone()))
+    # one-pass shared memory: 40 B per super tile of a band + 16 N B within 226 KB; one tile row (64 super tiles, 2.5 KB) leaves
+    # room for about 14,300 points, so 15,000 take count / scan / fill
+    res = [_bin_padded(R, monkeypatch, pts, n, None, sigma, ts, gS, gO) for n in (1500, 15000)]
     assert torch.equal(res[0][0], res[1][0]) and torch.equal(res[0][1], res[1][1])
     assert (res[0][2] - res[1][2]).norm() <= 1e-6 * res[1][2].norm()
     assert float(res[0][0].sum()) > 0 and torch.isfinite(res[0][2]).all()
