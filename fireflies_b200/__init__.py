@@ -16,7 +16,7 @@ from . import graphics  # noqa: F401
 from . import projection  # noqa: F401
 from . import postprocessing  # noqa: F401
 from .scene import Scene
-from .batch import SceneBatch, PatternStep  # noqa: F401
+from .batch import SceneBatch, PatternStep, TextureStep  # noqa: F401
 
 scene = Scene          # the README of the reference spells it ``ff.scene(mi_params)``
 

@@ -87,6 +87,7 @@ SIGNATURES = {
     "ffb_perlin_texture": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_double, _P, _P, _P, _P, _P, _P]),
     "ffb_respawn_rays": (C.c_int, [_P, C.c_int32, _P, _P, C.c_float, C.c_float, _P, C.c_uint64, C.c_uint64, _P, _P, _P]),
     "ffb_postprocess": (C.c_int, [C.POINTER(PostDesc), _P, _P, _P, _P, _P]),
+    "ffb_blur_bwd": (C.c_int, [C.POINTER(PostDesc), _P, _P, _P]),
     "ffb_nurbs_curve_eval": (C.c_int, [_P, _P, C.c_int32, C.c_int32, _P, C.c_int32, _P, _P]),
     "ffb_curve_pose": (C.c_int, [_P, _P, C.c_int32, C.c_int32, _P, C.c_int32, C.c_double, _P, _P, _P, _P, _P]),
     "ffb_ray_plane": (C.c_int, [_P, _P, _P, _P, C.c_int32, _P, _P]),

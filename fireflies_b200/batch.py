@@ -5,6 +5,7 @@ SURVEY.md section 3 (C)-(E)) becomes when B samples are processed at once.
 * :class:`SceneBatch`  -- ``Scene.randomize()`` for B samples: sampling (Philox / eval stepping), 4x4 compose
   with parent chains, vertex transform with animation gather.  3-4 launches, no host sync.
 * :class:`PatternStep` -- splat fwd (sum + soft-OR) -> loss -> splat bwd -> fold over samples -> allreduce.
+* :class:`TextureStep` -- the blurred projector texture from the laser rays, and its backward for B rendered samples.
 """
 from __future__ import annotations
 
@@ -506,3 +507,87 @@ class PatternStep:
         loss_host.copy_(loss, non_blocking=True)
         torch.cuda.current_stream().synchronize()
         return loss_host, out_host
+
+
+class TextureStep:
+    """The projector-texture optimisation step for B rendered scene samples per rank, with one exchange per step.
+
+    ``texture()`` builds the texture the renderer reads (:meth:`Laser.projector_texture`: the dense splat sum of the rays'
+    NDC xy, Gaussian-blurred, in channel 1 of ``[ts1, ts0, 3]``) from ``laser._rays`` and keeps what the backward needs.
+    ``backward(g_tex)`` takes the renderer's gradients w.r.t. that texture for this rank's samples (``[B, ts1, ts0, 3]`` or
+    ``[ts1, ts0, 3]``) and returns ``d loss / d rays`` ``[N, 3]`` summed over the samples and all ranks of
+    ``process_group``, also accumulated into ``laser._rays.grad`` the way autograd would (so ``torch.optim.Adam([laser._rays])``
+    works unchanged).  Every scene of the step sees the same texture and every backward stage is linear in the upstream
+    gradient, so the B gradients are folded first and the blur adjoint, the splat backward and the ray projection's backward
+    run once per step.  No autograd graph is built; the step's buffers are allocated by the first call and reused (the
+    returned tensor is overwritten by the next ``backward``)."""
+
+    def __init__(self, laser, sigma: float, texture_size, blur=((5, 5), (3.0, 3.0)), process_group=None):
+        from .postprocessing.gauss_blur import blur_spec
+        self.laser = laser
+        self.sigma = R._sigma(sigma)
+        self.ts0, self.ts1 = R._ts(texture_size)
+        self.blur = None if blur is None else blur_spec(blur[0], blur[1])
+        self.pg = process_group
+        self._saved = None                  # (rays, M, pts, plan) of the last texture()
+        self._bufs = None
+
+    def texture(self) -> torch.Tensor:
+        from .postprocessing.base import run_postprocess
+        L = nat.lib()
+        rays = nat.require_cuda(self.laser._rays.detach().float().contiguous(), torch.float32, "laser._rays")
+        M = self.laser._M()
+        N = rays.shape[0]
+        ndc = torch.empty_like(rays)
+        nat.check(L.ffb_transform_points(rays.data_ptr(), N, M.data_ptr(), 0, ndc.data_ptr(), nat.stream()), "ffb_transform_points")
+        nat.count()
+        pts = ndc[:, 0:2].contiguous()
+        plan = R._SplatPlan(pts, 1, self.sigma, self.ts0, self.ts1, 0, 0)
+        s, _ = plan.forward(pts, True, False, False)                        # [1, ts1, ts0]
+        if self.blur is not None:
+            s = run_postprocess(s, blur=self.blur)
+        tex = torch.zeros((self.ts1, self.ts0, 3), dtype=torch.float32, device=rays.device)
+        tex[..., 1] = s[0]
+        self._saved = (rays, M, pts, plan)
+        return tex
+
+    def _buffers(self, N: int, dev) -> dict:
+        b = self._bufs
+        if b is None or b["d_rays"].shape[0] != N or b["d_rays"].device != dev:
+            d_ndc = torch.zeros((N, 3), dtype=torch.float32, device=dev)        # column 2 stays 0: d ndc = (dx, dy, 0)
+            b = self._bufs = {"g1": torch.empty((1, self.ts1, self.ts0), dtype=torch.float32, device=dev),
+                              "g_in": torch.empty((1, self.ts1, self.ts0), dtype=torch.float32, device=dev),
+                              "d_pts": torch.empty((1, N, 2), dtype=torch.float32, device=dev),
+                              "d_ndc": d_ndc, "d_rays": torch.empty((N, 3), dtype=torch.float32, device=dev)}
+        return b
+
+    def backward(self, g_tex: torch.Tensor) -> torch.Tensor:
+        from .parallel import allreduce_sum_
+        from .postprocessing.gauss_blur import gaussian_blur2d_backward
+        if self._saved is None:
+            raise RuntimeError("TextureStep.backward: call texture() first")
+        rays, M, pts, plan = self._saved
+        g = nat.require_cuda(g_tex.contiguous(), torch.float32, "g_tex")
+        if g.dim() == 3:
+            g = g.unsqueeze(0)
+        if g.dim() != 4 or tuple(g.shape[1:]) != (self.ts1, self.ts0, 3):
+            raise ValueError(f"TextureStep.backward: g_tex must be [B, {self.ts1}, {self.ts0}, 3] or [{self.ts1}, {self.ts0}, 3]")
+        N = rays.shape[0]
+        b = self._buffers(N, rays.device)
+        folded = R.reduce_over_samples(g) if g.shape[0] > 1 else g[0]       # [ts1, ts0, 3]; channels 0 and 2 multiply constants
+        b["g1"][0].copy_(folded[..., 1])
+        g_sum = b["g1"]
+        if self.blur is not None:
+            g_sum = gaussian_blur2d_backward(b["g1"], *self.blur, out=b["g_in"])
+        d_pts = plan.backward(pts, g_sum, None, False, out=b["d_pts"])
+        b["d_ndc"][:, 0:2].copy_(d_pts[0])
+        nat.check(nat.lib().ffb_transform_points_bwd(rays.data_ptr(), N, M.data_ptr(), 0, b["d_ndc"].data_ptr(), b["d_rays"].data_ptr(),
+                                                     nat.stream()), "ffb_transform_points_bwd")
+        nat.count()
+        d_rays = allreduce_sum_(b["d_rays"], self.pg)
+        target = self.laser._rays
+        if target.grad is None:
+            target.grad = d_rays.to(target.dtype, copy=True)
+        else:
+            target.grad.add_(d_rays.to(target.dtype))
+        return d_rays

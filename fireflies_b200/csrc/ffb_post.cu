@@ -17,6 +17,8 @@
 // (vertical taps, noise / clip in registers, one 128-bit store).  No intermediate shared-memory pass.
 // Traffic: 4 B read (+ halo re-reads served by L2) + 4 B written per texel.
 // Other odd kernel sizes up to 15 take the generic kernel (blur_kernel: smem->smem horizontal, smem->register vertical).
+// The blur's adjoint (ffb_blur_bwd, what autograd needs to carry a gradient through the blur): blur_bwd_sw_kernel on the
+// sliding-window kernel's inputs, blur_bwd_kernel (plain loads) on every other input the forward accepts.
 #include <cuda.h>
 
 #include "ffb_common.cuh"
@@ -361,6 +363,175 @@ static int launch_blur_sw(const CUtensorMap& tmap, const PostParams& q, cudaStre
     return 0;
 }
 
+// ---- adjoint of the blur (ffb_blur_bwd) -------------------------------------------------------------------------------
+// Per axis the forward is y = W P x (P: reflect padding, W: valid correlation).  The taps are bitwise symmetric, so W^T is
+// the same correlation: Z = blur of g with g taken as ZERO outside the image, evaluated on the padded domain
+// [-h, n-1+h].  P^T then folds Z back onto the image: x_bar[j] = sum of Z over the preimage set of j under the reflection,
+// {j} + {-j if 1 <= j <= h} + {2(n-1)-j if n-1-h <= j <= n-2}; in 2-D over the product of the two axes' sets.  Only texels
+// within h of a border (the "band") have more than one preimage.
+__device__ __forceinline__ bool in_fold_band(int j, int n, int h) { return (j >= 1 && j <= h) || (j >= n - 1 - h && j <= n - 2); }
+// preimage u of j: u = 0 is j itself, 1 the reflection at the low border, 2 at the high one; false if it does not exist
+__device__ __forceinline__ bool fold_preimage(int u, int j, int n, int h, int& p) {
+    if (u == 0) { p = j; return true; }
+    if (u == 1) { p = -j; return j >= 1 && j <= h; }
+    p = 2 * (n - 1) - j;
+    return j >= n - 1 - h && j <= n - 2;
+}
+
+// Generic form: any odd sizes <= 15, W % 4 != 0, unaligned pointers.  One thread per texel, plain loads, the preimage
+// formula evaluated directly (q.img = g_out, q.out = g_in).
+__global__ void __launch_bounds__(THREADS) blur_bwd_kernel(const PostParams q) {
+    const size_t plane = (size_t)q.H * q.W, total = plane * q.B;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const int b = (int)(i / plane);
+        const int j = (int)((i - (size_t)b * plane) / q.W), c = (int)(i - (size_t)b * plane - (size_t)j * q.W);
+        const float* g = q.img + (size_t)b * plane;
+        float acc = 0.f;
+#pragma unroll 1
+        for (int u = 0; u < 3; ++u)
+#pragma unroll 1
+            for (int v = 0; v < 3; ++v) {
+                int p, pc;
+                if (!fold_preimage(u, j, q.H, q.hy, p) || !fold_preimage(v, c, q.W, q.hx, pc)) continue;
+                float z = 0.f;
+                for (int s = 0; s < q.ky; ++s) {
+                    const int y = p + s - q.hy;
+                    float hs = 0.f;
+                    if (y >= 0 && y < q.H)
+                        for (int t = 0; t < q.kx; ++t) {
+                            const int x = pc + t - q.hx;
+                            if (x >= 0 && x < q.W) hs = fmaf(q.wx[t], __ldg(g + (size_t)y * q.W + x), hs);
+                        }
+                    z = fmaf(q.wy[s], hs, z);
+                }
+                acc += z;
+            }
+        q.out[i] = acc;
+    }
+}
+
+// Z at padded position (p, c) from the staged tile of g.  g is zero outside the image, so the tap loops run over the
+// in-image rows / columns only; every in-image cell they read lies within h of a texel of this tile, so inside the box.
+// taps = wx[0..K) then wy[0..K), in shared memory (dynamic indices).
+template <int K>
+__device__ __forceinline__ float zval_tile(const float* in_s, const float* taps, const PostParams& q, int gy0, int gx0, int p, int c) {
+    constexpr int H = K / 2, BOXW = SwCfg<K>::BOXW;
+    const int s0 = max(0, H - p), s1 = min(K, q.H + H - p), t0 = max(0, H - c), t1 = min(K, q.W + H - c);
+    float acc = 0.f;
+    for (int s = s0; s < s1; ++s) {
+        const float* row = in_s + (p + s - H - gy0) * BOXW + (c - H - gx0);
+        float hs = 0.f;
+        for (int t = t0; t < t1; ++t) hs = fmaf(taps[t], row[t], hs);
+        acc = fmaf(taps[K + s], hs, acc);
+    }
+    return acc;
+}
+
+// adds the fold terms (every preimage but the texel itself) to the Z the interior loop stored for this band texel
+template <int K>
+__device__ __forceinline__ void fold_texel(const float* in_s, const float* taps, const PostParams& q, int b, int gy0, int gx0, int y, int x) {
+    float acc = 0.f;
+#pragma unroll 1
+    for (int u = 0; u < 3; ++u)
+#pragma unroll 1
+        for (int v = 0; v < 3; ++v) {
+            int p, c;
+            if ((u | v) != 0 && fold_preimage(u, y, q.H, K / 2, p) && fold_preimage(v, x, q.W, K / 2, c))
+                acc += zval_tile<K>(in_s, taps, q, gy0, gx0, p, c);
+        }
+    q.out[((size_t)b * q.H + y) * q.W + x] += acc;
+}
+
+// Production form (kx == ky in {3, 5, 11}, W % 4 == 0, sides >= 16, 16-byte aligned g_out / g_in): the sliding-window
+// kernel's skeleton.  One TMA load stages the tile of g + halo; the tensor map's out-of-bounds fill IS the zero extension
+// of g, so the interior loop is the forward's without its reflect patch and writes Z.  Tiles that hold band texels then
+// add the fold terms to those, read from the same staged tile (a few rows or columns of taps each: only the in-image part
+// of a padded position's support is nonzero).  The register bound keeps ptxas from spilling
+// (K = 11, two CTAs per SM: what its shared memory allows anyway) or from spending 94 registers (K = 5).
+template <int K>
+__global__ void __launch_bounds__(THREADS, K == 11 ? 2 : 4) blur_bwd_sw_kernel(const __grid_constant__ CUtensorMap tmap, const PostParams q) {
+    typedef SwCfg<K> CF;
+    constexpr int BOXW = CF::BOXW, BOXH = CF::BOXH, TH2 = CF::TH, RW = CF::RW, HK = CF::H;
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    float* in_s = reinterpret_cast<float*>(smem_raw);                  // [BOXH][BOXW]
+    __shared__ __align__(8) uint64_t bar;
+    __shared__ float taps_s[2 * K];
+    const int tiles_x = (q.W + SW_TW - 1) / SW_TW;
+    const int tx = blockIdx.x % tiles_x, ty = blockIdx.x / tiles_x, b = blockIdx.y;
+    const int x0 = tx * SW_TW, y0 = ty * TH2;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+
+    const int gx0 = x0 - CF::PADL, gy0 = y0 - HK;
+    if (tid < 2 * K) taps_s[tid] = tid < K ? q.wx[tid] : q.wy[tid - K];
+    if (tid == 0) {
+        mbar_init(&bar, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+    if (tid == 0) {
+        mbar_expect_tx(&bar, (uint32_t)(BOXW * BOXH * sizeof(float)));
+        tma_load_3d(in_s, &tmap, &bar, gx0, gy0, b);
+    }
+    mbar_wait(&bar, 0);
+
+    float wx[K], wy[K];
+#pragma unroll
+    for (int t = 0; t < K; ++t) { wx[t] = q.wx[t]; wy[t] = q.wy[t]; }
+    const int x = x0 + 4 * lane;
+    const float* colp = in_s + 4 * lane;
+    float win[K][4];
+#pragma unroll
+    for (int rr = 0; rr < RW + K - 1; ++rr) {
+        const float* rowp = colp + (warp * RW + rr) * BOXW;
+        float v[4 * (1 + 2 * CF::NQ)];
+#pragma unroll
+        for (int w4 = 0; w4 < 1 + 2 * CF::NQ; ++w4) {
+            const float4 a = *reinterpret_cast<const float4*>(rowp + 4 * w4);
+            v[4 * w4] = a.x; v[4 * w4 + 1] = a.y; v[4 * w4 + 2] = a.z; v[4 * w4 + 3] = a.w;
+        }
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            float acc = 0.f;
+#pragma unroll
+            for (int t = 0; t < K; ++t) acc = fmaf(wx[t], v[CF::PADL - HK + j + t], acc);
+            win[rr % K][j] = acc;
+        }
+        if (rr >= K - 1) {
+            const int y = y0 + warp * RW + rr - (K - 1);
+            float o[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+            for (int t = 0; t < K; ++t)
+#pragma unroll
+                for (int j = 0; j < 4; ++j) o[j] = fmaf(wy[t], win[(rr - (K - 1) + t) % K][j], o[j]);
+            if (y < q.H && x < q.W)
+                *reinterpret_cast<float4*>(q.out + ((size_t)b * q.H + y) * q.W + x) = make_float4(o[0], o[1], o[2], o[3]);
+        }
+    }
+
+    // ---- fold epilogue: band texels of this tile (rows 1..h and H-1-h..H-2, the same for columns) ----
+    const int ye = min(y0 + TH2, q.H), xe = min(x0 + SW_TW, q.W);
+    const bool rows_hit = y0 <= HK || ye > q.H - 1 - HK, cols_hit = x0 <= HK || xe > q.W - 1 - HK;
+    if (!rows_hit && !cols_hit) return;
+    __syncthreads();                          // the band texels' Z values are written: the additions below read them
+    // row band within the tile: [ra0, ra1) and [rb0, rb1), disjoint
+    const int ra0 = max(y0, 1), ra1 = max(ra0, min(ye, HK + 1));
+    const int rb0 = max(max(y0, q.H - 1 - HK), ra1), rb1 = max(rb0, min(ye, q.H - 1));
+    const int nra = ra1 - ra0, nr = nra + (rb1 - rb0), ncols = xe - x0;
+    for (int i = tid; i < nr * ncols; i += THREADS) {
+        const int r = i / ncols, y = r < nra ? ra0 + r : rb0 + r - nra;
+        fold_texel<K>(in_s, taps_s, q, b, gy0, gx0, y, x0 + i - r * ncols);
+    }
+    // column band within the tile, rows outside the row band
+    const int ca0 = max(x0, 1), ca1 = max(ca0, min(xe, HK + 1));
+    const int cb0 = max(max(x0, q.W - 1 - HK), ca1), cb1 = max(cb0, min(xe, q.W - 1));
+    const int nca = ca1 - ca0, nc = nca + (cb1 - cb0), nrows = ye - y0;
+    for (int i = tid; i < nrows * nc; i += THREADS) {
+        const int r = i / nc, k = i - r * nc, y = y0 + r;
+        if (in_fold_band(y, q.H, HK)) continue;
+        fold_texel<K>(in_s, taps_s, q, b, gy0, gx0, y, k < nca ? ca0 + k : cb0 + k - nca);
+    }
+}
+
 // no blur stage configured: pure streaming copy / noise / clip
 __global__ void __launch_bounds__(THREADS) pointwise_kernel(const PostParams q) {
     // one item = a 4-texel quad of a row pair (rows 2 rp, 2 rp + 1): both loads in flight, one Philox call for the 8 variates
@@ -655,6 +826,65 @@ static int postprocess_impl(const ffb_post_desc* d, const float* img, const uint
         if (smem > 48 * 1024) FFB_CUDA(cudaFuncSetAttribute(blur_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         blur_kernel<false><<<dim3(tiles, d->B), THREADS, smem, st>>>(tmap, q);
     }
+    FFB_CUDA(cudaGetLastError());
+    return 0;
+}
+
+template <int K>
+static int launch_blur_bwd_sw(const PostParams& q, cudaStream_t st, bool* launched) {
+    typedef SwCfg<K> CF;
+    *launched = false;
+    CUtensorMap tm;
+    memset(&tm, 0, sizeof(tm));
+    cuuint64_t gdim[3] = {(cuuint64_t)q.W, (cuuint64_t)q.H, (cuuint64_t)q.B};
+    cuuint64_t gstr[2] = {(cuuint64_t)q.W * 4, (cuuint64_t)q.W * q.H * 4};
+    cuuint32_t box[3] = {(cuuint32_t)CF::BOXW, (cuuint32_t)CF::BOXH, 1};
+    cuuint32_t estr[3] = {1, 1, 1};
+    EncodeTiledFn enc = get_encode();
+    if (!enc || enc(&tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(q.img), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                    CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+        return 0;
+    const size_t smem = (size_t)CF::BOXW * CF::BOXH * sizeof(float);
+    const unsigned tiles = (unsigned)(((q.W + SW_TW - 1) / SW_TW) * ((q.H + CF::TH - 1) / CF::TH));
+    if (smem > 48 * 1024) FFB_CUDA(cudaFuncSetAttribute(blur_bwd_sw_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    blur_bwd_sw_kernel<K><<<dim3(tiles, q.B), THREADS, smem, st>>>(tm, q);
+    FFB_CUDA(cudaGetLastError());
+    *launched = true;
+    return 0;
+}
+
+extern "C" int ffb_blur_bwd(const ffb_post_desc* d, const float* g_out, float* g_in, void* stream) {
+    if (!d || !g_out || !g_in) return fail_arg(FFB_E_ARG, "blur_bwd: null pointer");
+    if (d->B <= 0 || d->H <= 0 || d->W <= 0) return fail_arg(FFB_E_ARG, "blur_bwd: B, H, W must be positive");
+    if (d->B > 65535) return fail_arg(FFB_E_LIMIT, "blur_bwd: B > 65535");
+    if (d->noise != 0) return fail_arg(FFB_E_ARG, "blur_bwd: the noise stage has no backward (noise must be 0)");
+    if (d->blur_ky <= 0 || d->blur_kx <= 0) return fail_arg(FFB_E_ARG, "blur_bwd: the descriptor has no blur stage");
+    if (d->blur_kx > KMAX || d->blur_ky > KMAX) return fail_arg(FFB_E_LIMIT, "blur_bwd: blur kernel size > 15");
+    if (d->blur_kx % 2 == 0 || d->blur_ky % 2 == 0) return fail_arg(FFB_E_ARG, "blur_bwd: blur kernel sizes must be odd");
+    if (!(d->blur_sx > 0.f) || !(d->blur_sy > 0.f)) return fail_arg(FFB_E_ARG, "blur_bwd: blur sigma must be > 0");
+    if (d->blur_kx / 2 >= d->W || d->blur_ky / 2 >= d->H) return fail_arg(FFB_E_ARG, "blur_bwd: reflect border needs kernel/2 < image side");
+    const size_t bytes = (size_t)d->B * d->H * d->W * sizeof(float);
+    const uintptr_t a = reinterpret_cast<uintptr_t>(g_out), c = reinterpret_cast<uintptr_t>(g_in);
+    if (a < c + bytes && c < a + bytes) return fail_arg(FFB_E_ARG, "blur_bwd: g_out and g_in must not alias");
+    PostParams q;
+    memset(&q, 0, sizeof(q));
+    q.B = d->B; q.H = d->H; q.W = d->W;
+    q.kx = d->blur_kx; q.ky = d->blur_ky; q.hx = q.kx / 2; q.hy = q.ky / 2;
+    gaussian_taps(q.kx, d->blur_sx, q.wx);
+    gaussian_taps(q.ky, d->blur_sy, q.wy);
+    q.img = g_out; q.out = g_in;
+    cudaStream_t st = as_stream(stream);
+    // the forward's sliding-window conditions, plus an aligned g_in for the 128-bit stores
+    if (q.kx == q.ky && (q.kx == 3 || q.kx == 5 || q.kx == 11) && d->W % 4 == 0 && d->W >= 16 && d->H >= 16 && (a & 15) == 0 && (c & 15) == 0) {
+        bool launched = false;
+        int rc = q.kx == 3 ? launch_blur_bwd_sw<3>(q, st, &launched) : q.kx == 5 ? launch_blur_bwd_sw<5>(q, st, &launched)
+                                                                                 : launch_blur_bwd_sw<11>(q, st, &launched);
+        if (rc || launched) return rc;
+    }
+    const size_t total = bytes / sizeof(float);
+    size_t blocks = (total + THREADS - 1) / THREADS;
+    if (blocks > (size_t)kNumSMs * 16) blocks = (size_t)kNumSMs * 16;
+    blur_bwd_kernel<<<(unsigned)blocks, THREADS, 0, st>>>(q);
     FFB_CUDA(cudaGetLastError());
     return 0;
 }

@@ -16,6 +16,7 @@ import torch
 
 from .. import _native as nat
 from ..graphics import rasterization
+from ..postprocessing.gauss_blur import gaussian_blur2d
 from ..sampling import poisson
 from ..utils import math as ffmath
 from .camera import Camera
@@ -183,6 +184,18 @@ class Laser(Camera):
         points = self.projectRaysToNDC()[:, 0:2]
         s, o = rasterization.splat_reduce(points, sigma, texture_size, num_std_sum=None, num_std_softor=None, reduce=(reduce,))
         return s if reduce == "sum" else o
+
+    def projector_texture(self, sigma: float, texture_size, blur=((5, 5), (3.0, 3.0))) -> torch.Tensor:
+        """The projector texture the renderer reads (main.py:64-77): ``[ts[1], ts[0], 3]``, zeros in channels 0 and 2 and
+        the Gaussian-blurred dense splat sum of the rays' NDC xy in channel 1.  ``blur`` = ``(kernel_size, sigma)`` as in
+        ``kornia.filters.gaussian_blur2d``, None = no blur.  Differentiable w.r.t. ``_rays``.  For B rendered samples per
+        step see :class:`fireflies_b200.TextureStep`."""
+        points = self.projectRaysToNDC()[:, 0:2]
+        tex = rasterization.splat_reduce(points, sigma, texture_size, num_std_sum=None, num_std_softor=None, reduce=("sum",))[0]
+        if blur is not None:
+            tex = gaussian_blur2d(tex[None, None], blur[0], blur[1])[0, 0]
+        zero = torch.zeros_like(tex)
+        return torch.stack([zero, tex, zero]).movedim(0, -1)
 
     def render_epipolar_lines(self, sigma: float, texture_size: torch.Tensor, camera_to_world: torch.Tensor = None) -> torch.Tensor:
         """laser.py:298-325: the segments origin + [near_clip, far_clip] * ray, seen through ``camera_to_world`` (identity when

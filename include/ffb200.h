@@ -318,6 +318,11 @@ typedef struct ffb_post_desc {
 FFB_API int ffb_postprocess(const ffb_post_desc* d, const float* img, const uint8_t* gates,
                     const double* noise_injected, float* out, void* stream);
 
+/* Backward of ffb_postprocess's blur stage w.r.t. its input, per frame: g_in = A^T g_out, A = the separable Gaussian blur
+ * with kornia's reflect border that ffb_postprocess applies for d's blur fields (same rules: odd sizes <= 15,
+ * kernel/2 < side).  d->noise must be 0; seed / frame0 are ignored; no gates.  g_out, g_in f32 [B,H,W], must not alias. */
+FFB_API int ffb_blur_bwd(const ffb_post_desc* d, const float* g_out, float* g_in, void* stream);
+
 /* ApplySilhouette.post_process (fireflies/postprocessing/apply_silhouette.py:17-40) for B frames:
  * out = img * blur11x11,sigma5(disc(cx, cy, r)).  discs int32 [B,3] = (cx, cy, r) per frame -- the caller's
  * random.randint draws (:23-25).  The disc is the analytic set (x-cx)^2 + (y-cy)^2 <= r^2 (the reference
