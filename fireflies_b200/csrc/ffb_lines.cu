@@ -27,6 +27,8 @@ constexpr int WROWS = 8;       // rows per warp
 constexpr int TROWS = 64;
 constexpr int TCOLS = 32;
 constexpr int CHUNK = 128;     // lines staged per pass
+static_assert(CTA == 32 * (TROWS / WROWS), "one warp per WROWS x TCOLS block of the CTA tile");
+static_assert(CHUNK <= CTA, "stage_lines and the dl_s zeroing give each staged line one thread");
 
 struct Seg {
     float ax, ay, bx, by;      // end points * texture_size
@@ -238,8 +240,8 @@ __global__ void __launch_bounds__(CTA) reduce_bwd_kernel(ReduceParams q) {
             }
         }
         __syncthreads();
-        if ((int)threadIdx.x < 4 * n) {
-            const int k = threadIdx.x >> 2, j = threadIdx.x & 3;
+        for (int e = threadIdx.x; e < 4 * n; e += CTA) {      // 4 * CHUNK components, more than one per thread
+            const int k = e >> 2, j = e & 3;
             const float v = dl_s[k][j] * ((j & 1) ? (float)q.ts1 : (float)q.ts0);
             if (v != 0.f) atomicAdd(&q.d_lines[4 * (base + k) + j], v);
         }

@@ -334,6 +334,8 @@ def _lines(lines: torch.Tensor) -> torch.Tensor:
     lines = nat.require_cuda(lines.float().contiguous(), torch.float32, "lines")
     if lines.dim() != 3 or lines.shape[1:] != (2, 2):
         raise ValueError("lines must be [L, 2, 2] (start / end x X / Y)")
+    if lines.data_ptr() % 16 != 0:
+        lines = lines.clone()           # the kernels read each line as one float4; a fresh allocation is 16-byte aligned
     return lines
 
 

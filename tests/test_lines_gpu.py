@@ -1,6 +1,8 @@
 """GPU parity of the line and depth rasterisers (SURVEY.md 8(f) row 2) against the reference-generated fixture
 (tests/golden/lines_depth.npz, oracle/make_golden.py) and the CPU oracle.  Tolerances as for the point splat:
-forward 1e-5 relative (+1e-6 absolute), gradients 1e-4 relative to the largest component."""
+forward 1e-5 relative (+1e-6 absolute), gradients 1e-4 relative to the largest component.  The shapes here are small;
+tests/test_lines_ref_gpu.py checks the same kernels against fp64 across line counts, ragged textures, culling radii,
+geometry edges and every kernel instantiation."""
 import numpy as np
 import pytest
 import torch
