@@ -254,11 +254,12 @@ __device__ __forceinline__ PointRec make_rec(const PrepParams& q, float x, float
 }
 
 // window origin of the warp-tile kernels' Chebyshev masks along one axis: the reference's (unclipped) slice start
-// floor(P - half) plus half for a baked window (rasterization.py:186), floor(P) otherwise; clamped to int16.  Integer valued and
-// exact in fp32 (|result| < 2^24).
+// floor(P - half) plus half for a baked window (rasterization.py:186), floor(P) otherwise.  Exact for every point whose window
+// can reach a texture side of up to 65535; beyond 2^22 texels (and for NaN) a far sentinel that masks every texel.  Integer valued
+// and exact in fp32 (|result| < 2^23).
 __device__ __forceinline__ float origin_axis_f(float P, int baked, int half) {
     const float fo = floorf(baked ? P - (float)half : P);
-    if (!(fo > -30000.f && fo < 30000.f)) return fo > 0.f ? 32767.f : -32768.f;
+    if (!(fo > -4194304.f && fo < 4194304.f)) return fo > 0.f ? 4194304.f : -4194304.f;
     return baked ? fo + (float)half : fo;
 }
 
