@@ -382,19 +382,18 @@ class PatternStep:
                     ring[slot] = res
                 mark("randomize1", self._side)
                 nvtx.range_pop()
-        if points.dim() == 2:
-            if self.per_sample:
-                # one 8N-byte host->device copy, then a device-side broadcast (a copy from an expanded host view costs 0.5 ms)
-                self._pat_dev.copy_(points, non_blocking=True)
-                self.pts_dev.copy_(self._pat_dev.unsqueeze(0).expand_as(self.pts_dev))
-            else:
-                self.pts_dev.copy_(points.unsqueeze(0), non_blocking=True)
-        else:
-            self.pts_dev.copy_(points, non_blocking=True)
         if not self.per_sample:
+            self.pts_dev.copy_(points.unsqueeze(0) if points.dim() == 2 else points, non_blocking=True)
             loss, dp, s, o = self._shared_pattern(self.pts_dev[0], upstream)
             return self._finish(loss, dp, s, o, res)
-        pts = self.pts_dev
+        if points.dim() == 2:
+            # one pattern for every sample: binned once (a [N,2] plan), while the B textures and the per-sample gradients against
+            # the per-sample upstream gradients stay as they are
+            self._pat_dev.copy_(points, non_blocking=True)
+            pts = self._pat_dev
+        else:
+            self.pts_dev.copy_(points, non_blocking=True)
+            pts = self.pts_dev
         nvtx.range_push("ffb.prepare")
         plan = R._SplatPlan(pts, self.B, self.sigma, self.ts0, self.ts1, self.ns, self.no)
         nvtx.range_pop()

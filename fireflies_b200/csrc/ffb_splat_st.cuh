@@ -124,6 +124,11 @@ __device__ __forceinline__ float4 st_lds128(unsigned a) {
     asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(a));
     return v;
 }
+__device__ __forceinline__ float2 st_lds64(unsigned a) {
+    float2 v;
+    asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(a));
+    return v;
+}
 __device__ __forceinline__ float st_lds32(unsigned a) {
     float v;
     asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a));
@@ -331,6 +336,72 @@ __device__ __forceinline__ void st_weigh_triple(unsigned rec, StPend& pd, float&
     st_weigh_one_of_triple<SUM, MSK>(rc2, pd, accr, k2, tc, ln, lane, fc, gs, go, g2, g0, g1);
 }
 
+// tile with NK candidates (four: st_tile): each exponential once per texel, each candidate's exclusive product from a prefix product
+// (forward over the candidates) times a suffix product (backward) -- no pass 1, no reciprocal, and the product stays the one
+// torch.prod's backward forms.  NK candidates' g of all 8 texels do not fit in registers, so the work is blocked over the lane's four
+// texel pairs: per pair, NK values of g and of the prefix; the candidates' partial sums are carried across the pairs and then reduced
+// one visit per candidate, in the walk order of st_weigh.  The geometry is recomputed in the backward sweep rather than kept.
+// The upstream values are read pair by pair (up(v, gs, go)): all four pairs held through the sweeps would spill.
+template <bool SUM, bool MSK, int NK, class Up>
+__device__ __forceinline__ void st_weigh_few(unsigned rec, StPend& pd, float& accr, unsigned tm, const StTileCols& tc, const StLane& ln,
+                                             int lane, const WtConsts& fc, const Up& up) {
+    int kn[NK];
+    float4 rc[NK];
+#pragma unroll
+    for (int n = 0; n < NK; ++n) {
+        kn[n] = st_next(tm);
+        rc[n] = st_lds128(rec + 16u * (unsigned)kn[n]);
+    }
+    float a0[NK], a1[NK];                                                             // the lane's d/dp0, d/dp1 parts of candidate n
+#pragma unroll
+    for (int n = 0; n < NK; ++n) a0[n] = a1[n] = 0.f;
+#pragma unroll 1
+    for (int v = 0; v < 4; ++v) {
+        const float2 cx = (v & 1) ? tc.c23 : tc.c01;
+        const float ry = v < 2 ? ln.rabs.x : ln.rabs.y;
+        float2 gs = bc(0.f), p;
+        up(v, gs, p);                                                                 // p: gO * prod_{m < n}(1 - g_m)
+        float2 g[NK], pre[NK];
+#pragma unroll
+        for (int n = 0; n < NK; ++n) {
+            const float2 dxs = __fadd2_rn(cx, bc(-rc[n].x));
+            const float dys = ry - rc[n].y;
+            const float2 d2 = __ffma2_rn(dxs, dxs, bc(dys * dys));
+            const float2 t = __fmul2_rn(neg2(d2), d2);
+            g[n] = make_float2(ex2_approx(t.x), ex2_approx(t.y));
+            pre[n] = p;
+            if (n + 1 < NK) p = __ffma2_rn(neg2(g[n]), p, p);
+        }
+        float2 suf = bc(1.f);                                                         // prod_{m > n}(1 - g_m)
+#pragma unroll
+        for (int n = NK - 1; n >= 0; --n) {
+            const float2 dxs = __fadd2_rn(cx, bc(-rc[n].x));
+            const float dys = ry - rc[n].y;
+            const float2 d2 = __ffma2_rn(dxs, dxs, bc(dys * dys));
+            float2 x;                                                                 // gO * prod_{m != n}(1 - g_m) [+ gS]
+            if (SUM && !MSK) x = __ffma2_rn(pre[n], suf, gs);
+            else x = __fmul2_rn(pre[n], suf);
+            if (SUM && MSK) {
+                if (fabsf(dys + rc[n].w) <= fc.hs_r) {
+                    const float2 e = __fadd2_rn(dxs, bc(rc[n].z));
+                    const float2 mc = make_float2(__saturatef(fmaf(fabsf(e.x), fc.m_r, fc.thr_r)), __saturatef(fmaf(fabsf(e.y), fc.m_r, fc.thr_r)));
+                    x = __ffma2_rn(gs, mc, x);
+                }
+            }
+            if (n > 0) suf = __ffma2_rn(neg2(g[n]), suf, suf);
+            const float2 wgt = __fmul2_rn(__fmul2_rn(x, g[n]), d2);
+            const float s0 = fmaf(wgt.y, dxs.y, wgt.x * dxs.x), s1 = (wgt.x + wgt.y) * dys;
+            a0[n] += s0;
+            a1[n] += s1;
+        }
+    }
+#pragma unroll
+    for (int n = 0; n < NK; ++n) {
+        st_reduce(pd, accr, lane);
+        pd.s0 = a0[n]; pd.s1 = a1[n]; pd.k = kn[n];
+    }
+}
+
 // ---- staging: one candidate per lane -> tile masks (ballots) and 16-byte records {(P0 - c0) r1, (P1 - r0) r1, (P0 - f0) r1, (P1 - f1) r1} ----
 __device__ __forceinline__ WtMasks st_stage(const RasterParams& q, const WtConsts& fc, int bin, int beg, int n, int c0, int r0, int lane,
                                             float4* rec, int* idx) {
@@ -406,7 +477,7 @@ __device__ __forceinline__ float st_lds_s8(unsigned a) {
 }
 
 // one 16x16 tile of the resident super tile: upstream values of the lane's 8 texels from shared memory, then the tile's candidates
-template <bool SUM, bool SOFTOR, bool SUM_T, bool MSK, int MODE>
+template <bool SUM, bool SOFTOR, bool SUM_T, bool MSK, int MODE, bool FEW>
 __device__ __forceinline__ void st_tile(unsigned sbase, int j, unsigned tm, unsigned nm, unsigned rec, StPend& pd, float& accr,
                                         float& lacc, const StLane& ln, int lane, const WtConsts& fc) {
     typedef StSmem<SUM, SOFTOR, SUM_T, MODE> L;
@@ -426,7 +497,32 @@ __device__ __forceinline__ void st_tile(unsigned sbase, int j, unsigned tm, unsi
         v[2] = make_float2(st_lds32(b0), st_lds32(b0 + 64));
         v[3] = make_float2(st_lds32(b2), st_lds32(b2 + 64));
     };
+    StTileCols tc;
+    {
+        const float sc = fc.r1;
+        const float cfs = fmaf((float)j, (float)WT * sc, ln.cbs);
+        tc.c01 = make_float2(cfs, cfs + sc);
+        tc.c23 = make_float2(cfs + 2.f * sc, cfs + 3.f * sc);
+    }
     const bool one = (tm & (tm - 1u)) == 0u;               // at most one candidate on this tile (warp-uniform)
+    const int cands = __popc(tm);
+    // four candidates (14 % of the tiles, 21 % of the visits at config 3): one pass (st_weigh_few).  Five or six spill at the
+    // 80-register target, and so does the one-shot kernel with this branch (FEW = false there)
+    if (FEW && !LOSS && SOFTOR && cands == 4) {
+        auto up = [&](int v, float2& s, float2& o) {        // texel pair v of both upstream arrays
+            const unsigned n = sbase + nb + (unsigned)(v >> 1) * 1024u + (unsigned)(v & 1) * 8u;
+            o = st_lds64(n + L::off_go);
+            if (SUM && SUM_T) {
+                const unsigned t = sbase + L::off_gs + j * 1024;
+                const unsigned a = t + ((v < 2 ? ln.tA0 : (ln.tA0 ^ 32u)) ^ ((v & 1) ? 16u : 0u));
+                s = make_float2(st_lds32(a + ((v & 1) ? 128u : 0u)), st_lds32(a + ((v & 1) ? 192u : 64u)));
+            } else if (SUM) {
+                s = st_lds64(n + L::off_gs);
+            }
+        };
+        st_weigh_few<SUM, MSK, 4>(rec, pd, accr, tm, tc, ln, lane, fc, up);
+        return;
+    }
     if (LOSS) {
         // unit signs here; the 1 / numel of the mean is folded into the final scale of d/dP and of the loss
         float2 o[4], s[4];
@@ -455,18 +551,10 @@ __device__ __forceinline__ void st_tile(unsigned sbase, int j, unsigned tm, unsi
         if (SUM) { if (SUM_T) ld_tr(L::off_gs, gs); else ld_nat(L::off_gs, gs); }
         if (SOFTOR) ld_nat(L::off_go, gp);
     }
-    StTileCols tc;
-    {
-        const float sc = fc.r1;
-        const float cfs = fmaf((float)j, (float)WT * sc, ln.cbs);
-        tc.c01 = make_float2(cfs, cfs + sc);
-        tc.c23 = make_float2(cfs + 2.f * sc, cfs + 3.f * sc);
-    }
     if (one || !SOFTOR) {
         st_weigh<SUM, SOFTOR, MSK, 2>(rec, pd, accr, tm, tc, ln, lane, fc, gs, gp);
         return;
     }
-    const int cands = __popc(tm);
     if (cands == 2) {                                       // exclusive products are the other candidate's factor (no pass 1, no reciprocal)
         st_weigh_pair<SUM, MSK>(rec, pd, accr, tm, tc, ln, lane, fc, gs, gp);
         return;
@@ -608,7 +696,7 @@ __global__ void __launch_bounds__(32, ST_MINB) splat_bwd_st(RasterParams q, WtCo
         const unsigned tm = tbits & 0xffffu, nm = nbits & 0xffffu;
         tbits >>= 16; nbits >>= 16;
         if (tm == 0u) continue;
-        st_tile<SUM, SOFTOR, SUM_T, MSK, ST_REBUILD>(sbase, j, tm, nm, sbase + L::off_rec, pd, accr, lacc, ln, lane, fc);
+        st_tile<SUM, SOFTOR, SUM_T, MSK, ST_REBUILD, false>(sbase, j, tm, nm, sbase + L::off_rec, pd, accr, lacc, ln, lane, fc);
     }
     st_flush(q, st_scale(q, fc, lane), pd, accr, lane, n, b, idx);
 }
@@ -734,7 +822,7 @@ __global__ void __launch_bounds__(32, ST_MINB) splat_bwd_stp(RasterParams q, WtC
             const unsigned tm = tbits & 0xffffu, nm = nbits & 0xffffu;
             tbits >>= 16; nbits >>= 16;
             if (!LOSS && tm == 0u) continue;
-            st_tile<SUM, SOFTOR, SUM_T, MSK, MODE>(sbase, j, tm, nm, sbase + L::off_rec, pd, accr, lacc, ln, lane, fc);
+            st_tile<SUM, SOFTOR, SUM_T, MSK, MODE, true>(sbase, j, tm, nm, sbase + L::off_rec, pd, accr, lacc, ln, lane, fc);
         }
         __syncwarp();
         if (more) st_issue_half<SUM, SOFTOR, SUM_T, MODE>(st_smem, bar + 1, 1, nx.bx * (4 * WT), nx.sty * WT, nx.b, &tm_gs, &tm_go, &tm_sv, &tm_ot, TWO);
