@@ -49,6 +49,11 @@ class PostDesc(C.Structure):
                 ("noise_std", C.c_float), ("seed", C.c_uint64), ("frame0", C.c_uint64)]
 
 
+class PerlinParams(C.Structure):
+    _fields_ = [("res0", C.c_int32), ("res1", C.c_int32), ("octaves", C.c_int32), ("_pad", C.c_int32),
+                ("persistence", C.c_double), ("angle_offset", C.c_int64)]
+
+
 # symbol -> (restype, argtypes); the complete export list of include/ffb200.h
 _P = C.c_void_p
 SIGNATURES = {
@@ -85,6 +90,8 @@ SIGNATURES = {
     "ffb_clamp_to_fov": (C.c_int, [_P, C.c_int32, _P, _P, C.c_float, C.c_float, _P, _P]),
     "ffb_silhouette": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P]),
     "ffb_perlin_texture": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_double, _P, _P, _P, _P, _P, _P]),
+    "ffb_perlin_texture_batch": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_uint64, C.c_uint64, C.c_int32, _P, _P, C.c_int64,
+                                           _P, _P, _P, _P, _P, _P, _P]),
     "ffb_respawn_rays": (C.c_int, [_P, C.c_int32, _P, _P, C.c_float, C.c_float, _P, C.c_uint64, C.c_uint64, _P, _P, _P]),
     "ffb_postprocess": (C.c_int, [C.POINTER(PostDesc), _P, _P, _P, _P, _P]),
     "ffb_blur_bwd": (C.c_int, [C.POINTER(PostDesc), _P, _P, _P]),

@@ -3,14 +3,15 @@ of launches.  This is what the reference's per-sample loop (``scene.randomize()`
 SURVEY.md section 3 (C)-(E)) becomes when B samples are processed at once.
 
 * :class:`SceneBatch`  -- ``Scene.randomize()`` for B samples: sampling (Philox / eval stepping), 4x4 compose
-  with parent chains, vertex transform with animation gather.  3-4 launches, no host sync.
+  with parent chains, vertex transform with animation gather, Perlin material textures.  3-4 launches (plus 3 per
+  texture attribute), no host sync.
 * :class:`PatternStep` -- splat fwd (sum + soft-OR) -> loss -> splat bwd -> fold over samples -> allreduce.
 * :class:`TextureStep` -- the blurred projector texture from the laser rays, and its backward for B rendered samples.
 """
 from __future__ import annotations
 
 import ctypes as C
-from dataclasses import dataclass
+from dataclasses import dataclass, field
 from typing import Dict, List, Optional, Tuple
 
 import numpy as np
@@ -20,9 +21,10 @@ from . import _native as nat
 from .entity import Mesh, Transformable
 from .entity.base import _ENT_INTS, _ENT_WORDS
 from .graphics import rasterization as R
-from .sampling import AnimationSampler, Sampler
+from .sampling import AnimationSampler, NoiseTextureLerpSampler, Sampler
 from .sampling.base import _WORDS as _SMP_WORDS
 from .sampling.base import rehome
+from .sampling.noise_texture_lerp import PERLIN_TILE, perlin_texture_batch
 
 
 @dataclass
@@ -32,6 +34,7 @@ class BatchResult:
     sampled: torch.Tensor               # [B,S,3]
     vertices: Optional[torch.Tensor]    # [B,Vtot,3] (padded slots) or None
     batch: "SceneBatch"
+    textures: Dict[Tuple[str, str], tuple] = field(default_factory=dict)   # (entity, key) -> ([B,3,H,W], PerlinDraws)
 
     def mesh_vertices(self, name: str) -> torch.Tensor:
         off, n = self.batch._mesh_slices[name]
@@ -41,13 +44,17 @@ class BatchResult:
         return self.world[:, self.batch._entity_index[name]]
 
     def attribute(self, entity_name: str, key: str) -> torch.Tensor:
+        """``[B,dim]`` sampled values, or ``[B,3,H,W]`` for a texture attribute."""
+        if (entity_name, key) in self.textures:
+            return self.textures[(entity_name, key)][0]
         row, dim = self.batch._attr_rows[(entity_name, key)]
         return self.sampled[:, row, :dim]
 
     # ---- hand-off to Mitsuba (SURVEY.md 8(f) row 1; reference: Scene.update_*, scene.py:243-342) ----------------------
     def to_host(self):
         """ONE device->host copy (pinned, asynchronous + one event wait) of every 4x4 matrix and sampled attribute of all B
-        samples.  The reference pays a `.tolist()` / `.item()` sync per entity and attribute (scene.py:257-342)."""
+        samples.  The reference pays a `.tolist()` / `.item()` sync per entity and attribute (scene.py:257-342).  Textures
+        stay on the device."""
         if getattr(self, "_host", None) is None:
             B = self.world.shape[0]
             nw, ns = self.world[0].numel(), self.sampled[0].numel()
@@ -63,8 +70,8 @@ class BatchResult:
     def write_sample(self, b: int, update: bool = True) -> None:
         """Write scene sample ``b`` into the Mitsuba parameter map, like ``Scene.randomize()``'s update_* tail
         (scene.py:243-342, 371-384), from the host copy made by :meth:`to_host` -- no further device syncs.  Mesh vertices
-        are handed over as slices of the device buffer (``Float32`` takes them through DLPack /
-        ``__cuda_array_interface__`` without a copy)."""
+        and textures are handed over as slices of the device buffers (``Float32`` / ``TensorXf`` take them through
+        DLPack / ``__cuda_array_interface__`` without a copy)."""
         sb, sc = self.batch, self.batch.scene
         params, T = sc._mitsuba_params, sc._types
         world, sampled = self.to_host()
@@ -81,6 +88,9 @@ class BatchResult:
             joined = name + "." + key
             tp = type(params[joined])
             params[joined] = tp(float(sampled[b, row, 0])) if dim == 1 else tp(sampled[b, row, :dim].tolist())
+        for (name, key), (tex, _) in self.textures.items():
+            joined = name + "." + key
+            params[joined] = type(params[joined])(tex[b])
         if update:
             params.update()
 
@@ -119,6 +129,8 @@ class SceneBatch:
         # ---- sampler table ----
         samplers: List[Sampler] = []
         self._attr_rows: Dict[Tuple[str, str], Tuple[int, int]] = {}
+        # texture samplers get rows of their own, numbered in attribute order: (entity, key) -> (row, [H, W], color_a, color_b)
+        self._textures: Dict[Tuple[str, str], tuple] = {}
         trs_rows = []
         for e in ents:
             rows = []
@@ -133,6 +145,9 @@ class SceneBatch:
             if isinstance(e, Mesh) or not e.randomizable():
                 continue
             for key, s in list(e._float_attributes.items()) + list(e._vec3_attributes.items()):
+                if isinstance(s, NoiseTextureLerpSampler):
+                    self._add_texture(e.name(), key, s)
+                    continue
                 self._attr_rows[(e.name(), key)] = (len(samplers), 3 if getattr(s, "_KIND", None) == nat.SAMPLER_SCALAR_TO_VEC3 else s._dim)
                 samplers.append(s)
         for s in samplers:
@@ -158,6 +173,14 @@ class SceneBatch:
         self._frames_keepalive = []
         if self.meshes:
             self._build_meshes()
+
+    def _add_texture(self, name: str, key: str, s: NoiseTextureLerpSampler) -> None:
+        H, W = (int(x) for x in s._texture_shape)
+        if H % PERLIN_TILE or W % PERLIN_TILE:
+            raise ValueError(f"SceneBatch: the texture of {name}.{key} is {H}x{W}; batched Perlin textures need both sides to be "
+                             f"multiples of {PERLIN_TILE} (the largest lattice resolution x 2^(octaves-1) the sampler draws)")
+        colours = [torch.as_tensor(c).detach().to(self.device, torch.float32).reshape(3).contiguous() for c in (s._color_a, s._color_b)]
+        self._textures[(name, key)] = (len(self._textures), (H, W), *colours)
 
     def refresh(self) -> None:
         """Re-read world matrices, centroids, flags and parent links from the python objects."""
@@ -248,7 +271,9 @@ class SceneBatch:
                   out: Optional[BatchResult] = None) -> BatchResult:
         """B scene samples.  Train mode: sample ``sample0 + b`` depends only on (seed, sample0 + b, sampler row)
         -- identical for any batch split or rank layout.  Eval mode: B successive ``sample_eval`` steps per
-        sampler.  ``variates`` ([B,S,3]) switches to injected mode (parity tests).  ``out``: a ``BatchResult`` of an earlier
+        sampler.  ``variates`` ([B,S,3]) switches the scalar samplers to injected mode (parity tests).  Texture
+        samplers draw from Philox in every mode (the reference's eval mode is its train mode), keyed by
+        (seed, sample0 + b, texture row).  ``out``: a ``BatchResult`` of an earlier
         call with the same ``B`` whose tensors are overwritten and returned (no allocation: a loop that runs ahead of the
         device otherwise makes the caching allocator grow by one vertex buffer per step in flight, and a ``cudaMalloc`` of
         B x V x 12 bytes blocks the host for 10-90 ms -- ``scripts/stall_probe2.py``)."""
@@ -299,11 +324,15 @@ class SceneBatch:
             nat.check(L.ffb_transform_vertices(C.byref(mt), self.verts.data_ptr(), E, B, nat.ptr(idx), world.data_ptr(),
                                                verts.data_ptr(), nat.stream()), "ffb_transform_vertices")
             nat.count()
+        textures = {k: perlin_texture_batch(shape, B, ca, cb, seed=self.seed, sample0=int(sample0), row=row,
+                                            out=out.textures[k] if out is not None else None, device=self.device)
+                     for k, (row, shape, ca, cb) in self._textures.items()}
         if out is not None:
+            out.textures = textures
             out._host = None                                # the cached host copy belongs to the overwritten samples
             out._anim_idx = idx
             return out
-        res = BatchResult(world, sampled, verts, self)
+        res = BatchResult(world, sampled, verts, self, textures)
         res._anim_idx = idx                                 # kept for reuse through `out=`
         return res
 
@@ -464,6 +493,8 @@ class PatternStep:
             for t in (res.world, res.sampled, res.vertices):      # produced on the side stream, consumed by the caller on this one
                 if t is not None:
                     t.record_stream(cur)
+            for tex, _ in res.textures.values():
+                tex.record_stream(cur)
         if per_sample is not None:
             from .parallel import fold_allreduce
             dp = fold_allreduce(per_sample, self.pg)        # fold over the samples + the step's only exchange, one kernel on NVLink

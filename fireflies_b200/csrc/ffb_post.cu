@@ -614,9 +614,10 @@ __global__ void __launch_bounds__(256) disc_mask_kernel(const int* __restrict__ 
 }
 
 // ---- Perlin material textures (SURVEY.md 8(f) row 4) ---------------------------------------------------------------
-// rand_perlin_2d_octaves (fireflies/sampling/noise_texture_lerp.py:8-62) with the lattice angles supplied by the caller
-// (the reference draws them with torch.rand on the CPU generator; the Python mirror does the same, so the stream is
-// consumed identically), then NoiseTextureLerpSampler.sample_train's min/max normalisation and colour lerp (:86-98).
+// rand_perlin_2d_octaves (fireflies/sampling/noise_texture_lerp.py:8-62), then NoiseTextureLerpSampler.sample_train's
+// min/max normalisation and colour lerp (:86-98).  ffb_perlin_texture is the single-sample call with the lattice angles
+// supplied by the caller (the reference draws them with torch.rand on the CPU generator; the Python mirror does the same,
+// so the stream is consumed identically).
 __device__ __forceinline__ float torch_lerp(float a, float b, float w) {     // ATen lerp: two-sided form
     const float d = b - a;
     return w < 0.5f ? __fadd_rn(a, __fmul_rn(w, d)) : __fadd_rn(b, -__fmul_rn(d, __fadd_rn(1.f, -w)));
@@ -629,67 +630,205 @@ __device__ __forceinline__ float fade5(float t) {                             //
 __device__ __forceinline__ int f2ord(float f) { const int i = __float_as_int(f); return i >= 0 ? i : i ^ 0x7fffffff; }
 __device__ __forceinline__ float ord2f(int i) { return __int_as_float(i >= 0 ? i : i ^ 0x7fffffff); }
 
-struct PerlinParams {
-    const float* angles;       // per octave (R0+1) x (R1+1) uniforms in [0,1), concatenated
-    int H, W, res0, res1, octaves;
-    float amp[8];              // float32(persistence^k)
-    float* noise;              // [H, W]
-    int* minmax;               // [2] ordered-int min / max
+// B textures per launch, each with its own lattice resolution, octave count and persistence.  The parameters and lattice
+// angles are either given (injected) or drawn here from Philox (include/ffb200.h states the keying):
+//   parameters of sample g = sample0 + b:  r = Philox(seed, (0, lo32(g), hi32(g), PERLIN_TAG_PARAMS | row))
+//   angle of node n of that sample:        u01(Philox(seed, (n, lo32(g), hi32(g), PERLIN_TAG_ANGLES | row))[0])
+// Three launches: perlin_setup_kernel (extrema reset, drawn parameters out), perlin_octaves_kernel (octave sum into the
+// noise buffer and per-sample extrema), perlin_lerp_kernel (normalisation + colour lerp).  The per-texel arithmetic is
+// the reference's, rounding step by rounding step; what depends only on the row (gx, its fade, the lattice row), only
+// on the column, or only on the lattice node (cos / sin of its angle) is evaluated once per CTA tile and octave.
+constexpr uint32_t PERLIN_TAG_PARAMS = 0x9E700000u, PERLIN_TAG_ANGLES = 0x9E710000u;
+constexpr int PT_H = 32, PT_W = 64, PT_THREADS = 256;        // CTA tile: 64 columns x 4 row phases, 8 texels per thread
+constexpr int PT_ROWS = PT_H / (PT_THREADS / PT_W);
+static_assert(PT_THREADS >= 64 + PT_W && PT_H <= 64, "the row table is filled by threads 0..PT_H-1, the column table by 64..64+PT_W-1");
+
+struct PerlinBatch {
+    int B, H, W, row;
+    uint64_t seed, sample0;
+    bool philox;
+    const ffb_perlin_params* prm;   // injected: device [B]; nullptr -> `one` for the single sample
+    ffb_perlin_params one;
+    const float* angles;            // injected lattice angles
+    ffb_perlin_params* prm_out;     // Philox: the drawn parameters (nullable)
+    const float* ca;
+    const float* cb;
+    float* noise;                   // [B, H, W]
+    int* minmax;                    // [B, 2] ordered-int min / max
+    float* out;                     // [B, 3, H, W] or nullptr
 };
 
-__global__ void __launch_bounds__(256) perlin_kernel(PerlinParams q) {
-    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const bool live = t < (long long)q.H * q.W;
-    float acc = 0.f;
-    if (live) {
-        const int i = (int)(t / q.W), j = (int)(t - (long long)i * q.W);
-        const float* ang = q.angles;
-        int f = 1;
-        for (int o = 0; o < q.octaves; ++o, f *= 2) {
-            const int R0 = f * q.res0, R1 = f * q.res1;
-            const int d0 = q.H / R0, d1 = q.W / R1;
-            // torch.arange(0, R, R / shape) is start + i * step in double, stored as float32; then % 1
-            const float a0 = (float)((double)i * ((double)R0 / (double)q.H)), a1 = (float)((double)j * ((double)R1 / (double)q.W));
-            const float gx = a0 - floorf(a0), gy = a1 - floorf(a1);
-            const int ci = i / d0, cj = j / d1;
-            const float TWO_PI = 6.283185307179586f;
-            float n[4];
+// random.randint(1, 6) -> i = 2^k, random.randint(1, 4) -> octaves, random.uniform(0.1, 2.0) -> persistence
+// (noise_texture_lerp.py:77-79): integers by multiply-shift of one 32-bit word, the fp64 uniform from two words the way
+// CPython's random() builds its 53 bits
+__device__ __forceinline__ ffb_perlin_params perlin_draw(uint64_t seed, uint64_t g, int row) {
+    uint32_t r[4];
+    Philox::gen(seed, 0u, (uint32_t)g, (uint32_t)(g >> 32), PERLIN_TAG_PARAMS | (uint32_t)row, r);
+    ffb_perlin_params p;
+    const int k = 1 + (int)(((uint64_t)r[0] * 6u) >> 32);
+    p.res0 = p.res1 = 1 << k;
+    p.octaves = 1 + (int)(((uint64_t)r[1] * 4u) >> 32);
+    p._pad = 0;
+    const double u53 = __dmul_rn(__dadd_rn((double)(r[2] >> 5) * 67108864.0, (double)(r[3] >> 6)), 1.0 / 9007199254740992.0);
+    p.persistence = __dadd_rn(0.1, __dmul_rn(1.9, u53));
+    p.angle_offset = 0;
+    return p;
+}
+
+__device__ __forceinline__ ffb_perlin_params perlin_params(const PerlinBatch& q, int b) {
+    if (q.philox) return perlin_draw(q.seed, q.sample0 + (uint64_t)b, q.row);
+    return q.prm ? q.prm[b] : q.one;
+}
+
+__global__ void __launch_bounds__(128) perlin_setup_kernel(PerlinBatch q) {
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= q.B) return;
+    if (q.philox && q.prm_out) q.prm_out[b] = perlin_draw(q.seed, q.sample0 + (uint64_t)b, q.row);
+    q.minmax[2 * b] = 0x7f800000;                 // ordered(+inf)
+    q.minmax[2 * b + 1] = (int)0x807fffff;        // ordered(-inf)
+}
+
+__global__ void __launch_bounds__(PT_THREADS) perlin_octaves_kernel(PerlinBatch q) {
+    __shared__ float2 node_s[(PT_H + 1) * (PT_W + 1)];     // (cos, sin) of the lattice nodes under the tile
+    __shared__ float4 row_s[PT_H];                          // (gx, fade5(gx), lattice row - first node row)
+    __shared__ float4 col_s[PT_W];                          // (gy, fade5(gy), lattice column - first node column)
+    __shared__ int red_s[2][PT_THREADS / 32];
+    const int b = blockIdx.y, t = threadIdx.x;
+    const ffb_perlin_params p = perlin_params(q, b);
+    const int tiles_x = (q.W + PT_W - 1) / PT_W;
+    const int y0 = (int)(blockIdx.x / tiles_x) * PT_H, x0 = (int)(blockIdx.x % tiles_x) * PT_W;
+    const int yend = min(y0 + PT_H, q.H), xend = min(x0 + PT_W, q.W);
+    const int tx = t % PT_W, ty = t / PT_W, j = x0 + tx;
+    const uint64_t g = q.sample0 + (uint64_t)b;
+    const float* ang = q.philox ? nullptr : q.angles + p.angle_offset;
+    const float TWO_PI = 6.283185307179586f;
+    float acc[PT_ROWS];
 #pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                const int di = k & 1, dj = k >> 1;                   // n00, n10, n01, n11
-                const float th = __fmul_rn(TWO_PI, __ldg(ang + (size_t)(ci + di) * (R1 + 1) + cj + dj));
-                float sn, cs;
-                sincosf(th, &sn, &cs);
-                n[k] = __fadd_rn(__fmul_rn(gx - (float)di, cs), __fmul_rn(gy - (float)dj, sn));
-            }
-            const float t0 = fade5(gx), t1 = fade5(gy);
-            const float v = __fmul_rn(1.4142135623730951f, torch_lerp(torch_lerp(n[0], n[1], t0), torch_lerp(n[2], n[3], t0), t1));
-            acc = __fadd_rn(acc, __fmul_rn(q.amp[o], v));
-            ang += (size_t)(R0 + 1) * (R1 + 1);
+    for (int k = 0; k < PT_ROWS; ++k) acc[k] = 0.f;
+    long long node0 = 0;                                    // index of the octave's first lattice node
+    double amp = 1.0;
+    int f = 1;
+    for (int o = 0; o < p.octaves; ++o, f *= 2) {
+        const int R0 = f * p.res0, R1 = f * p.res1;
+        const int d0 = q.H / R0, d1 = q.W / R1;
+        const int ci0 = y0 / d0, cj0 = x0 / d1;
+        const int nc = (xend - 1) / d1 + 2 - cj0, nn = ((yend - 1) / d0 + 2 - ci0) * nc;
+        // torch.arange(0, R, R / shape) is start + i * step in double, stored as float32; then % 1
+        if (t < PT_H) {
+            const int i = y0 + t;
+            const float a0 = (float)((double)i * ((double)R0 / (double)q.H)), gx = a0 - floorf(a0);
+            row_s[t] = make_float4(gx, fade5(gx), __int_as_float(i / d0 - ci0), 0.f);
+        } else if (t >= 64 && t < 64 + PT_W) {
+            const int jj = x0 + t - 64;
+            const float a1 = (float)((double)jj * ((double)R1 / (double)q.W)), gy = a1 - floorf(a1);
+            col_s[t - 64] = make_float4(gy, fade5(gy), __int_as_float(jj / d1 - cj0), 0.f);
         }
-        q.noise[t] = acc;
+        for (int n = t; n < nn; n += PT_THREADS) {
+            const int r = n / nc, c = n - r * nc;
+            const long long idx = node0 + (long long)(ci0 + r) * (R1 + 1) + cj0 + c;
+            float u;
+            if (q.philox) {
+                uint32_t w[4];
+                Philox::gen(q.seed, (uint32_t)idx, (uint32_t)g, (uint32_t)(g >> 32), PERLIN_TAG_ANGLES | (uint32_t)q.row, w);
+                u = Philox::u01(w[0]);
+            } else {
+                u = __ldg(ang + idx);
+            }
+            float sn, cs;
+            sincosf(__fmul_rn(TWO_PI, u), &sn, &cs);
+            node_s[n] = make_float2(cs, sn);
+        }
+        __syncthreads();
+        const float4 cv = col_s[tx];
+        const float gy = cv.x, t1 = cv.y;
+        const int lj = __float_as_int(cv.z);
+        const float a32 = (float)amp;                       // float32(persistence^o): the running fp64 product, rounded
+#pragma unroll
+        for (int k = 0; k < PT_ROWS; ++k) {
+            const int r = ty + k * (PT_THREADS / PT_W);
+            if (y0 + r < yend && j < xend) {
+                const float4 rv = row_s[r];
+                const float gx = rv.x, t0 = rv.y;
+                const float2* nd = node_s + __float_as_int(rv.z) * nc + lj;
+                const float2 e00 = nd[0], e10 = nd[nc], e01 = nd[1], e11 = nd[nc + 1];
+                const float n00 = __fadd_rn(__fmul_rn(gx, e00.x), __fmul_rn(gy, e00.y));
+                const float n10 = __fadd_rn(__fmul_rn(gx - 1.f, e10.x), __fmul_rn(gy, e10.y));
+                const float n01 = __fadd_rn(__fmul_rn(gx, e01.x), __fmul_rn(gy - 1.f, e01.y));
+                const float n11 = __fadd_rn(__fmul_rn(gx - 1.f, e11.x), __fmul_rn(gy - 1.f, e11.y));
+                const float v = __fmul_rn(1.4142135623730951f, torch_lerp(torch_lerp(n00, n10, t0), torch_lerp(n01, n11, t0), t1));
+                acc[k] = __fadd_rn(acc[k], __fmul_rn(a32, v));
+            }
+        }
+        __syncthreads();
+        amp *= p.persistence;
+        node0 += (long long)(R0 + 1) * (R1 + 1);
     }
-    float mn = live ? acc : INFINITY, mx = live ? acc : -INFINITY;
+    float mn = INFINITY, mx = -INFINITY;
+    float* nz = q.noise + (size_t)b * q.H * q.W;
+#pragma unroll
+    for (int k = 0; k < PT_ROWS; ++k) {
+        const int i = y0 + ty + k * (PT_THREADS / PT_W);
+        if (i < yend && j < xend) {
+            nz[(size_t)i * q.W + j] = acc[k];
+            mn = fminf(mn, acc[k]);
+            mx = fmaxf(mx, acc[k]);
+        }
+    }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
         mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
     }
-    if ((threadIdx.x & 31) == 0) {
-        atomicMin(q.minmax, f2ord(mn));
-        atomicMax(q.minmax + 1, f2ord(mx));
+    if ((t & 31) == 0) { red_s[0][t >> 5] = f2ord(mn); red_s[1][t >> 5] = f2ord(mx); }
+    __syncthreads();
+    if (t == 0) {
+        int a = red_s[0][0], z = red_s[1][0];
+        for (int w = 1; w < PT_THREADS / 32; ++w) { a = min(a, red_s[0][w]); z = max(z, red_s[1][w]); }
+        atomicMin(q.minmax + 2 * b, a);
+        atomicMax(q.minmax + 2 * b + 1, z);
     }
 }
 
-// out[c, i, j] = lerp(color_a[c], color_b[c], (noise - min) / (max - min))
-__global__ void __launch_bounds__(256) noise_lerp_kernel(const float* __restrict__ noise, const int* __restrict__ minmax, long long n,
-                                                         const float* __restrict__ ca, const float* __restrict__ cb, float* __restrict__ out) {
-    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= n) return;
-    const float mn = ord2f(minmax[0]), mx = ord2f(minmax[1]);
-    const float w = __fdiv_rn(noise[t] - mn, mx - mn);
+// out[b, c, i, j] = lerp(color_a[c], color_b[c], (noise[b, i, j] - min_b) / (max_b - min_b)), four texels per thread
+__global__ void __launch_bounds__(256) perlin_lerp_kernel(PerlinBatch q) {
+    const int b = blockIdx.y;
+    const long long n = (long long)q.H * q.W, t0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 4;
+    if (t0 >= n) return;
+    const float mn = ord2f(q.minmax[2 * b]), mx = ord2f(q.minmax[2 * b + 1]);
+    const float* nz = q.noise + (size_t)b * n;
+    float* o = q.out + (size_t)b * 3 * n;
+    float ca[3], cb[3];
 #pragma unroll
-    for (int c = 0; c < 3; ++c) out[(size_t)c * n + t] = torch_lerp(__ldg(ca + c), __ldg(cb + c), w);
+    for (int c = 0; c < 3; ++c) { ca[c] = __ldg(q.ca + c); cb[c] = __ldg(q.cb + c); }
+    if ((n & 3) == 0) {
+        const float4 v = *reinterpret_cast<const float4*>(nz + t0);
+        const float w0 = __fdiv_rn(v.x - mn, mx - mn), w1 = __fdiv_rn(v.y - mn, mx - mn);
+        const float w2 = __fdiv_rn(v.z - mn, mx - mn), w3 = __fdiv_rn(v.w - mn, mx - mn);
+#pragma unroll
+        for (int c = 0; c < 3; ++c)
+            *reinterpret_cast<float4*>(o + (size_t)c * n + t0) = make_float4(torch_lerp(ca[c], cb[c], w0), torch_lerp(ca[c], cb[c], w1),
+                                                                             torch_lerp(ca[c], cb[c], w2), torch_lerp(ca[c], cb[c], w3));
+    } else {
+        for (long long t = t0; t < t0 + 4 && t < n; ++t) {
+            const float w = __fdiv_rn(nz[t] - mn, mx - mn);
+#pragma unroll
+            for (int c = 0; c < 3; ++c) o[(size_t)c * n + t] = torch_lerp(ca[c], cb[c], w);
+        }
+    }
+}
+
+static int perlin_launch(const PerlinBatch& q, cudaStream_t st) {
+    perlin_setup_kernel<<<(unsigned)((q.B + 127) / 128), 128, 0, st>>>(q);
+    FFB_CUDA(cudaGetLastError());
+    const unsigned tiles = (unsigned)(((q.W + PT_W - 1) / PT_W) * ((q.H + PT_H - 1) / PT_H));
+    perlin_octaves_kernel<<<dim3(tiles, q.B), PT_THREADS, 0, st>>>(q);
+    FFB_CUDA(cudaGetLastError());
+    if (q.out) {
+        const long long n4 = ((long long)q.H * q.W + 3) / 4;
+        perlin_lerp_kernel<<<dim3((unsigned)((n4 + 255) / 256), q.B), 256, 0, st>>>(q);
+        FFB_CUDA(cudaGetLastError());
+    }
+    return 0;
 }
 
 }  // namespace post
@@ -705,25 +844,55 @@ extern "C" int ffb_perlin_texture(const float* angles, int32_t H, int32_t W, int
         return fail_arg(FFB_E_ARG, "perlin_texture: bad argument");
     if (octaves < 1 || octaves > 8) return fail_arg(FFB_E_LIMIT, "perlin_texture: 1..8 octaves");
     if (out && (!color_a || !color_b)) return fail_arg(FFB_E_ARG, "perlin_texture: colours required with an output");
-    const int top = 1 << (octaves - 1);
-    if (H % (res0 * top) != 0 || W % (res1 * top) != 0)
+    if (H % ((int64_t)res0 << (octaves - 1)) != 0 || W % ((int64_t)res1 << (octaves - 1)) != 0)
         return fail_arg(FFB_E_ARG, "perlin_texture: shape must be a multiple of res * 2^(octaves-1) (as in the reference, whose tiling fails otherwise)");
-    PerlinParams q;
-    q.angles = angles; q.H = H; q.W = W; q.res0 = res0; q.res1 = res1; q.octaves = octaves;
-    double a = 1.0;
-    for (int o = 0; o < 8; ++o) { q.amp[o] = (float)a; a *= persistence; }
-    q.noise = noise_scratch; q.minmax = minmax_scratch;
+    PerlinBatch q;
+    memset(&q, 0, sizeof(q));
+    q.B = 1; q.H = H; q.W = W;
+    q.one.res0 = res0; q.one.res1 = res1; q.one.octaves = octaves; q.one.persistence = persistence;
+    q.angles = angles; q.ca = color_a; q.cb = color_b;
+    q.noise = noise_scratch; q.minmax = minmax_scratch; q.out = out;
+    return perlin_launch(q, as_stream(stream));
+}
+
+extern "C" int ffb_perlin_texture_batch(int32_t B, int32_t H, int32_t W, uint64_t seed, uint64_t sample0, int32_t row,
+                                        const ffb_perlin_params* params_host, const float* angles, int64_t n_angles,
+                                        ffb_perlin_params* params_out, const float* color_a, const float* color_b, float* noise,
+                                        int32_t* minmax, float* out, void* stream) {
+    if (!noise || !minmax || B <= 0 || H <= 0 || W <= 0) return fail_arg(FFB_E_ARG, "perlin_texture_batch: bad argument");
+    if (B > 65535) return fail_arg(FFB_E_LIMIT, "perlin_texture_batch: B > 65535");
+    if (out && (!color_a || !color_b)) return fail_arg(FFB_E_ARG, "perlin_texture_batch: colours required with an output");
+    PerlinBatch q;
+    memset(&q, 0, sizeof(q));
+    q.B = B; q.H = H; q.W = W; q.seed = seed; q.sample0 = sample0; q.row = row;
+    q.ca = color_a; q.cb = color_b; q.noise = noise; q.minmax = minmax; q.out = out;
     cudaStream_t st = as_stream(stream);
-    const int init[2] = {0x7f800000, (int)0x807fffff};       // ordered(+inf), ordered(-inf)
-    FFB_CUDA(cudaMemcpyAsync(minmax_scratch, init, sizeof(init), cudaMemcpyHostToDevice, st));
-    const long long n = (long long)H * W;
-    perlin_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(q);
-    FFB_CUDA(cudaGetLastError());
-    if (out) {
-        noise_lerp_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(noise_scratch, minmax_scratch, n, color_a, color_b, out);
-        FFB_CUDA(cudaGetLastError());
+    if (!params_host) {
+        if (angles) return fail_arg(FFB_E_ARG, "perlin_texture_batch: lattice angles are drawn in Philox mode (angles must be NULL)");
+        if (row < 0 || row > 0xffff) return fail_arg(FFB_E_LIMIT, "perlin_texture_batch: sampler row must be in 0..65535");
+        if (H % FFB_PERLIN_TILE != 0 || W % FFB_PERLIN_TILE != 0)
+            return fail_arg(FFB_E_ARG, "perlin_texture_batch: Philox mode needs H and W to be multiples of 512 (the largest i * 2^(octaves-1) it draws)");
+        q.philox = true;
+        q.prm_out = params_out;
+        return perlin_launch(q, st);
     }
-    return 0;
+    if (!angles || !params_out) return fail_arg(FFB_E_ARG, "perlin_texture_batch: injected mode needs angles and params_out");
+    for (int b = 0; b < B; ++b) {
+        const ffb_perlin_params& p = params_host[b];
+        if (p.res0 <= 0 || p.res1 <= 0 || p.octaves < 1 || p.octaves > 8)
+            return fail_arg(FFB_E_ARG, "perlin_texture_batch: injected parameters need res > 0 and 1..8 octaves");
+        const int64_t top0 = (int64_t)p.res0 << (p.octaves - 1), top1 = (int64_t)p.res1 << (p.octaves - 1);
+        if (H % top0 != 0 || W % top1 != 0)
+            return fail_arg(FFB_E_ARG, "perlin_texture_batch: shape must be a multiple of res * 2^(octaves-1) for every sample");
+        int64_t nodes = 0;
+        for (int o = 0; o < p.octaves; ++o) nodes += (((int64_t)p.res0 << o) + 1) * (((int64_t)p.res1 << o) + 1);
+        if (p.angle_offset < 0 || p.angle_offset > n_angles - nodes)
+            return fail_arg(FFB_E_ARG, "perlin_texture_batch: a sample's lattice angles run past the end of `angles`");
+    }
+    FFB_CUDA(cudaMemcpyAsync(params_out, params_host, (size_t)B * sizeof(ffb_perlin_params), cudaMemcpyHostToDevice, st));
+    q.prm = params_out;
+    q.angles = angles;
+    return perlin_launch(q, st);
 }
 
 static int postprocess_impl(const ffb_post_desc* d, const float* img, const uint8_t* gates, const double* noise_injected,

@@ -340,6 +340,39 @@ FFB_API int ffb_perlin_texture(const float* angles, int32_t H, int32_t W, int32_
                        double persistence, const float* color_a, const float* color_b, float* noise_scratch,
                        int32_t* minmax_scratch, float* out, void* stream);
 
+/* The parameters of one Perlin texture. */
+typedef struct ffb_perlin_params {
+    int32_t res0, res1;     /* lattice resolution (drawn: res0 = res1 = 2^k)                    */
+    int32_t octaves;        /* 1..8 (drawn: 1..4)                                               */
+    int32_t _pad;
+    double  persistence;    /* octave o has amplitude float32(persistence^o)                    */
+    int64_t angle_offset;   /* injected: index in `angles` of the sample's first lattice angle  */
+} ffb_perlin_params;
+
+#define FFB_PERLIN_TILE 512 /* Philox mode: H and W multiples of this, the largest res * 2^(octaves-1) it draws (64 * 8) */
+
+/* B Perlin textures in one call, each with its own parameters: ffb_perlin_texture per sample.  noise f32 [B,H,W],
+ * minmax int32 [B,2] (ordered-int extrema per sample), out (nullable) f32 [B,3,H,W]; colours f32 [3], shared by the
+ * samples.  Every buffer is DEVICE memory; the call enqueues three kernels on `stream` and never waits for the device.
+ *   Injected mode (params_host != NULL): params_host HOST [B]; each sample's angles are the concatenated per-octave
+ *     (f*res0+1) x (f*res1+1) lattices of ffb_perlin_texture, starting at angles[angle_offset] (angles f32 [n_angles]).
+ *     The parameters are checked here, then copied into params_out (DEVICE [B], required), which the kernels read.
+ *     The texture of each sample is bit-identical to ffb_perlin_texture fed the same parameters and angles.
+ *   Philox mode (params_host == NULL, angles == NULL): H and W multiples of FFB_PERLIN_TILE, 0 <= row <= 65535.
+ *     Sample g = sample0 + b of sampler `row` draws, with r = Philox4x32-10(key = seed,
+ *     counter = (0, lo32(g), hi32(g), 0x9E700000 | row)):
+ *       k           = 1 + (r[0] * 6 >> 32)           res0 = res1 = 2^k        (random.randint(1, 6))
+ *       octaves     = 1 + (r[1] * 4 >> 32)                                    (random.randint(1, 4))
+ *       persistence = 0.1 + 1.9 * u53, u53 = ((r[2] >> 5) * 2^26 + (r[3] >> 6)) / 2^53, in fp64 (random.uniform(0.1, 2.0))
+ *     and the angle of its lattice node n (the index into the concatenation above, octave by octave, row-major) is
+ *       u = (w[0] >> 8) / 2^24, w = Philox4x32-10(key = seed, counter = (n, lo32(g), hi32(g), 0x9E710000 | row)).
+ *     A texture depends only on (seed, sample0 + b, row): never on B or on how samples are split over calls.
+ *     params_out (nullable) DEVICE [B] receives the drawn parameters (angle_offset = 0). */
+FFB_API int ffb_perlin_texture_batch(int32_t B, int32_t H, int32_t W, uint64_t seed, uint64_t sample0, int32_t row,
+                       const ffb_perlin_params* params_host, const float* angles, int64_t n_angles,
+                       ffb_perlin_params* params_out, const float* color_a, const float* color_b, float* noise,
+                       int32_t* minmax, float* out, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * 5. NURBS-curve camera paths and batched intersections  (fireflies/entity/curve.py, utils/intersections.py)
  * ------------------------------------------------------------------------------------------ */
