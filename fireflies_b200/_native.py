@@ -86,6 +86,8 @@ SIGNATURES = {
     "ffb_transform_vertices": (C.c_int, [C.POINTER(MeshTable), _P, C.c_int32, C.c_int32, _P, _P, _P, _P]),
     "ffb_transform_points": (C.c_int, [_P, C.c_int64, _P, C.c_int, _P, _P]),
     "ffb_transform_points_bwd": (C.c_int, [_P, C.c_int64, _P, C.c_int, _P, _P, _P]),
+    "ffb_transform_bwd_workspace_bytes": (C.c_size_t, [C.c_int64]),
+    "ffb_transform_points_bwd_full": (C.c_int, [_P, C.c_int64, _P, C.c_int, _P, _P, _P, _P, C.c_size_t, _P]),
     "ffb_rays_to_ndc": (C.c_int, [_P, C.c_int32, _P, _P, _P]),
     "ffb_clamp_to_fov": (C.c_int, [_P, C.c_int32, _P, _P, C.c_float, C.c_float, _P, _P]),
     "ffb_silhouette": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P]),

@@ -547,7 +547,9 @@ class TextureStep:
     ``backward(g_tex)`` takes the renderer's gradients w.r.t. that texture for this rank's samples (``[B, ts1, ts0, 3]`` or
     ``[ts1, ts0, 3]``) and returns ``d loss / d rays`` ``[N, 3]`` summed over the samples and all ranks of
     ``process_group``, also accumulated into ``laser._rays.grad`` the way autograd would (so ``torch.optim.Adam([laser._rays])``
-    works unchanged).  Every scene of the step sees the same texture and every backward stage is linear in the upstream
+    works unchanged).  When ``laser._perspective`` requires grad, the same pass of the ray projection's backward also gives
+    ``d loss / d _perspective`` [4, 4], which travels in the same exchange and is accumulated into ``laser._perspective.grad``
+    in its dtype.  Every scene of the step sees the same texture and every backward stage is linear in the upstream
     gradient, so the B gradients are folded first and the blur adjoint, the splat backward and the ray projection's backward
     run once per step.  No autograd graph is built; the step's buffers are allocated by the first call and reused (the
     returned tensor is overwritten by the next ``backward``)."""
@@ -566,7 +568,7 @@ class TextureStep:
         from .postprocessing.base import run_postprocess
         L = nat.lib()
         rays = nat.require_cuda(self.laser._rays.detach().float().contiguous(), torch.float32, "laser._rays")
-        M = self.laser._M()
+        M = self.laser._M().detach()
         N = rays.shape[0]
         ndc = torch.empty_like(rays)
         nat.check(L.ffb_transform_points(rays.data_ptr(), N, M.data_ptr(), 0, ndc.data_ptr(), nat.stream()), "ffb_transform_points")
@@ -585,10 +587,13 @@ class TextureStep:
         b = self._bufs
         if b is None or b["d_rays"].shape[0] != N or b["d_rays"].device != dev:
             d_ndc = torch.zeros((N, 3), dtype=torch.float32, device=dev)        # column 2 stays 0: d ndc = (dx, dy, 0)
+            packed = torch.empty(3 * N + 16, dtype=torch.float32, device=dev)   # [d_rays, d_perspective]: one exchange
             b = self._bufs = {"g1": torch.empty((1, self.ts1, self.ts0), dtype=torch.float32, device=dev),
                               "g_in": torch.empty((1, self.ts1, self.ts0), dtype=torch.float32, device=dev),
                               "d_pts": torch.empty((1, N, 2), dtype=torch.float32, device=dev),
-                              "d_ndc": d_ndc, "d_rays": torch.empty((N, 3), dtype=torch.float32, device=dev)}
+                              "d_ndc": d_ndc, "packed": packed, "d_rays": packed[:3 * N].view(N, 3),
+                              "d_K": packed[3 * N:].view(4, 4),
+                              "ws": torch.empty(nat.lib().ffb_transform_bwd_workspace_bytes(N), dtype=torch.uint8, device=dev)}
         return b
 
     def backward(self, g_tex: torch.Tensor) -> torch.Tensor:
@@ -611,13 +616,30 @@ class TextureStep:
             g_sum = gaussian_blur2d_backward(b["g1"], *self.blur, out=b["g_in"])
         d_pts = plan.backward(pts, g_sum, None, False, out=b["d_pts"])
         b["d_ndc"][:, 0:2].copy_(d_pts[0])
-        nat.check(nat.lib().ffb_transform_points_bwd(rays.data_ptr(), N, M.data_ptr(), 0, b["d_ndc"].data_ptr(), b["d_rays"].data_ptr(),
-                                                     nat.stream()), "ffb_transform_points_bwd")
-        nat.count()
-        d_rays = allreduce_sum_(b["d_rays"], self.pg)
-        target = self.laser._rays
-        if target.grad is None:
-            target.grad = d_rays.to(target.dtype, copy=True)
+        K = self.laser._perspective
+        if not K.requires_grad:
+            nat.check(nat.lib().ffb_transform_points_bwd(rays.data_ptr(), N, M.data_ptr(), 0, b["d_ndc"].data_ptr(), b["d_rays"].data_ptr(),
+                                                         nat.stream()), "ffb_transform_points_bwd")
+            nat.count()
+            d_rays = allreduce_sum_(b["d_rays"], self.pg)
         else:
-            target.grad.add_(d_rays.to(target.dtype))
+            ws = b["ws"]
+            nat.check(nat.lib().ffb_transform_points_bwd_full(rays.data_ptr(), N, M.data_ptr(), 0, b["d_ndc"].data_ptr(),
+                                                              b["d_rays"].data_ptr(), b["d_K"].data_ptr(),
+                                                              ws.data_ptr() if ws.numel() else None, ws.numel(), nat.stream()),
+                      "ffb_transform_points_bwd_full")
+            nat.count(2 if ws.numel() else 1)
+            b["d_K"][:, 1].neg_()                       # d_M -> d_perspective: M = K @ FLIP_Y, d_K = d_M @ FLIP_Y^T
+            allreduce_sum_(b["packed"], self.pg)
+            d_rays = b["d_rays"]
+            _accumulate_grad(K, b["d_K"])
+        _accumulate_grad(self.laser._rays, d_rays)
         return d_rays
+
+
+def _accumulate_grad(target: torch.Tensor, d: torch.Tensor) -> None:
+    """``target.grad += d`` in the target's dtype, creating the gradient on first use, the way autograd accumulates a leaf."""
+    if target.grad is None:
+        target.grad = d.to(target.dtype, copy=True)
+    else:
+        target.grad.add_(d.to(target.dtype))

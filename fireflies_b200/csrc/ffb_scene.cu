@@ -5,7 +5,7 @@
 //   gaussian_distribution.py:19-20, animation.py:27-45          -> ffb_sample, ffb_sample_anim_index
 //   fireflies/utils/math.py:24-60,203-209; entity/base.py:194-244; entity/mesh.py:131-150
 //                                                                -> ffb_compose_world
-//   fireflies/utils/math.py:220-235; entity/mesh.py:158-165,183-198 -> ffb_transform_vertices/points
+//   fireflies/utils/math.py:220-235; entity/mesh.py:158-165,183-198 -> ffb_transform_vertices/points(_bwd, _bwd_full)
 //   fireflies/projection/laser.py:199-206,262-290                -> ffb_rays_to_ndc, ffb_clamp_to_fov
 //
 // The reference spends ~190 tiny aten ops and 12 host syncs per entity per sample (SURVEY.md 0-7); here a
@@ -245,41 +245,46 @@ __device__ __forceinline__ void xform_dir(const float* T, float x, float y, floa
     oz = fmaf(T[8], x, fmaf(T[9], y, T[10] * z));
 }
 
+// 4 consecutive xyz vertices (48 B) at s: three 128-bit accesses when all four exist (n == 12 floats) and s is 16-byte
+// aligned, scalar accesses otherwise (misaligned storage, tail); missing floats read as 0
+__device__ __forceinline__ void ld_vert4(const float* __restrict__ s, int n, float v[12]) {
+    if (n == 12 && ((reinterpret_cast<uintptr_t>(s) & 15) == 0)) {
+        const float4 a = __ldg(reinterpret_cast<const float4*>(s));
+        const float4 b = __ldg(reinterpret_cast<const float4*>(s) + 1);
+        const float4 c = __ldg(reinterpret_cast<const float4*>(s) + 2);
+        v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
+        v[8] = c.x; v[9] = c.y; v[10] = c.z; v[11] = c.w;
+    } else {
+#pragma unroll
+        for (int k = 0; k < 12; ++k) v[k] = k < n ? __ldg(s + k) : 0.f;
+    }
+}
+__device__ __forceinline__ void st_vert4(float* __restrict__ d, int n, const float v[12]) {
+    if (n == 12 && ((reinterpret_cast<uintptr_t>(d) & 15) == 0)) {
+        reinterpret_cast<float4*>(d)[0] = make_float4(v[0], v[1], v[2], v[3]);
+        reinterpret_cast<float4*>(d)[1] = make_float4(v[4], v[5], v[6], v[7]);
+        reinterpret_cast<float4*>(d)[2] = make_float4(v[8], v[9], v[10], v[11]);
+    } else {
+#pragma unroll
+        for (int k = 0; k < 12; ++k)
+            if (k < n) d[k] = v[k];
+    }
+}
+
 template <bool DIRS>
 __device__ __forceinline__ void xform_block4(const float* __restrict__ src, float* __restrict__ dst, long long v0, long long V,
                                              const float* T) {
     // src/dst point at vertex 0 of the mesh; this thread owns vertices [v0, v0+4)
     if (v0 >= V) return;
-    const float* s = src + v0 * 3;
-    float* d = dst + v0 * 3;
+    const int n = v0 + 4 <= V ? 12 : (int)(V - v0) * 3;
     float in[12], o[12];
-    const bool full = v0 + 4 <= V;
-    if (full && ((reinterpret_cast<uintptr_t>(s) & 15) == 0)) {
-        const float4 a = __ldg(reinterpret_cast<const float4*>(s));
-        const float4 b = __ldg(reinterpret_cast<const float4*>(s) + 1);
-        const float4 c = __ldg(reinterpret_cast<const float4*>(s) + 2);
-        in[0] = a.x; in[1] = a.y; in[2] = a.z; in[3] = a.w; in[4] = b.x; in[5] = b.y; in[6] = b.z; in[7] = b.w;
-        in[8] = c.x; in[9] = c.y; in[10] = c.z; in[11] = c.w;
-    } else {
-        const int n = full ? 12 : (int)(V - v0) * 3;
-#pragma unroll
-        for (int k = 0; k < 12; ++k) in[k] = k < n ? __ldg(s + k) : 0.f;
-    }
+    ld_vert4(src + v0 * 3, n, in);
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
         if (DIRS) xform_dir(T, in[3 * k], in[3 * k + 1], in[3 * k + 2], o[3 * k], o[3 * k + 1], o[3 * k + 2]);
         else xform_point(T, in[3 * k], in[3 * k + 1], in[3 * k + 2], o[3 * k], o[3 * k + 1], o[3 * k + 2]);
     }
-    if (full && ((reinterpret_cast<uintptr_t>(d) & 15) == 0)) {
-        reinterpret_cast<float4*>(d)[0] = make_float4(o[0], o[1], o[2], o[3]);
-        reinterpret_cast<float4*>(d)[1] = make_float4(o[4], o[5], o[6], o[7]);
-        reinterpret_cast<float4*>(d)[2] = make_float4(o[8], o[9], o[10], o[11]);
-    } else {
-        const int n = full ? 12 : (int)(V - v0) * 3;
-#pragma unroll
-        for (int k = 0; k < 12; ++k)
-            if (k < n) d[k] = o[k];
-    }
+    st_vert4(dst + v0 * 3, n, o);
 }
 
 __global__ void __launch_bounds__(VT_THREADS) transform_vertices_kernel(const ffb_mesh_table mt, const float* __restrict__ verts,
@@ -318,33 +323,119 @@ __global__ void __launch_bounds__(VT_THREADS) transform_points_kernel(const floa
     xform_block4<DIRS>(pts, out, ((long long)blockIdx.x * VT_THREADS + threadIdx.x) * VT_PER_THREAD, V, T);
 }
 
-// backward of transform_points / transform_directions w.r.t. the points (the laser rays are optimised
-// through projectRaysToNDC, projection/laser.py:262-275): y = h[:3]/h[3], h = T @ [x,1]
+// backward of transform_points / transform_directions (utils/math.py:220-235, torch autograd of a broadcast matmul in the
+// reference; the laser rays and the projector / camera matrices are optimised through it, projection/laser.py:262-275).
+// Per point: y = h[:3] / h[3] with h = T @ [p, 1] (points) or y = (T @ [p, 0])[:3] (directions), d = dL/dh, then
+//   d_pts[v] = (T^T d)[:3]            and            d_T[i][j] = sum_v d_i(v) p~_j(v),  p~ = (x, y, z, 1) or (x, y, z, 0).
+// One template serves the points-only backward (DT off: one 4-vertex group per thread, 64-thread CTAs) and the
+// matrix gradient (DT on: a grid-stride loop over at most TB_MAX_CTAS CTAs, fp32 sums per thread, an fp32 shuffle tree per
+// warp, a fixed-order sum over the 8 warps, one 16-float partial per CTA).  The grid depends on V only -- not on the device
+// -- so the summation order, and with it every bit of d_T, is the same on every call.
+constexpr int TB_MAX_CTAS = 3 * kNumSMs;      // all resident at once: 3 CTAs x 256 threads per SM (<= 80 registers)
+constexpr int TB_PTS_THREADS = 64;            // points only: small CTAs spread the V / 4 threads over every SM
+constexpr int TB_FOLD_THREADS = 1024;
+
+__host__ __device__ constexpr long long transform_bwd_grid(long long V, bool dT) {
+    return dT ? ((V + VT_CHUNK - 1) / VT_CHUNK > TB_MAX_CTAS ? TB_MAX_CTAS : (V + VT_CHUNK - 1) / VT_CHUNK)
+              : (V + TB_PTS_THREADS * VT_PER_THREAD - 1) / (TB_PTS_THREADS * VT_PER_THREAD);
+}
+
 template <bool DIRS>
-__global__ void __launch_bounds__(128) transform_points_bwd_kernel(const float* __restrict__ pts, long long V,
-                                                                   const float* __restrict__ Tg, const float* __restrict__ g,
-                                                                   float* __restrict__ d_pts) {
-    const long long v = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (v >= V) return;
-    float T[16];
-#pragma unroll
-    for (int k = 0; k < 16; ++k) T[k] = Tg[k];
-    const float x = pts[3 * v], y = pts[3 * v + 1], z = pts[3 * v + 2];
-    const float g0 = g[3 * v], g1 = g[3 * v + 1], g2 = g[3 * v + 2];
-    float d0, d1, d2, d3;
-    if (DIRS) { d0 = g0; d1 = g1; d2 = g2; d3 = 0.f; }
+__device__ __forceinline__ void xform_bwd_point(const float* T, float x, float y, float z, float g0, float g1, float g2, float d[4]) {
+    if (DIRS) { d[0] = g0; d[1] = g1; d[2] = g2; d[3] = 0.f; }
     else {
         const float h0 = fmaf(T[0], x, fmaf(T[1], y, fmaf(T[2], z, T[3])));
         const float h1 = fmaf(T[4], x, fmaf(T[5], y, fmaf(T[6], z, T[7])));
         const float h2 = fmaf(T[8], x, fmaf(T[9], y, fmaf(T[10], z, T[11])));
         const float h3 = fmaf(T[12], x, fmaf(T[13], y, fmaf(T[14], z, T[15])));
         const float inv = 1.0f / h3;
-        d0 = g0 * inv; d1 = g1 * inv; d2 = g2 * inv;
-        d3 = -(g0 * h0 + g1 * h1 + g2 * h2) * inv * inv;
+        d[0] = g0 * inv; d[1] = g1 * inv; d[2] = g2 * inv;
+        d[3] = -(g0 * h0 + g1 * h1 + g2 * h2) * inv * inv;
     }
-    d_pts[3 * v] = fmaf(T[0], d0, fmaf(T[4], d1, fmaf(T[8], d2, T[12] * d3)));
-    d_pts[3 * v + 1] = fmaf(T[1], d0, fmaf(T[5], d1, fmaf(T[9], d2, T[13] * d3)));
-    d_pts[3 * v + 2] = fmaf(T[2], d0, fmaf(T[6], d1, fmaf(T[10], d2, T[14] * d3)));
+}
+
+// DT: `out` receives d_T itself when gridDim.x == 1, else this CTA's partial at out + 16 * blockIdx.x
+template <bool DIRS, bool DPTS, bool DT, int THREADS = DT ? VT_THREADS : TB_PTS_THREADS>
+__global__ void __launch_bounds__(THREADS, 3 * VT_THREADS / THREADS) transform_bwd_kernel(const float* __restrict__ pts, long long V,
+                                                                      const float* __restrict__ Tg, const float* __restrict__ g,
+                                                                      float* __restrict__ d_pts, float* __restrict__ out) {
+    __shared__ float red[THREADS / 32][16];
+    const float* T = Tg;                       // read where used: the loads overlap the first points' (no staging barrier)
+    constexpr int R = DIRS ? 3 : 4;            // directions: row 3 and column 3 of d_T are zero
+    float acc[16];
+#pragma unroll
+    for (int k = 0; k < 16; ++k) acc[k] = 0.f;
+    for (long long v0 = ((long long)blockIdx.x * THREADS + threadIdx.x) * VT_PER_THREAD; v0 < V;
+         v0 += (long long)gridDim.x * THREADS * VT_PER_THREAD) {
+        const int n = v0 + 4 <= V ? 12 : (int)(V - v0) * 3;
+        float p[12], gi[12], o[12];
+        ld_vert4(pts + v0 * 3, n, p);
+        ld_vert4(g + v0 * 3, n, gi);
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const float x = p[3 * k], y = p[3 * k + 1], z = p[3 * k + 2];
+            float d[4];
+            xform_bwd_point<DIRS>(T, x, y, z, gi[3 * k], gi[3 * k + 1], gi[3 * k + 2], d);
+            if (DPTS) {
+                o[3 * k] = fmaf(T[0], d[0], fmaf(T[4], d[1], fmaf(T[8], d[2], T[12] * d[3])));
+                o[3 * k + 1] = fmaf(T[1], d[0], fmaf(T[5], d[1], fmaf(T[9], d[2], T[13] * d[3])));
+                o[3 * k + 2] = fmaf(T[2], d[0], fmaf(T[6], d[1], fmaf(T[10], d[2], T[14] * d[3])));
+            }
+            if (DT && 3 * k < n) {
+#pragma unroll
+                for (int i = 0; i < R; ++i) {
+                    acc[4 * i] = fmaf(d[i], x, acc[4 * i]);
+                    acc[4 * i + 1] = fmaf(d[i], y, acc[4 * i + 1]);
+                    acc[4 * i + 2] = fmaf(d[i], z, acc[4 * i + 2]);
+                    if (!DIRS) acc[4 * i + 3] += d[i];
+                }
+            }
+        }
+        if (DPTS) st_vert4(d_pts + v0 * 3, n, o);
+    }
+    if (!DT) return;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int k = 0; k < 16; ++k) {
+        if (k / 4 < R && (k % 4) < R) {
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) acc[k] += __shfl_xor_sync(0xffffffffu, acc[k], off);
+        }
+        if (lane == 0) red[warp][k] = acc[k];
+    }
+    __syncthreads();
+    if (threadIdx.x < 16) {
+        float s = red[0][threadIdx.x];
+#pragma unroll
+        for (int w = 1; w < THREADS / 32; ++w) s += red[w][threadIdx.x];
+        out[(gridDim.x == 1 ? 0 : 16 * blockIdx.x) + threadIdx.x] = s;
+    }
+}
+
+// d_T = sum of the G partials in fp64: 64 row groups sum every 64th partial in turn, then a fixed pairwise tree
+__global__ void __launch_bounds__(TB_FOLD_THREADS) transform_bwd_fold_kernel(const float* __restrict__ partials, int G,
+                                                                             float* __restrict__ d_T) {
+    constexpr int ROWS = TB_FOLD_THREADS / 16;
+    __shared__ double s[ROWS][16];
+    const int j = threadIdx.x & 15, r = threadIdx.x >> 4;
+    double a = 0.0;
+    for (int c = r; c < G; c += ROWS) a += (double)partials[16 * c + j];
+    s[r][j] = a;
+    __syncthreads();
+#pragma unroll
+    for (int h = ROWS / 2; h > 0; h >>= 1) {
+        if (r < h) s[r][j] += s[r + h][j];
+        __syncthreads();
+    }
+    if (threadIdx.x < 16) d_T[threadIdx.x] = (float)s[0][threadIdx.x];
+}
+
+template <bool DPTS, bool DT>
+static void launch_transform_bwd(bool dirs, unsigned grid, const float* pts, long long V, const float* T, const float* g,
+                                 float* d_pts, float* out, cudaStream_t st) {
+    constexpr int threads = DT ? VT_THREADS : TB_PTS_THREADS;
+    if (dirs) transform_bwd_kernel<true, DPTS, DT><<<grid, threads, 0, st>>>(pts, V, T, g, d_pts, out);
+    else transform_bwd_kernel<false, DPTS, DT><<<grid, threads, 0, st>>>(pts, V, T, g, d_pts, out);
 }
 
 __global__ void __launch_bounds__(128) clamp_fov_kernel(const float* __restrict__ rays, int N, const float* __restrict__ M,
@@ -525,10 +616,38 @@ extern "C" int ffb_transform_points_bwd(const float* pts, int64_t V, const float
                                         float* d_pts, void* stream) {
     if (!pts || !T || !g_out || !d_pts || V < 0) return fail_arg(FFB_E_ARG, "transform_points_bwd: bad argument");
     if (V == 0) return 0;
-    const unsigned grid = (unsigned)((V + 127) / 128);
-    if (as_directions) transform_points_bwd_kernel<true><<<grid, 128, 0, as_stream(stream)>>>(pts, V, T, g_out, d_pts);
-    else transform_points_bwd_kernel<false><<<grid, 128, 0, as_stream(stream)>>>(pts, V, T, g_out, d_pts);
+    launch_transform_bwd<true, false>(as_directions, (unsigned)transform_bwd_grid(V, false), pts, V, T, g_out, d_pts, nullptr,
+                                      as_stream(stream));
     FFB_CUDA(cudaGetLastError());
+    return 0;
+}
+
+extern "C" size_t ffb_transform_bwd_workspace_bytes(int64_t V) {
+    if (V < 0) { fail_arg(FFB_E_ARG, "transform_bwd_workspace_bytes: V < 0"); return 0; }
+    const long long G = transform_bwd_grid(V, true);
+    return G > 1 ? (size_t)G * 16 * sizeof(float) : 0;
+}
+
+extern "C" int ffb_transform_points_bwd_full(const float* pts, int64_t V, const float* T, int as_directions, const float* g_out,
+                                             float* d_pts, float* d_T, void* workspace, size_t workspace_bytes, void* stream) {
+    if (!pts || !T || !g_out || !d_T || V < 0) return fail_arg(FFB_E_ARG, "transform_points_bwd_full: bad argument");
+    const size_t need = ffb_transform_bwd_workspace_bytes(V);
+    if (need && !workspace) return fail_arg(FFB_E_ARG, "transform_points_bwd_full: null workspace");
+    if (workspace_bytes < need) return fail_arg(FFB_E_WORKSPACE, "transform_points_bwd_full: workspace too small");
+    const cudaStream_t st = as_stream(stream);
+    if (V == 0) {
+        FFB_CUDA(cudaMemsetAsync(d_T, 0, 16 * sizeof(float), st));
+        return 0;
+    }
+    const int G = (int)transform_bwd_grid(V, true);
+    float* out = G > 1 ? static_cast<float*>(workspace) : d_T;
+    if (d_pts) launch_transform_bwd<true, true>(as_directions, G, pts, V, T, g_out, d_pts, out, st);
+    else launch_transform_bwd<false, true>(as_directions, G, pts, V, T, g_out, nullptr, out, st);
+    FFB_CUDA(cudaGetLastError());
+    if (G > 1) {
+        transform_bwd_fold_kernel<<<1, TB_FOLD_THREADS, 0, st>>>(out, G, d_T);
+        FFB_CUDA(cudaGetLastError());
+    }
     return 0;
 }
 

@@ -49,5 +49,7 @@ class Camera:
         self._transformable.randomize()
 
     def pointsToNDC(self, points) -> torch.Tensor:
+        """camera.py:67-74: points through ``world().inverse()`` and ``_perspective``; differentiable w.r.t. ``points``, the pose
+        and ``_perspective``."""
         view_space_points = ffmath.transform_points(points, self.world().inverse())
         return ffmath.transform_points(view_space_points, self._perspective)

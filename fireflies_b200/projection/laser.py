@@ -166,11 +166,11 @@ class Laser(Camera):
         self._transformable.set_world(to_world)
 
     def projectRaysToNDC(self) -> torch.Tensor:
-        """laser.py:262-275: ``transform_points(rays, K @ FLIP_Y)`` (differentiable w.r.t. ``_rays``)."""
+        """laser.py:262-275: ``transform_points(rays, K @ FLIP_Y)`` (differentiable w.r.t. ``_rays`` and ``_perspective``)."""
         return ffmath.transform_points(self._rays, self._M())
 
     def projectNDCPointsToWorld(self, points: torch.Tensor) -> torch.Tensor:
-        """laser.py:277-290."""
+        """laser.py:277-290 (differentiable w.r.t. ``points`` and ``_perspective``)."""
         return ffmath.transform_points(points, self._M().inverse())
 
     def generateTexture(self, sigma: float, texture_size: List[int]) -> torch.Tensor:
@@ -188,8 +188,8 @@ class Laser(Camera):
     def projector_texture(self, sigma: float, texture_size, blur=((5, 5), (3.0, 3.0))) -> torch.Tensor:
         """The projector texture the renderer reads (main.py:64-77): ``[ts[1], ts[0], 3]``, zeros in channels 0 and 2 and
         the Gaussian-blurred dense splat sum of the rays' NDC xy in channel 1.  ``blur`` = ``(kernel_size, sigma)`` as in
-        ``kornia.filters.gaussian_blur2d``, None = no blur.  Differentiable w.r.t. ``_rays``.  For B rendered samples per
-        step see :class:`fireflies_b200.TextureStep`."""
+        ``kornia.filters.gaussian_blur2d``, None = no blur.  Differentiable w.r.t. ``_rays`` and ``_perspective``.  For B rendered
+        samples per step see :class:`fireflies_b200.TextureStep`."""
         points = self.projectRaysToNDC()[:, 0:2]
         tex = rasterization.splat_reduce(points, sigma, texture_size, num_std_sum=None, num_std_softor=None, reduce=("sum",))[0]
         if blur is not None:
@@ -201,7 +201,8 @@ class Laser(Camera):
         """laser.py:298-325: the segments origin + [near_clip, far_clip] * ray, seen through ``camera_to_world`` (identity when
         omitted) and ``_perspective``, rasterised with ``rasterize_lines``.  The reference reads the camera pose through an
         attribute that does not exist (``self._fireflies.entity.Transformable.world()``, :304); the evident intent is the
-        viewing camera's world matrix, which the caller passes here."""
+        viewing camera's world matrix, which the caller passes here.  Differentiable w.r.t. ``_rays``, ``_perspective`` and
+        ``camera_to_world``."""
         lo = self.originPerRay() + self._near_clip * self.rays()
         hi = self.originPerRay() + self._far_clip * self.rays()
         if camera_to_world is None:

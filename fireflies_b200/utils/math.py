@@ -127,11 +127,6 @@ def convert_points_to_nonhomogeneous(points: torch.Tensor) -> torch.Tensor:
 class _TransformFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, points, transform, as_directions):
-        if torch.is_tensor(transform) and transform.requires_grad:
-            # the reference is plain torch, so d/d(transform) flows there; this kernel has no such backward -- say so instead of
-            # returning a silent None
-            raise NotImplementedError("fireflies_b200.transform_points / transform_directions: gradient w.r.t. the transform is not "
-                                      "implemented (only w.r.t. the points); detach the transform or compose it in torch")
         pts = nat.require_cuda(points.detach().float().contiguous(), torch.float32, "points")
         T = nat.require_cuda(transform.detach().float().contiguous(), torch.float32, "transform")
         if pts.dim() != 2 or pts.shape[1] != 3 or T.shape != (4, 4):
@@ -142,24 +137,39 @@ class _TransformFn(torch.autograd.Function):
         nat.count()
         ctx.save_for_backward(pts, T)
         ctx.dirs = as_directions
+        ctx.t_dtype = transform.dtype
         return out
 
     @staticmethod
+    @torch.autograd.function.once_differentiable
     def backward(ctx, g):
         pts, T = ctx.saved_tensors
         g = g.contiguous().float()
-        d = torch.empty_like(pts)
-        nat.check(nat.lib().ffb_transform_points_bwd(pts.data_ptr(), pts.shape[0], T.data_ptr(), int(ctx.dirs),
-                                                     g.data_ptr(), d.data_ptr(), nat.stream()), "ffb_transform_points_bwd")
-        nat.count()
-        return d, None, None
+        L = nat.lib()
+        if not ctx.needs_input_grad[1]:
+            d = torch.empty_like(pts)
+            nat.check(L.ffb_transform_points_bwd(pts.data_ptr(), pts.shape[0], T.data_ptr(), int(ctx.dirs),
+                                                 g.data_ptr(), d.data_ptr(), nat.stream()), "ffb_transform_points_bwd")
+            nat.count()
+            return d, None, None
+        d = torch.empty_like(pts) if ctx.needs_input_grad[0] else None
+        d_T = torch.empty(16, dtype=torch.float32, device=pts.device)
+        ws = torch.empty(L.ffb_transform_bwd_workspace_bytes(pts.shape[0]), dtype=torch.uint8, device=pts.device)
+        nat.check(L.ffb_transform_points_bwd_full(pts.data_ptr(), pts.shape[0], T.data_ptr(), int(ctx.dirs), g.data_ptr(),
+                                                  nat.ptr(d), d_T.data_ptr(), ws.data_ptr() if ws.numel() else None, ws.numel(),
+                                                  nat.stream()), "ffb_transform_points_bwd_full")
+        nat.count(2 if ws.numel() else 1)
+        return d, d_T.view(4, 4).to(ctx.t_dtype), None
 
 
 def transform_points(points: torch.Tensor, transform: torch.Tensor) -> torch.Tensor:
-    """utils/math.py:220-228: ``(T @ [x,y,z,1])[:3] / w``.  Differentiable w.r.t. ``points``."""
+    """utils/math.py:220-228: ``(T @ [x,y,z,1])[:3] / w``.  Differentiable w.r.t. ``points`` and ``transform`` (the
+    transform's gradient has its shape and dtype).  CUDA tensors only.  First derivatives only: differentiating the
+    gradient again (``create_graph=True``) raises."""
     return _TransformFn.apply(points, transform, False)
 
 
 def transform_directions(points: torch.Tensor, transform: torch.Tensor) -> torch.Tensor:
-    """utils/math.py:231-235: ``(T @ [x,y,z,0])[:3]``.  Differentiable w.r.t. ``points``."""
+    """utils/math.py:231-235: ``(T @ [x,y,z,0])[:3]``.  Differentiable w.r.t. ``points`` and ``transform`` (row 3 and
+    column 3 of its gradient are zero).  CUDA tensors only; first derivatives only, as :func:`transform_points`."""
     return _TransformFn.apply(points, transform, True)

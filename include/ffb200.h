@@ -278,6 +278,18 @@ FFB_API int ffb_transform_points(const float* pts, int64_t V, const float* T, in
  * projectRaysToNDC): d_pts[v] = J(pts[v])^T g_out[v]. */
 FFB_API int ffb_transform_points_bwd(const float* pts, int64_t V, const float* T, int as_directions, const float* g_out,
                                      float* d_pts, void* stream);
+/* The same backward w.r.t. the matrix as well (utils/math.py:220-235: the reference is a broadcast torch matmul, so autograd
+ * reaches T; the projector intrinsics and camera poses are optimised through it).  With d = dL/dh for h = T @ p~,
+ * p~ = [x,y,z,1] (points; d[3] carries the perspective divide) or [x,y,z,0] (directions):
+ *   d_T[i][j] = sum_v d_i(v) p~_j(v)      (f32 [16] row-major, DEVICE; row 3 and column 3 are 0 for directions)
+ *   d_pts[v]  = as ffb_transform_points_bwd, bit for bit; d_pts may be NULL (d_T only).
+ * One pass over pts and g_out; fp32 sums per CTA into `workspace` (DEVICE, at least ffb_transform_bwd_workspace_bytes(V),
+ * which is 0 -- NULL allowed -- when one CTA covers V), folded in fp64 in a fixed order.  The grid depends on V only, so
+ * repeated calls give the same bits.  One launch when the workspace size is 0, else two; V == 0 writes zeros.
+ * FFB_E_ARG: null pointer, V < 0, NULL workspace when one is needed.  FFB_E_WORKSPACE: workspace_bytes too small. */
+FFB_API size_t ffb_transform_bwd_workspace_bytes(int64_t V);
+FFB_API int ffb_transform_points_bwd_full(const float* pts, int64_t V, const float* T, int as_directions, const float* g_out,
+                                          float* d_pts, float* d_T, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Laser glue (projection/laser.py:199-206, 262-290).  M = K @ FLIP_Y and Minv are DEVICE f32 [16].
  * rays_to_ndc: ndc[n] = persp_div(M @ [ray,1]).
